@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: GraphDiT molecules/s (500-step sampling) and GIN graphs/s on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One JSON line on rank 0 (contract in the task statement / DESIGN.md section "Measurement"):
   * headline `value`  = GraphDiT molecules/s, whole job over all N GPUs, BASELINE.json configs[2]
@@ -15,6 +15,8 @@ One JSON line on rank 0 (contract in the task statement / DESIGN.md section "Mea
   * `roofline`       = dominant kernel (live CUDA-event timing inside the timed region) against the measured peak.
   * `cpu_baseline`   = the CPU oracle (the reference's algorithm in PyTorch fp32) on the box's host cores.
 `--impl reference` times that CPU implementation alone with the same metric/config keys.
+`--dump-outputs DIR` writes what the timed paths returned in their last timed step (see dump_outputs); every input is seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,10 +37,29 @@ import torch  # noqa: E402
 METRIC = "GraphDiT molecules/sec (500-step sampling) and GIN graphs/sec at 1/2/4/8 B200"
 DIT = dict(hidden=1024, depth=28, heads=16, mlp_ratio=4.0, T=500, guide_scale=2.0, max_nodes=50)
 GIN = dict(hidden=768, layers=5)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(path, arrays):
+    """Writes `arrays` (name -> tensor) as <path>/<name>.npy: float32, or float64 for integers float32 cannot hold exactly.  The
+    default workload's outputs come to ~37 MB; when they exceed DUMP_MAX_BYTES in all, each array keeps a fixed, seeded sample of
+    its rows (leading dimension), listed in <name>_rows.npy."""
+    import numpy as np
+
+    arrays = {k: (v.float() if v.is_floating_point() or int(v.abs().max()) < 2 ** 24 else v.double()) for k, v in arrays.items()}
+    frac = min(1.0, 0.9 * DUMP_MAX_BYTES / sum(v.numel() * v.element_size() + 8 * v.shape[0] for v in arrays.values()))
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        if frac < 1.0:
+            rows = torch.randperm(v.shape[0], generator=torch.Generator().manual_seed(0))[: max(1, int(v.shape[0] * frac))].sort().values
+            v = v[rows]
+            np.save(os.path.join(path, f"{name}_rows.npy"), rows.double().numpy())
+        np.save(os.path.join(path, f"{name}.npy"), v.numpy())
+    log(f"[bench] wrote {', '.join(sorted(arrays))} to {path}" + (f" (row sample: {frac:.3f} of each)" if frac < 1.0 else ""))
 
 
 def peaks():
@@ -191,11 +212,11 @@ def run_reference(args, rank, world):
     meta = synth.dit_meta(DIT["max_nodes"])
     sd = synth.dit_state_dict(cfg, DIT["max_nodes"], seed=1234)
     B = 16
-    sec = cpu_dit_step_seconds(cfg, meta, sd, B, max(1, args.steps), max(0, args.warmup))
+    sec = cpu_dit_step_seconds(cfg, meta, sd, B, args.steps, args.warmup)
     val = B / (DIT["T"] * sec)
     enc, proj = synth.gin_encoder_state_dicts(GIN["layers"], GIN["hidden"], seed=11)
     graphs = synth.molecular_graphs(512, seed=0)
-    gsec = cpu_gin_seconds(enc, proj, graphs)
+    gsec = cpu_gin_seconds(enc, proj, graphs, reps=args.steps)
     cores = torch.get_num_threads()
     sample = f"{B} of {args.dit_batch} molecules per step (one reverse step = cond+uncond denoiser pass + posterior + sampling), fp32, {cores} threads"
     out = {
@@ -205,7 +226,7 @@ def run_reference(args, rank, world):
         "config": workload_config(args),
         "cpu_baseline": {"value": val, "unit": "molecules/s", "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": val, "unit": "molecules/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-        "gin": {"value": 512 / gsec, "unit": "graphs/s", "sample": "512 of 4096 graphs, one encoder forward", "cores": cores},
+        "gin": {"value": 512 / gsec, "unit": "graphs/s", "sample": f"512 of 4096 graphs, mean of {args.steps} encoder forwards", "cores": cores},
         "gpu_launches": 0,
     }
     print(json.dumps(out), flush=True)
@@ -230,8 +251,14 @@ def workload_config(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed iterations of every timed loop, 1..500 (one sampling run has 500 reverse steps): the reverse steps of the "
+                         "throughput, ragged and end-to-end DiT sections, the GIN forwards and the predictor passes.  Fixed counts: the "
+                         "latency section times 200 steps per batch size, since one step there lasts 1.3-1.8 ms (--no-latency skips it), "
+                         "and the CPU baseline of the B200 path samples 3 steps and one GIN forward, as its `sample` strings say")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed steps before each timed loop.  The B200 path runs at least 3 (the first launches load modules and fill "
+                         "the TMA descriptor cache), logs it when it raises the number and reports the number it ran")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--dit-batch", type=int, default=2048)
     ap.add_argument("--gin-graphs", type=int, default=4096)
@@ -242,14 +269,22 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true", help="skip the small-batch latency section (profiler captures of the throughput step)")
     ap.add_argument("--only", default="", choices=["", "gin", "predictor"], help="development: time one GIN sub-benchmark alone and print its object")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the timed paths returned in their last step as DIR/<name>.npy (rank 0's shard): "
+                         "the sampled graphs dit_X (B, N) and dit_E (B, N, N), gin_embedding, predictor_probs, predictor_indices")
     args = ap.parse_args()
+    if not 1 <= args.steps <= DIT["T"] or args.warmup < 0:
+        ap.error(f"--steps must be in 1..{DIT['T']} and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         return run_reference(args, rank, world)
-    args.warmup = max(3, args.warmup)
-    args.steps = max(1, args.steps)
+    if args.warmup < 3:
+        log(f"[bench] --warmup {args.warmup} raised to 3: the first launches load modules and fill the TMA descriptor cache")
+        args.warmup = 3
 
     import torch.distributed as dist
 
@@ -282,7 +317,10 @@ def main():
     if args.only:
         fn = bench_gin if args.only == "gin" else bench_predictor
         out = fn(args, device, rank, world, barrier, max_over_ranks, pk)
+        outputs = out.pop("_outputs")
         if rank == 0:
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps(out), flush=True)
         if world > 1:
             dist.destroy_process_group()
@@ -346,6 +384,10 @@ def main():
     prof = _cabi.profile_read()
     _cabi.profile_enable(False)
     dit_launches = eng.launch_count() - launches0
+    outputs = {}
+    if args.dump_outputs:
+        Xd, Ed = eng.get_state()    # the sampled graphs after the last timed step, as the step loop's caller reads them
+        outputs.update(dit_X=Xd.cpu(), dit_E=Ed.cpu())
     ms_step = ms_total / args.steps
     value = world * B / (T * ms_step / 1e3)
     flops_step = 2 * dit_flops_per_pass(n_nodes, cfg["hidden_size"], cfg["depth"], 16 + 5 * N)
@@ -376,7 +418,7 @@ def main():
                        "peak": pk["hbm"], "unit": "GB/s", "frac": sk_bytes / (sk_ms / 1e3) / 1e9 / pk["hbm"], "share_of_step": sk_ms / ms_step,
                        "note": "latency-bound (one CTA per molecule, two 106 KB CTAs per SM), not bandwidth-bound: 1.3 % of the step"}
     # ------------------------------------------------------------------ e2e through the public API (host buffers)
-    k_e2e = min(args.steps, 10)
+    k_e2e = args.steps
     outX = torch.empty((B, N), dtype=torch.int64).pin_memory()
     outE = torch.empty((B, N, N), dtype=torch.int64).pin_memory()
     if world > 1:
@@ -417,10 +459,10 @@ def main():
         for i in range(args.warmup):
             eng.step(T - i, 7)
         barrier()
-        k_rag = min(args.steps, 10)
+        k_rag = args.steps
         ev0.record()
         for i in range(k_rag):
-            eng.step(T - args.warmup - i, 7)
+            eng.step(T - ((args.warmup + i) % T), 7)
         ev1.record()
         barrier()
         rag_ms = max_over_ranks(ev0.elapsed_time(ev1)) / k_rag
@@ -431,9 +473,11 @@ def main():
                   "note": "node counts ~ the (synthetic) checkpoint histogram, uniform on 5..N; varlen packing: only valid atoms are computed"}
     # ------------------------------------------------------------------ GIN encoder
     gin = bench_gin(args, device, rank, world, barrier, max_over_ranks, pk)
+    outputs.update(gin.pop("_outputs"))
     pred = None
     if not args.no_predictor and not args.small:
         pred = bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk)
+        outputs.update(pred.pop("_outputs"))
     # ------------------------------------------------------------------ CPU baseline (rank 0, N=1)
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline and not args.small:
@@ -447,6 +491,8 @@ def main():
             pred["cpu_baseline"] = predictor_cpu_baseline(args)
         log(f"cpu baseline took {time.time() - t0:.1f}s")
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         out = {
             "metric": METRIC, "value": value, "unit": "molecules/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
@@ -525,8 +571,8 @@ def bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk):
     n, e = int(x.numel()), int(ea.numel())
     eng = m.engine()
     log(f"predictor set-up took {time.time() - t0:.1f}s")
-    iters = 5
-    for _ in range(3):
+    iters = args.steps
+    for _ in range(args.warmup):
         eng.bind(xd, eid, ead, bd, num_graphs=G, want_logits=True, validate=False)
         probs, idx = eng.predictor_topk(c, k)
     barrier()
@@ -547,9 +593,10 @@ def bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk):
     prof = _cabi.profile_read()
     _cabi.profile_enable(False)
     launches = eng.launch_count() - l0
+    outputs = {"predictor_probs": probs.cpu(), "predictor_indices": idx.cpu()} if args.dump_outputs else {}
     head_stats = eng.head_stats()
     # strong scaling of BASELINE.json configs[3]: 65 536 reactant graphs in total, 65 536 / N per GPU (the local batch repeated with
-    # node offsets; same graph statistics), one bind + top-50 pass + gather
+    # node offsets; same graph statistics), `--steps` timed passes of bind + top-50 + gather
     strong = None
     total_graphs = 65536
     if total_graphs % (world * G) == 0 or total_graphs // world >= G:
@@ -565,13 +612,14 @@ def bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk):
             ps, is_ = eng.predictor_topk(cs, k)
         barrier()
         ev0.record()
-        eng.bind(xs, eis, eas, bs, num_graphs=Gs, want_logits=True, validate=False)
-        ps, is_ = eng.predictor_topk(cs, k)
-        if world > 1:
-            sharding.all_gather_rows(torch.cat([ps, is_.to(torch.float32)], dim=1), sizes=[Gs] * world)
+        for _ in range(args.steps):
+            eng.bind(xs, eis, eas, bs, num_graphs=Gs, want_logits=True, validate=False)
+            ps, is_ = eng.predictor_topk(cs, k)
+            if world > 1:
+                sharding.all_gather_rows(torch.cat([ps, is_.to(torch.float32)], dim=1), sizes=[Gs] * world)
         ev1.record()
         barrier()
-        ms_s = max_over_ranks(ev0.elapsed_time(ev1))
+        ms_s = max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
         strong = {"total_graphs": world * Gs, "graphs_per_gpu": Gs, "ms": ms_s, "value": world * Gs / (ms_s / 1e3), "unit": "graphs/s", "scaling": "strong",
                   "note": "fixed total of 65 536 candidate graphs split over the GPUs; compare `ms` across N"}
         del xs, eas, eis, bs, cs, ps, is_
@@ -581,7 +629,7 @@ def bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk):
     hi = torch.empty((G, k), dtype=torch.int32).pin_memory()
     barrier()
     t0 = time.perf_counter()
-    reps = 3
+    reps = args.steps
     for _ in range(reps):
         pr, ix = m.topk_templates(xp.to(device, non_blocking=True), eip.to(device, non_blocking=True), eap.to(device, non_blocking=True),
                                   bp.to(device, non_blocking=True), cp.to(device, non_blocking=True), k)
@@ -603,7 +651,7 @@ def bench_predictor(args, device, rank, world, barrier, max_over_ranks, pk):
                      "traffic": None, "peak_source": pk["source"], "flops_per_batch": head_flops, "whole_batch_tflops": (trunk_flops + head_flops) / (ms / 1e3) / 1e12},
         "kernel_breakdown": {k_: {"ms_per_batch": v[0] / iters, "launches": v[1] / iters} for k_, v in prof.items() if k_.startswith("gin_")},
         "strong_scaling": strong, "head": head_stats,
-        "_launches": launches,
+        "_launches": launches, "_outputs": outputs,
     }
     del m, eng
     torch.cuda.empty_cache()
@@ -656,8 +704,8 @@ def bench_gin(args, device, rank, world, barrier, max_over_ranks, pk):
     xd, eid, ead, bd = (t.to(device) for t in (x, ei, ea, batch))
     n, e = int(x.numel()), int(ea.numel())
     eng = g.engine()
-    iters = max(10, args.steps)
-    for _ in range(max(3, args.warmup)):
+    iters = args.steps
+    for _ in range(args.warmup):
         eng.bind(xd, eid, ead, bd, num_graphs=G, validate=False)
         out = eng.encoder_forward()
     barrier()
@@ -674,6 +722,7 @@ def bench_gin(args, device, rank, world, barrier, max_over_ranks, pk):
     prof = _cabi.profile_read()
     _cabi.profile_enable(False)
     launches = eng.launch_count() - l0
+    outputs = {"gin_embedding": out.cpu()} if args.dump_outputs else {}
     H, L = GIN["hidden"], GIN["layers"]
     agg_bytes = (e + 2 * n) * H * 2      # per layer launch (SURVEY.md section 8d: gathered neighbours + self, bf16, + output)
     agg_ms = prof["gin_aggregate"][0] / prof["gin_aggregate"][1]
@@ -686,7 +735,7 @@ def bench_gin(args, device, rank, world, barrier, max_over_ranks, pk):
     host_out.copy_(emb)   # one untimed call: allocator / pinned-copy warm-up
     barrier()
     t0 = time.perf_counter()
-    reps = 5
+    reps = args.steps
     for _ in range(reps):
         emb = g(xp.to(device, non_blocking=True), eip.to(device, non_blocking=True), eap.to(device, non_blocking=True), bp.to(device, non_blocking=True))
         host_out.copy_(emb, non_blocking=True)
@@ -706,7 +755,7 @@ def bench_gin(args, device, rank, world, barrier, max_over_ranks, pk):
         "whole_forward": {"tflops": mlp_flops / (ms / 1e3) / 1e12, "frac_of_sustained": mlp_flops / (ms / 1e3) / 1e12 / pk["tf_sustained"],
                           "note": "algorithmic MLP FLOPs over the whole forward (CSR build, aggregation, GEMMs, pooling, head)"},
         "kernel_breakdown": {k: {"ms_per_forward": v[0] / iters, "launches": v[1] / iters} for k, v in prof.items()},
-        "_launches": launches,
+        "_launches": launches, "_outputs": outputs,
     }
 
 

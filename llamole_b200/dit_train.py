@@ -8,7 +8,7 @@ and to `text_embedding`.  It is plain eager PyTorch on whatever device the modul
 semantics (no reference import, no oracle import), and it consumes torch's global RNG in the reference's order -- timestep
 draw, the two multinomial noise draws, then per property the condition-dropout uniforms and the N(0,1) embedding noise, then
 the text-dropout uniforms -- so that with the same `torch.manual_seed` it reproduces the reference's loss
-(tests/test_oracle_vs_reference.py checks that against the verbatim module).
+(checked against the verbatim module when it was written; the repository holds no copy of that module).
 
 Reference behaviours kept on purpose (they define the loss value):
   * padded atom pairs carry the "no bond" class after `encode_no_edge` (diffusion_utils.py:128-141), so they DO enter the bond

@@ -6,10 +6,9 @@ loudly when its CUDA library is missing.
 
 Parity status: PINNED.  The reference ships no tests or golden vectors (SURVEY.md section 4), so the
 pin is the reference itself: oracle/make_golden.py imports the reference's modules verbatim from
-/root/reference in the authoring container (oracle/ref_import.py), runs them on seeded inputs and
+a checkout of the original repository (oracle/ref_import.py), runs them on seeded inputs and
 pre-drawn noise, and commits the outputs under tests/golden/; tests/test_oracle.py checks every
-function here against those fixtures, and tests/test_oracle_vs_reference.py repeats the comparison
-live whenever /root/reference is present.
+function here against those fixtures.
 
 Every function works on a flat `state_dict` (name -> tensor, the reference's checkpoint layout,
 SURVEY.md section 8b) instead of nn.Modules, and cites the reference lines it follows.  Paths are relative

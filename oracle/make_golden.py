@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.pt by running the UNMODIFIED reference modules (authoring container only).
+"""Generate tests/golden/*.pt by running the UNMODIFIED reference modules (needs LLAMOLE_REFERENCE_ROOT, see oracle/ref_import.py).
 
-TEST INFRASTRUCTURE ONLY.  Usage:  python -m oracle.make_golden  [--out tests/golden]
+TEST INFRASTRUCTURE ONLY.  Usage:  LLAMOLE_REFERENCE_ROOT=<checkout> python -m oracle.make_golden  [--out tests/golden]
 
 The reference has no tests or golden vectors of its own (SURVEY.md section 4), so the pin is made here:
 the reference's GraphDiT / GraphCLIP / GraphPredictor are imported verbatim (oracle/ref_import.py),
@@ -11,6 +11,7 @@ with pre-drawn Exp(1) noise.  Fixtures hold inputs + outputs + the seeds that re
 from __future__ import annotations
 
 import argparse
+import hashlib
 import os
 import sys
 import tempfile
@@ -31,11 +32,29 @@ def checksum(sd) -> float:
     return float(sum(v.double().abs().sum() for v in sd.values()))
 
 
+def _sha256(t) -> str:
+    return hashlib.sha256(t.contiguous().numpy().tobytes()).hexdigest()
+
+
 def pack_meta(meta):
-    """Lossless compact form: the big nested lists become float32 tensors (they were float32 to begin with)."""
+    """Compact form: transition_E (118 x 118 x 5 floats, a third of the fixture) is not stored.  load_fixture regenerates it
+    from params["meta_seed"] and checks it against the SHA-256 of its float32 bytes kept here."""
     m = dict(meta)
-    m["transition_E"] = torch.tensor(meta["transition_E"], dtype=torch.float32)
+    m["transition_E_sha256"] = _sha256(torch.tensor(m.pop("transition_E"), dtype=torch.float32))
     return m
+
+
+def load_fixture(path):
+    """A fixture written by this script, with the DiT meta back in the checkpoint's form (transition_E a nested list)."""
+    fx = torch.load(path, weights_only=False)
+    if "meta" in fx:
+        P, m = fx["params"], dict(fx["meta"])
+        trans = synth.dit_meta(P["max_nodes"], P["meta_seed"], min_nodes=1)["transition_E"]
+        if _sha256(torch.tensor(trans, dtype=torch.float32)) != m.pop("transition_E_sha256"):
+            raise AssertionError("synthetic meta generator drifted: transition_E differs from the one the fixture was made with")
+        m["transition_E"] = trans
+        fx["meta"] = m
+    return fx
 
 
 def exp_noise(g, *shape):

@@ -1,15 +1,14 @@
-"""Import the reference's three hot-path packages VERBATIM from /root/reference.
+"""Import the reference's three hot-path packages VERBATIM from a checkout of the original Llamole repository.
 
 TEST INFRASTRUCTURE ONLY (never imported by the product path).
 
-Works only where /root/reference exists (the authoring container).  It is used by
-  * oracle/make_golden.py  -> writes tests/golden/*.pt (the fixtures that travel to the GPU box)
-  * tests/test_oracle_vs_reference.py -> pins oracle/llamole_oracle.py against the real modules
-Nothing under tests -m gpu, smoke() or bench.py may call this.
+Works only where LLAMOLE_REFERENCE_ROOT names such a checkout; the repository does not contain one.  Its one user is
+oracle/make_golden.py, which writes tests/golden/*.pt (the stored reference outputs the suite compares against).
+Nothing under tests/, smoke() or bench.py may call this.
 
 The reference packages have no __init__.py; they import as namespace packages once
-/root/reference/src/model is on sys.path (SURVEY.md section 8c).  torch_geometric / rdkit / rdchiral
-are not installed here, so the stand-ins under oracle/standins are put on sys.path first.
+<checkout>/src/model is on sys.path (SURVEY.md section 8c).  torch_geometric / rdkit / rdchiral
+need not be installed: where they are missing, the stand-ins under oracle/standins are put on sys.path first.
 """
 from __future__ import annotations
 
@@ -19,12 +18,13 @@ from contextlib import contextmanager
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("LLAMOLE_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("LLAMOLE_REFERENCE_ROOT", "")
+REFERENCE_MODEL_DIR = os.path.join(REFERENCE_ROOT, "src", "model")
 _STANDINS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "standins")
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "src", "model", "graph_decoder"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_MODEL_DIR, "graph_decoder"))
 
 
 _cache = {}
@@ -35,16 +35,15 @@ def load_reference():
     if "mods" in _cache:
         return _cache["mods"]
     if not reference_available():
-        raise FileNotFoundError(f"reference tree not found under {REFERENCE_ROOT}")
+        raise FileNotFoundError(f"reference tree not found under {REFERENCE_ROOT!r}: set LLAMOLE_REFERENCE_ROOT to a checkout of the original Llamole repository")
     for name in ("torch_geometric", "rdkit", "rdchiral"):
         try:
             __import__(name)
         except Exception:
             if _STANDINS not in sys.path:
                 sys.path.insert(0, _STANDINS)
-    model_dir = os.path.join(REFERENCE_ROOT, "src", "model")
-    if model_dir not in sys.path:
-        sys.path.append(model_dir)
+    if REFERENCE_MODEL_DIR not in sys.path:
+        sys.path.append(REFERENCE_MODEL_DIR)
     import graph_decoder.diffusion_model as dm  # type: ignore
     import graph_decoder.diffusion_utils as du  # type: ignore
     import graph_encoder.model as ge  # type: ignore

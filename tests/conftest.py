@@ -15,13 +15,9 @@ def pytest_configure(config):
 
 
 def load_golden(name):
-    import torch
+    from oracle.make_golden import load_fixture
 
-    fx = torch.load(os.path.join(GOLDEN, name), weights_only=False)
-    if "meta" in fx and not isinstance(fx["meta"]["transition_E"], list):
-        fx["meta"] = dict(fx["meta"])
-        fx["meta"]["transition_E"] = fx["meta"]["transition_E"].tolist()
-    return fx
+    return load_fixture(os.path.join(GOLDEN, name))
 
 
 @pytest.fixture(scope="session")

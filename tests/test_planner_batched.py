@@ -1,17 +1,12 @@
 """Batched A* expansion (llamole_b200/planner.py, SURVEY.md section 8f-1): with beam = 1 it is the reference's search loop
-(planner/molstar.py:11-76) -- checked LIVE against the verbatim `molstar` + `MolTree` wherever /root/reference exists, and
-against a literal restatement of that loop on a stand-in tree everywhere; with beam > 1 the expansions and the value
-evaluations arrive in batches."""
+(planner/molstar.py:11-76) -- checked against a literal restatement of that loop on a stand-in tree; with beam > 1 the
+expansions and the value evaluations arrive in batches."""
 import hashlib
-import os
-import sys
 
 import numpy as np
 import pytest
 
 from llamole_b200.planner import ValueCache, molstar_batched, predictor_expand_batch_fn
-
-REF_MODEL_DIR = "/root/reference/src/model"
 
 
 def _h(*parts) -> int:
@@ -59,54 +54,6 @@ class Network:
     def value_batch_fn(self, mols):
         self.value_calls.append(list(mols))
         return [self.value_one(m) for m in mols]
-
-
-def _reference_planner():
-    if not os.path.isdir(os.path.join(REF_MODEL_DIR, "planner")):
-        pytest.skip("/root/reference is not present on this machine")
-    if REF_MODEL_DIR not in sys.path:
-        sys.path.append(REF_MODEL_DIR)
-    import importlib
-
-    ms = importlib.import_module("planner.molstar")   # (the package's __init__ rebinds `planner.molstar` to the function)
-    mt = importlib.import_module("planner.mol_tree")
-    return ms.molstar, mt.MolTree
-
-
-def _route_key(route):
-    if route is None:
-        return None
-    return (tuple(route.mols), tuple(route.templates), round(float(route.total_cost), 9), int(route.length))
-
-
-@pytest.mark.parametrize("seed", range(12))
-def test_beam_one_is_the_reference_search(seed):
-    molstar, MolTree = _reference_planner()
-    net_a, net_b = Network(seed), Network(seed)
-    want = molstar("m0", 0, net_a.starting, net_a.expand_fn, net_a.value_fn, iterations=25, max_time=60)
-    got = molstar_batched("m0", 0, net_b.starting, net_b.expand_batch_fn, net_b.value_batch_fn, iterations=25, beam=1, max_time=60,
-                          tree_factory=MolTree)
-    assert got[0] == want[0] and got[2] == want[2]
-    assert _route_key(got[1]) == _route_key(want[1])
-    assert [c[0] for c in net_b.expand_calls] == [c[0] for c in net_a.expand_calls]      # same molecules expanded, in the same order
-
-
-@pytest.mark.parametrize("seed", range(6))
-def test_beam_batches_expansions_and_values_on_the_reference_tree(seed):
-    _, MolTree = _reference_planner()
-    net1, net8 = Network(seed), Network(seed)
-    r1 = molstar_batched("m0", 0, net1.starting, net1.expand_batch_fn, net1.value_batch_fn, iterations=40, beam=1, tree_factory=MolTree)
-    stats = {}
-    r8 = molstar_batched("m0", 0, net8.starting, net8.expand_batch_fn, net8.value_batch_fn, iterations=40, beam=8, tree_factory=MolTree,
-                         stats=stats)
-    assert all(1 <= len(c) <= 8 for c in net8.expand_calls) and r8[2] <= 40
-    assert stats["expand_calls"] == len(net8.expand_calls) and stats["value_batch_calls"] == len(net8.value_calls)
-    assert stats["value_batch_calls"] <= stats["expand_calls"] + 1          # one batched evaluation per round (+ the target)
-    if r1[0]:
-        # a wider beam explores a superset frontier per round: whenever the serial search succeeds within its budget the batched
-        # one does too, with far fewer (batched) model calls
-        assert r8[0] and len(net8.expand_calls) <= len(net1.expand_calls)
-        assert r8[1].total_cost <= r1[1].total_cost + 1e-9 or r8[1].length >= 1
 
 
 class _Node:
