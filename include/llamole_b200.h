@@ -211,7 +211,8 @@ int llb_dit_posterior_sample(llb_dit* h, int t, const float* lc_X, const float* 
  * GIN encoder / predictor  (graph_encoder/model.py:37-41,124-205; graph_predictor/model.py:306-353,387-391)
  * ---------------------------------------------------------------------------------------------------- */
 typedef struct {
-  int32_t hidden;      /* H, multiple of 64 */
+  int32_t hidden;      /* H >= 1, any value: stored zero-padded to a multiple of 64 (and 4H likewise), so a width that is not a
+                          multiple of 64 costs the FLOPs and bytes of the padded one */
   int32_t layers;      /* L >= 2 */
   int32_t predictor;   /* 0 = GraphCLIP encoder, 1 = GNNRetrosynthsizer */
   int32_t out_dim;     /* predictor: template classes; encoder: ignored */

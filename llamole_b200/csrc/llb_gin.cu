@@ -25,13 +25,20 @@ constexpr int HEAD_PILOT_COLS = 4096;         // strided sample of the templates
 constexpr int HEAD_CAND_CAP = 2048;           // candidates above the threshold kept per row
 constexpr int HEAD_ROW_CHUNK = 8192;          // rows per fused pass: 50 MB of head inputs stay L2-resident while the weight streams once
 
+// Widths.  H is the model's hidden size, any H >= 1.  Every H-wide operand and activation is stored with Hp = round_up(H, 64)
+// columns and every 4H-wide one with I = round_up(4H, 64); the padding of the parameters is zero, so the padded columns of every
+// activation stay exactly 0 through embeddings, GEMMs, biases, GELU (gelu(0) = 0), residuals, pooling and the virtual node.  The
+// only code that must know the true width is the LayerNorm statistics (divide by H / 4H) and the predictor's non-affine
+// LayerNorm, which would otherwise write -mean * rstd into the padded columns (row LayerNorms get `valid` = the true width).
+// When H % 64 == 0, Hp == H and I == 4H.  Below, "(4H,H)" etc. name the true shape and the stored shape is (I,Hp).
 struct GinLayout {
-  int H, L, predictor, out_dim, tdim, HH, HO;
+  int H, Hp, I, L, predictor, out_dim, tdim;
+  int HH, HHt, HO;   // head: hidden width (padded, true), output width (padded: Hp for the encoder, out_dim for the predictor)
   std::vector<size_t> mlp0_w, mlp4_w, vn0_w, vn4_w, adapter_w;   // bf16
   std::vector<size_t> mlp_chol;                                    // bf16 (H,H): Cholesky factor of the node MLP's first linear (analytic LayerNorm)
-  std::vector<size_t> mlp_stat;                                    // fp32 [r (H) | c0, 0, 0, 0]: bias column and constant of that factor
+  std::vector<size_t> mlp_stat;                                    // fp32 [r (Hp, 0 past H) | c0 at Hp, 0, 0, 0]: bias column and constant of that factor
   std::vector<size_t> mlp_bg;                                      // fp32 (4H): centred bias x LayerNorm gamma
-  size_t chol_scratch;                                             // fp64 (H+1, H+1) Gram matrix, pack time only
+  size_t chol_scratch;                                             // fp64 (H+1, H+1) Gram matrix (true H), pack time only
   size_t head0_w, head4_w;
   size_t pilot_w, pilot_b;     // (pilot_cols, HH) bf16 / (pilot_cols) fp32: every pilot_stride-th template of the head (fused top-k)
   int pilot_cols, pilot_stride;
@@ -43,12 +50,14 @@ struct GinLayout {
 };
 
 int make_layout(const llb_gin_config& c, GinLayout& G) {
-  LLB_CHECK_ARG(c.hidden > 0 && c.hidden % 64 == 0, "gin: hidden=%d must be a positive multiple of 64", c.hidden);
+  LLB_CHECK_ARG(c.hidden > 0, "gin: hidden=%d must be positive", c.hidden);
   LLB_CHECK_ARG(c.layers >= 2, "gin: layers=%d must be >= 2 (reference raises ValueError too)", c.layers);
   LLB_CHECK_ARG(!c.predictor || (c.out_dim >= 1 && c.text_dim > 0 && c.text_dim % 8 == 0), "gin: bad predictor out_dim/text_dim");
   G.H = c.hidden, G.L = c.layers, G.predictor = c.predictor ? 1 : 0, G.out_dim = c.out_dim, G.tdim = c.text_dim;
-  G.HH = G.predictor ? 4 * G.H : G.H;
-  G.HO = G.predictor ? G.out_dim : G.H;
+  G.Hp = (int)align_up(G.H, 64), G.I = (int)align_up(4 * (size_t)G.H, 64);
+  G.HH = G.predictor ? G.I : G.Hp;
+  G.HHt = G.predictor ? 4 * G.H : G.H;
+  G.HO = G.predictor ? G.out_dim : G.Hp;
   size_t off = 0;
   auto take = [&](size_t bytes) {
     off = align_up(off, 256);
@@ -56,14 +65,14 @@ int make_layout(const llb_gin_config& c, GinLayout& G) {
     off += bytes;
     return o;
   };
-  const size_t H = G.H;
+  const size_t H = G.Hp, I = G.I;
   for (int l = 0; l < G.L; ++l) {
-    G.mlp0_w.push_back(take(4 * H * H * 2));
-    G.mlp4_w.push_back(take(4 * H * H * 2));
+    G.mlp0_w.push_back(take(I * H * 2));
+    G.mlp4_w.push_back(take(I * H * 2));
     G.mlp_chol.push_back(take(H * H * 2));
     if (l < G.L - 1) {
-      G.vn0_w.push_back(take(4 * H * H * 2));
-      G.vn4_w.push_back(take(4 * H * H * 2));
+      G.vn0_w.push_back(take(I * H * 2));
+      G.vn4_w.push_back(take(I * H * 2));
     }
     if (G.predictor) G.adapter_w.push_back(take(3 * H * (size_t)G.tdim * 2));
   }
@@ -74,14 +83,14 @@ int make_layout(const llb_gin_config& c, GinLayout& G) {
   G.text_drop = take((size_t)(G.predictor ? G.tdim : 1) * 4);
   for (int l = 0; l < G.L; ++l) {
     G.eps.push_back(take(4));
-    G.mlp0_b.push_back(take(4 * H * 4)), G.mlp_ln_w.push_back(take(4 * H * 4)), G.mlp_ln_b.push_back(take(4 * H * 4));
+    G.mlp0_b.push_back(take(I * 4)), G.mlp_ln_w.push_back(take(I * 4)), G.mlp_ln_b.push_back(take(I * 4));
     G.mlp4_b.push_back(take(H * 4));
     G.mlp_stat.push_back(take((H + 4) * 4));
-    G.mlp_bg.push_back(take(4 * H * 4));
+    G.mlp_bg.push_back(take(I * 4));
     G.bond_emb.push_back(take(BOND_VOCAB * H * 4));
     G.norm_w.push_back(take(H * 4)), G.norm_b.push_back(take(H * 4));
     if (l < G.L - 1) {
-      G.vn0_b.push_back(take(4 * H * 4)), G.vn_ln_w.push_back(take(4 * H * 4)), G.vn_ln_b.push_back(take(4 * H * 4));
+      G.vn0_b.push_back(take(I * 4)), G.vn_ln_w.push_back(take(I * 4)), G.vn_ln_b.push_back(take(I * 4));
       G.vn4_b.push_back(take(H * 4));
     }
     if (G.predictor) G.adapter_b.push_back(take(3 * H * 4));
@@ -92,7 +101,7 @@ int make_layout(const llb_gin_config& c, GinLayout& G) {
   G.pilot_cols = (G.predictor && G.out_dim >= HEAD_FUSED_MIN_WIDTH) ? HEAD_PILOT_COLS : 0;
   G.pilot_stride = G.pilot_cols ? G.out_dim / G.pilot_cols : 0;
   G.pilot_w = take((size_t)G.pilot_cols * G.HH * 2), G.pilot_b = take((size_t)G.pilot_cols * 4);
-  G.chol_scratch = take((H + 1) * (H + 1) * 8);
+  G.chol_scratch = take(((size_t)G.H + 1) * (G.H + 1) * 8);
   G.total = align_up(off, 256);
   return LLB_OK;
 }
@@ -329,11 +338,12 @@ __global__ void __launch_bounds__(256) gin_colmean_kernel(const float* __restric
   for (int o = 0; o < rows; ++o) s += (double)W[(size_t)o * H + k];
   wbar[k] = (float)(s / rows);
 }
+// W (rows, H) contiguous -> out (rows, H) with row stride out_ld
 __global__ void gin_center_weight_kernel(const float* __restrict__ W, const float* __restrict__ wbar, int rows, int H,
-                                         __nv_bfloat16* __restrict__ out) {
+                                         __nv_bfloat16* __restrict__ out, int out_ld) {
   const size_t total = (size_t)rows * H;
   for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x)
-    out[idx] = __float2bfloat16(W[idx] - wbar[idx % H]);
+    out[(idx / H) * out_ld + idx % H] = __float2bfloat16(W[idx] - wbar[idx % H]);
 }
 // bc = b - mean(b), bg = bc * gamma (one block)
 __global__ void __launch_bounds__(1024) gin_center_bias_kernel(const float* __restrict__ b, const float* __restrict__ gamma, int rows,
@@ -358,15 +368,16 @@ __global__ void __launch_bounds__(1024) gin_center_bias_kernel(const float* __re
     bg[o] = c * gamma[o];
   }
 }
-// Gram matrix of the augmented weight Wt = [Wc (bf16) | bc] in fp64: Gm (H+1, H+1), one thread per entry, pack time only.
-__global__ void __launch_bounds__(256) gin_gram64_kernel(const __nv_bfloat16* __restrict__ Wc, const float* __restrict__ bc, int rows, int H,
-                                                         double* __restrict__ Gm) {
+// Gram matrix of the augmented weight Wt = [Wc (bf16, row stride ld) | bc] in fp64: Gm (H+1, H+1), one thread per entry, pack
+// time only.  H is the true width: the padded columns of Wc would make the matrix singular.
+__global__ void __launch_bounds__(256) gin_gram64_kernel(const __nv_bfloat16* __restrict__ Wc, int ld, const float* __restrict__ bc, int rows,
+                                                         int H, double* __restrict__ Gm) {
   const int j = blockIdx.x * 16 + (threadIdx.x & 15), i = blockIdx.y * 16 + (threadIdx.x >> 4);
   if (i > H || j > H || j < i) return;   // upper triangle; the host mirrors it
   double acc = 0.0;
   for (int o = 0; o < rows; ++o) {
-    const double wi = i < H ? (double)__bfloat162float(Wc[(size_t)o * H + i]) : (double)bc[o];
-    const double wj = j < H ? (double)__bfloat162float(Wc[(size_t)o * H + j]) : (double)bc[o];
+    const double wi = i < H ? (double)__bfloat162float(Wc[(size_t)o * ld + i]) : (double)bc[o];
+    const double wj = j < H ? (double)__bfloat162float(Wc[(size_t)o * ld + j]) : (double)bc[o];
     acc = fma(wi, wj, acc);
   }
   Gm[(size_t)i * (H + 1) + j] = acc;
@@ -440,7 +451,9 @@ struct EpiLnGelu {
   __device__ __forceinline__ const float* warp_vec(int i) const { return i == 0 ? gamma : (i == 1 ? bgamma : beta); }
   const float* part;                    // (M, slots) from EpiRowSq
   int slots;                            // even
-  float c0, inv_rows;                   // constant of the factor, 1 / 4H
+  // constant of the factor, 1 / 4H with the TRUE 4H: at a padded width the GEMM runs N = I columns, but the padded ones have
+  // zc = 0 and gamma = bgamma = beta = 0, so they come out as GELU(0) = 0 and add nothing to the statistics
+  float c0, inv_rows;
   struct RowState {
     float rstd;
   };
@@ -474,10 +487,12 @@ struct EpiLnGelu {
   __device__ __forceinline__ void row_end(int, int, RowState&, int) const {}
 };
 
-// fp32 (rows, cols) -> fp16, same shape (second linear of the node MLP: its A operand is the fp16 intermediate above)
-__global__ void gin_f32_to_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst, size_t total) {
+// fp32 (rows, cols) -> fp16 (rows, cols) with row strides src_ld / dst_ld (second linear of the node MLP: its A operand is the
+// fp16 intermediate above)
+__global__ void gin_f32_to_f16_kernel(const float* __restrict__ src, int src_ld, __half* __restrict__ dst, int dst_ld, int rows, int cols) {
+  const size_t total = (size_t)rows * cols;
   for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x)
-    dst[idx] = __float2half_rn(src[idx]);
+    dst[(idx / cols) * dst_ld + idx % cols] = __float2half_rn(src[(idx / cols) * src_ld + idx % cols]);
 }
 
 // Per-graph pooling over the contiguous node range (graph_encoder/model.py:148,152): max -> bf16 operand of the
@@ -850,11 +865,12 @@ static void launch_softmax_topk(const float* logits, int rows, int W, int ld, in
 // Rows with fewer than k candidates, an overflowing list or a non-finite / zero sum are FLAGGED; the host reads the flag count
 // (the one synchronisation of llb_gin_predictor_topk) and sends flagged rows through the exact materialising path.
 // ---------------------------------------------------------------------------------------------
+// W (rows, K) contiguous -> Wp (cols, K) with row stride ld (the padded head width)
 __global__ void gin_pilot_pack_kernel(const float* __restrict__ W, const float* __restrict__ b, int K, int stride, int cols,
-                                      __nv_bfloat16* __restrict__ Wp, float* __restrict__ bp) {
+                                      __nv_bfloat16* __restrict__ Wp, int ld, float* __restrict__ bp) {
   const int j = blockIdx.x;
   const float* src = W + (size_t)j * stride * K;
-  for (int k = threadIdx.x; k < K; k += blockDim.x) Wp[(size_t)j * K + k] = __float2bfloat16(src[k]);
+  for (int k = threadIdx.x; k < K; k += blockDim.x) Wp[(size_t)j * ld + k] = __float2bfloat16(src[k]);
   if (threadIdx.x == 0) bp[j] = b[(size_t)j * stride];
 }
 
@@ -1079,7 +1095,7 @@ static const int TOPK_CHUNK = 4096;
 
 static int gin_carve(llb_gin* g, void* ws, size_t ws_bytes, int n, int e, int B, bool want_logits, size_t* need) {
   const GinLayout& G = g->G;
-  const size_t H = G.H;
+  const size_t H = G.Hp, I = G.I;
   Arena a(ws, ws_bytes);
   g->x32 = a.take<int32_t>(n), g->batch32 = a.take<int32_t>(n), g->graph_ptr = a.take<int32_t>(B + 1);
   g->rowptr = a.take<int32_t>(n + 1), g->col = a.take<int32_t>(e > 0 ? e : 1), g->eid = a.take<int32_t>(e > 0 ? e : 1);
@@ -1088,12 +1104,12 @@ static int gin_carve(llb_gin* g, void* ws, size_t ws_bytes, int n, int e, int B,
   const int nb = ceil_div(n + 1, 1024);
   g->blk = a.take<int32_t>(nb + 1), g->blk2 = a.take<int32_t>(ceil_div(nb, 1024) + 1);
   g->h = a.take<float>((size_t)n * H), g->hb = a.take<__nv_bfloat16>((size_t)n * H), g->agg = a.take<__nv_bfloat16>((size_t)n * H);
-  g->z = a.take<__nv_bfloat16>((size_t)n * 4 * H);
+  g->z = a.take<__nv_bfloat16>((size_t)n * I);
   g->u = a.take<float>((size_t)n * H);
   g->ln_slots = ceil_div((int)H, 256) * (GEMM_EPI_WARPS / 4);
   g->ln_part = a.take<float>((size_t)n * g->ln_slots);   // analytic LayerNorm statistics
   g->vn_cur = a.take<float>((size_t)B * H), g->vn_next = a.take<float>((size_t)B * H), g->vu = a.take<float>((size_t)B * H);
-  g->pool_b = a.take<__nv_bfloat16>((size_t)B * H), g->vz = a.take<__nv_bfloat16>((size_t)B * 4 * H);
+  g->pool_b = a.take<__nv_bfloat16>((size_t)B * H), g->vz = a.take<__nv_bfloat16>((size_t)B * I);
   if (G.predictor) {
     g->mod = a.take<float>((size_t)G.L * B * 3 * H);
     g->ctext = a.take<__nv_bfloat16>((size_t)B * G.tdim);
@@ -1153,10 +1169,11 @@ static int gin_scan(llb_gin* g, cudaStream_t s) {
 }
 
 static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, size_t b0, size_t lnw, size_t lnb, size_t w4, size_t b4,
-                    int hidden, int out_f, __nv_bfloat16* zbuf, float* out, int out_ld, cudaStream_t s, int slot0 = LLB_PROF_GIN_MISC,
-                    int slot4 = LLB_PROF_GIN_MISC, int gram_layer = -1, bool first_half_only = false) {
-  // Linear -> LayerNorm(hidden) -> GELU -> Linear  (the 4H MLP of GINConv / virtual node / heads)
-  const int H = g->G.H;
+                    int hidden, int hidden_true, int out_f, __nv_bfloat16* zbuf, float* out, int out_ld, cudaStream_t s,
+                    int slot0 = LLB_PROF_GIN_MISC, int slot4 = LLB_PROF_GIN_MISC, int gram_layer = -1, bool first_half_only = false) {
+  // Linear -> LayerNorm(hidden_true) -> GELU -> Linear  (the 4H MLP of GINConv / virtual node / heads); `hidden` is the padded
+  // width of the intermediate, the input width is Hp
+  const int H = g->G.Hp;
   if (gram_layer >= 0) {
     // node MLP with analytic LayerNorm statistics: statistics GEMM (no output matrix) -> first linear with LayerNorm + GELU in
     // its epilogue -> second linear.  The un-normalised 4H-wide intermediate never exists.
@@ -1166,7 +1183,7 @@ static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, si
     LLB_TRY((launch_gemm<256>(in, H, g->w<void>(G.mlp_chol[gram_layer]), H, rows, H, H, es, s, &g->ctr)));
     g->ctr.slot = slot0;
     EpiLnGelu el{zbuf, hidden, g->w<float>(lnw), g->w<float>(G.mlp_bg[gram_layer]), g->w<float>(lnb), g->ln_part, g->ln_slots,
-                 g->chol_c0[gram_layer], 1.0f / (float)hidden};
+                 g->chol_c0[gram_layer], 1.0f / (float)hidden_true};
     LLB_TRY((launch_gemm<256>(in, H, g->w<void>(w0), H, rows, hidden, H, el, s, &g->ctr)));
     g->ctr.slot = slot4;
     if (first_half_only) return LLB_OK;   // the caller fuses the second linear with the layer tail
@@ -1177,7 +1194,7 @@ static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, si
   g->ctr.slot = slot0;
   LLB_TRY(gemm_bias_act(in, H, g->w<void>(w0), H, g->w<float>(b0), zbuf, hidden, rows, hidden, H, LLB_ACT_NONE, false, s, &g->ctr));
   RowLnArgs a;
-  a.in = zbuf, a.in_ld = hidden, a.in_bf16 = true, a.rows = rows, a.width = hidden;
+  a.in = zbuf, a.in_ld = hidden, a.in_bf16 = true, a.rows = rows, a.width = hidden, a.valid = hidden_true;
   a.gamma = g->w<float>(lnw), a.beta = g->w<float>(lnb), a.act = LLB_ACT_GELU;
   a.out_bf16 = zbuf, a.out_bf16_ld = hidden;
   a.prof_slot = LLB_PROF_GIN_ROWLN;
@@ -1187,10 +1204,10 @@ static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, si
   return gemm_bias_act(zbuf, hidden, g->w<void>(w4), hidden, g->w<float>(b4), out, out_ld, rows, out_f, hidden, LLB_ACT_NONE, true, s, &g->ctr);
 }
 
-// Trunk up to the pooled graph vector (B,H).
+// Trunk up to the pooled graph vector (B,H), stored (B,Hp).
 static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
   const GinLayout& G = g->G;
-  const int H = G.H, L = G.L, n = g->n, B = g->B;
+  const int H = G.Hp, L = G.L, n = g->n, B = g->B;   // H: the padded width of every H-wide buffer here
   LLB_CHECK_ARG(n > 0 && B > 0, "gin: no graph batch bound");
   const int eb = (int)(((size_t)n * (H / 4) + 255) / 256 < 8192 ? ((size_t)n * (H / 4) + 255) / 256 : 8192);
   gin_embed_kernel<<<eb, 256, 0, s>>>(g->x32, g->w<float>(G.atom_emb), g->w<float>(G.vn_emb), g->h, g->hb, n, H);
@@ -1226,7 +1243,7 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
     g->launches++;
     // LLB_GIN_FUSED_TAIL=0: second linear + row kernel instead of the fused GEMM + layer-tail kernel (launch_gin_tail)
     static const bool tail_env_off = getenv("LLB_GIN_FUSED_TAIL") && getenv("LLB_GIN_FUSED_TAIL")[0] == '0';
-    const bool fused_tail = !tail_env_off && gin_tail_supported(H, 4 * H);
+    const bool fused_tail = !tail_env_off && G.H == G.Hp && gin_tail_supported(H, G.I);   // the fused tail has no column mask
     if (!last) {
       // virtual node of the next layer from the max-pool of this layer's INPUT (model.py:148 / :343): the fused tail of the
       // previous layer has already accumulated it while it wrote that input; layer 0 (and the unfused path) pool explicitly
@@ -1242,8 +1259,8 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
       }
       LLB_CUDA_OK(cudaGetLastError());
       g->launches++;
-      LLB_TRY(gin_mlp4(g, g->pool_b, B, G.vn0_w[l], G.vn0_b[l], G.vn_ln_w[l], G.vn_ln_b[l], G.vn4_w[l], G.vn4_b[l], 4 * H, H, g->vz,
-                       g->vu, H, s));
+      LLB_TRY(gin_mlp4(g, g->pool_b, B, G.vn0_w[l], G.vn0_b[l], G.vn_ln_w[l], G.vn_ln_b[l], G.vn4_w[l], G.vn4_b[l], G.I, 4 * G.H, H,
+                       g->vz, g->vu, H, s));
       RowLnArgs a;
       a.in = g->vu, a.in_ld = H, a.rows = B, a.width = H, a.normalize = false;
       a.resid = g->vn_cur, a.resid_ld = H, a.out_f32 = g->vn_next, a.out_f32_ld = H;
@@ -1253,8 +1270,8 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
     }
     // LayerNorm + GELU of the node MLP in the first linear's epilogue, from analytic row statistics (see EpiRowSq); the
     // intermediate is fp16 and the second linear multiplies it by the fp16 copy of its weight
-    LLB_TRY(gin_mlp4(g, g->agg, n, G.mlp0_w[l], G.mlp0_b[l], G.mlp_ln_w[l], G.mlp_ln_b[l], G.mlp4_w[l], G.mlp4_b[l], 4 * H, H, g->z,
-                     g->u, H, s, LLB_PROF_GIN_GEMM_MLP0, LLB_PROF_GIN_GEMM_MLP4, l, fused_tail));
+    LLB_TRY(gin_mlp4(g, g->agg, n, G.mlp0_w[l], G.mlp0_b[l], G.mlp_ln_w[l], G.mlp_ln_b[l], G.mlp4_w[l], G.mlp4_b[l], G.I, 4 * G.H, H,
+                     g->z, g->u, H, s, LLB_PROF_GIN_GEMM_MLP0, LLB_PROF_GIN_GEMM_MLP4, l, fused_tail));
     const float* mod = G.predictor ? g->mod + (size_t)l * B * 3 * H : nullptr;
     if (fused_tail) {
       // second linear + LayerNorm + affine / text-adaLN + GELU + gate + residual + next virtual node in ONE kernel; it also
@@ -1271,10 +1288,10 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
       t.pool_max = want_pool ? g->pool_enc : nullptr, t.pool_ld = H;
       t.a_f16 = 1;
       g->ctr.slot = LLB_PROF_GIN_GEMM_MLP4;
-      LLB_TRY(launch_gin_tail(g->z, 4 * H, g->w<void>(G.mlp4_w[l]), 4 * H, n, H, 4 * H, t, g->tail_sync, gemm_ln_pair_workspace_bytes(), s, &g->ctr));
+      LLB_TRY(launch_gin_tail(g->z, G.I, g->w<void>(G.mlp4_w[l]), G.I, n, H, G.I, t, g->tail_sync, gemm_ln_pair_workspace_bytes(), s, &g->ctr));
     } else {
       RowLnArgs a;
-      a.in = g->u, a.in_ld = H, a.rows = n, a.width = H;
+      a.in = g->u, a.in_ld = H, a.rows = n, a.width = H, a.valid = G.H;
       a.row_group = g->batch32;
       if (G.predictor) {
         a.shift = mod, a.scale = mod + H, a.gate = mod + 2 * H, a.mod_ld = 3 * H;
@@ -1319,15 +1336,19 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
   if (packed_bytes < G.total) return fail(LLB_ERR_WORKSPACE, "gin: packed blob needs %zu bytes, got %zu", G.total, packed_bytes);
   cudaStream_t s = (cudaStream_t)stream;
   uint8_t* base = (uint8_t*)packed;
-  const int H = G.H;
+  const int H = G.H, Hp = G.Hp, I = G.I;   // every tensor is written at its true shape into the padded strides (see GinLayout)
   auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(base + off); };
   auto cp = [&](size_t off, const float* src, size_t n) {
     return cudaMemcpyAsync(base + off, src, n * 4, cudaMemcpyDeviceToDevice, s);
   };
-  LLB_CUDA_OK(cp(G.atom_emb, w->atom_emb, (size_t)ATOM_VOCAB * H));
+  auto cp_rows = [&](size_t off, int dst_ld, const float* src, int rows, int cols) {   // (rows, cols) -> row stride dst_ld
+    return cudaMemcpy2DAsync(base + off, (size_t)dst_ld * 4, src, (size_t)cols * 4, (size_t)cols * 4, rows, cudaMemcpyDeviceToDevice, s);
+  };
+  LLB_CUDA_OK(cudaMemsetAsync(base, 0, G.total, s));   // the padding of every parameter is zero
+  LLB_CUDA_OK(cp_rows(G.atom_emb, Hp, w->atom_emb, ATOM_VOCAB, H));
   LLB_CUDA_OK(cp(G.vn_emb, w->vn_emb, H));
   for (int l = 0; l < G.L; ++l) {
-    gin_f32_to_f16_kernel<<<1024, 256, 0, s>>>(w->mlp4_w[l], reinterpret_cast<__half*>(base + G.mlp4_w[l]), (size_t)4 * H * H);   // fp16: see EpiLnGelu
+    gin_f32_to_f16_kernel<<<1024, 256, 0, s>>>(w->mlp4_w[l], 4 * H, reinterpret_cast<__half*>(base + G.mlp4_w[l]), I, H, 4 * H);   // fp16: see EpiLnGelu
     LLB_CUDA_OK(cudaGetLastError());
     LLB_CUDA_OK(cp(G.eps[l], w->eps[l], 1));
     LLB_CUDA_OK(cp(G.mlp_ln_w[l], w->mlp_ln_w[l], 4 * H));
@@ -1336,14 +1357,16 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
     // first linear of the node MLP, CENTRED over its 4H outputs (LayerNorm is shift-invariant; see EpiRowSq), and the Cholesky
     // factor of its augmented Gram matrix for the analytic LayerNorm statistics: fp64 on the host, from the bf16-rounded
     // weight the tensor core multiplies by.  This is the one place where pack_weights synchronises the stream.
+    // At a padded width the centring and the Gram matrix cover the true 4H rows and (H+1) columns only: the padded rows stay 0
+    // (not centred), and a padded Gram matrix would be singular.
     {
       float* wbar = reinterpret_cast<float*>(base + G.chol_scratch);   // scratch doubles as the column-mean buffer first
       gin_colmean_kernel<<<ceil_div(H, 256), 256, 0, s>>>(w->mlp0_w[l], 4 * H, H, wbar);
-      gin_center_weight_kernel<<<1024, 256, 0, s>>>(w->mlp0_w[l], wbar, 4 * H, H, bf(G.mlp0_w[l]));
+      gin_center_weight_kernel<<<1024, 256, 0, s>>>(w->mlp0_w[l], wbar, 4 * H, H, bf(G.mlp0_w[l]), Hp);
       gin_center_bias_kernel<<<1, 1024, 0, s>>>(w->mlp0_b[l], w->mlp_ln_w[l], 4 * H, reinterpret_cast<float*>(base + G.mlp0_b[l]),
                                                  reinterpret_cast<float*>(base + G.mlp_bg[l]));
       double* Gd = reinterpret_cast<double*>(base + G.chol_scratch);
-      gin_gram64_kernel<<<dim3(ceil_div(H + 1, 16), ceil_div(H + 1, 16)), 256, 0, s>>>(bf(G.mlp0_w[l]), reinterpret_cast<const float*>(base + G.mlp0_b[l]),
+      gin_gram64_kernel<<<dim3(ceil_div(H + 1, 16), ceil_div(H + 1, 16)), 256, 0, s>>>(bf(G.mlp0_w[l]), Hp, reinterpret_cast<const float*>(base + G.mlp0_b[l]),
                                                                                       4 * H, H, Gd);
       LLB_CUDA_OK(cudaGetLastError());
       const int n1 = H + 1;
@@ -1351,46 +1374,52 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
       LLB_CUDA_OK(cudaMemcpyAsync(Gh.data(), Gd, Gh.size() * 8, cudaMemcpyDeviceToHost, s));
       LLB_CUDA_OK(cudaStreamSynchronize(s));
       cholesky_lower_host(Gh, n1, Lh);
-      // R[k][i] = L[i][k] (upper factor, k = output row of the statistics GEMM's weight), r[k] = L[H][k], c0 = L[H][H]^2
-      std::vector<__nv_bfloat16> Rb((size_t)H * H);
-      std::vector<float> st(H + 4, 0.f);
+      // R[k][i] = L[i][k] (upper factor, k = output row of the statistics GEMM's weight), r[k] = L[H][k], c0 = L[H][H]^2.
+      // R is stored (Hp, Hp) and r with Hp entries, zero past H; c0 sits at index Hp (EpiRowSq adds r_k to all Hp columns).
+      std::vector<__nv_bfloat16> Rb((size_t)Hp * Hp, __float2bfloat16(0.f));
+      std::vector<float> st(Hp + 4, 0.f);
       for (int k = 0; k < H; ++k) {
-        for (int i = 0; i < H; ++i) Rb[(size_t)k * H + i] = __float2bfloat16(i >= k ? (float)Lh[(size_t)i * n1 + k] : 0.f);
+        for (int i = 0; i < H; ++i) Rb[(size_t)k * Hp + i] = __float2bfloat16(i >= k ? (float)Lh[(size_t)i * n1 + k] : 0.f);
         st[k] = (float)Lh[(size_t)H * n1 + k];
       }
-      st[H] = (float)(Lh[(size_t)H * n1 + H] * Lh[(size_t)H * n1 + H]);
+      st[Hp] = (float)(Lh[(size_t)H * n1 + H] * Lh[(size_t)H * n1 + H]);
       LLB_CUDA_OK(cudaMemcpyAsync(base + G.mlp_chol[l], Rb.data(), Rb.size() * 2, cudaMemcpyHostToDevice, s));
       LLB_CUDA_OK(cudaMemcpyAsync(base + G.mlp_stat[l], st.data(), st.size() * 4, cudaMemcpyHostToDevice, s));
       LLB_CUDA_OK(cudaStreamSynchronize(s));   // Rb / st die with this scope
     }
-    LLB_CUDA_OK(cp(G.bond_emb[l], w->bond_emb[l], (size_t)BOND_VOCAB * H));
+    LLB_CUDA_OK(cp_rows(G.bond_emb[l], Hp, w->bond_emb[l], BOND_VOCAB, H));
     if (!G.predictor) {
       LLB_CHECK_ARG(w->norm_w && w->norm_b, "gin: the encoder needs norms.{l}.weight/bias");
       LLB_CUDA_OK(cp(G.norm_w[l], w->norm_w[l], H));
       LLB_CUDA_OK(cp(G.norm_b[l], w->norm_b[l], H));
     }
     if (l < G.L - 1) {
-      LLB_TRY(launch_f32_to_bf16(w->vn0_w[l], H, bf(G.vn0_w[l]), H, 4 * H, H, H, s));
-      LLB_TRY(launch_f32_to_bf16(w->vn4_w[l], 4 * H, bf(G.vn4_w[l]), 4 * H, H, 4 * H, 4 * H, s));
+      LLB_TRY(launch_f32_to_bf16(w->vn0_w[l], H, bf(G.vn0_w[l]), Hp, 4 * H, H, Hp, s));
+      LLB_TRY(launch_f32_to_bf16(w->vn4_w[l], 4 * H, bf(G.vn4_w[l]), I, H, 4 * H, I, s));
       LLB_CUDA_OK(cp(G.vn0_b[l], w->vn0_b[l], 4 * H));
       LLB_CUDA_OK(cp(G.vn_ln_w[l], w->vn_ln_w[l], 4 * H));
       LLB_CUDA_OK(cp(G.vn_ln_b[l], w->vn_ln_b[l], 4 * H));
       LLB_CUDA_OK(cp(G.vn4_b[l], w->vn4_b[l], H));
     }
     if (G.predictor) {
-      LLB_TRY(launch_f32_to_bf16(w->adapter_w[l], G.tdim, bf(G.adapter_w[l]), G.tdim, 3 * H, G.tdim, G.tdim, s));
-      LLB_CUDA_OK(cp(G.adapter_b[l], w->adapter_b[l], 3 * H));
+      // [shift | scale | gate] as three row blocks of Hp rows: the forward reads them at mod, mod + Hp, mod + 2 Hp
+      for (int b = 0; b < 3; ++b) {
+        LLB_TRY(launch_f32_to_bf16(w->adapter_w[l] + (size_t)b * H * G.tdim, G.tdim, bf(G.adapter_w[l]) + (size_t)b * Hp * G.tdim, G.tdim, H,
+                                   G.tdim, G.tdim, s));
+        LLB_CUDA_OK(cp(G.adapter_b[l] + (size_t)b * Hp * 4, w->adapter_b[l] + (size_t)b * H, H));
+      }
     }
   }
   if (G.predictor) LLB_CUDA_OK(cp(G.text_drop, w->text_dropping, G.tdim));
-  LLB_TRY(launch_f32_to_bf16(w->head0_w, H, bf(G.head0_w), H, G.HH, H, H, s));
-  LLB_TRY(launch_f32_to_bf16(w->head4_w, G.HH, bf(G.head4_w), G.HH, G.HO, G.HH, G.HH, s));
-  LLB_CUDA_OK(cp(G.head0_b, w->head0_b, G.HH));
-  LLB_CUDA_OK(cp(G.head_ln_w, w->head_ln_w, G.HH));
-  LLB_CUDA_OK(cp(G.head_ln_b, w->head_ln_b, G.HH));
-  LLB_CUDA_OK(cp(G.head4_b, w->head4_b, G.HO));
+  const int HOt = G.predictor ? G.out_dim : H;   // true output width of the head
+  LLB_TRY(launch_f32_to_bf16(w->head0_w, H, bf(G.head0_w), Hp, G.HHt, H, Hp, s));
+  LLB_TRY(launch_f32_to_bf16(w->head4_w, G.HHt, bf(G.head4_w), G.HH, HOt, G.HHt, G.HH, s));
+  LLB_CUDA_OK(cp(G.head0_b, w->head0_b, G.HHt));
+  LLB_CUDA_OK(cp(G.head_ln_w, w->head_ln_w, G.HHt));
+  LLB_CUDA_OK(cp(G.head_ln_b, w->head_ln_b, G.HHt));
+  LLB_CUDA_OK(cp(G.head4_b, w->head4_b, HOt));
   if (G.pilot_cols > 0) {
-    gin_pilot_pack_kernel<<<G.pilot_cols, 256, 0, s>>>(w->head4_w, w->head4_b, G.HH, G.pilot_stride, G.pilot_cols, bf(G.pilot_w),
+    gin_pilot_pack_kernel<<<G.pilot_cols, 256, 0, s>>>(w->head4_w, w->head4_b, G.HHt, G.pilot_stride, G.pilot_cols, bf(G.pilot_w), G.HH,
                                                        reinterpret_cast<float*>(base + G.pilot_b));
     LLB_CUDA_OK(cudaGetLastError());
   }
@@ -1412,7 +1441,7 @@ int llb_gin_create(const llb_gin_config* cfg, const void* packed, size_t packed_
   g->blob = (const uint8_t*)packed;
   g->chol_c0.resize(g->G.L);
   for (int l = 0; l < g->G.L; ++l) {   // synchronous: create is not on the hot path
-    cudaError_t e = cudaMemcpy(&g->chol_c0[l], g->blob + g->G.mlp_stat[l] + (size_t)g->G.H * 4, 4, cudaMemcpyDeviceToHost);
+    cudaError_t e = cudaMemcpy(&g->chol_c0[l], g->blob + g->G.mlp_stat[l] + (size_t)g->G.Hp * 4, 4, cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) {
       delete g;
       return fail(LLB_ERR_CUDA, "gin: reading the packed statistics back failed: %s", cudaGetErrorString(e));
@@ -1482,16 +1511,24 @@ int llb_gin_encoder_forward(llb_gin* g, float* out, float* pooled_or_null, llb_s
   LLB_CHECK_ARG(g && out && !g->G.predictor, "llb_gin_encoder_forward: needs an encoder handle and an output buffer");
   cudaStream_t s = (cudaStream_t)stream;
   const GinLayout& G = g->G;
+  const int B = g->B;
   LLB_TRY(gin_trunk(g, nullptr, s));
-  if (pooled_or_null) LLB_CUDA_OK(cudaMemcpyAsync(pooled_or_null, g->pooled, (size_t)g->B * G.H * 4, cudaMemcpyDeviceToDevice, s));
-  LLB_TRY(gin_mlp4(g, g->pooled_b, g->B, G.head0_w, G.head0_b, G.head_ln_w, G.head_ln_b, G.head4_w, G.head4_b, G.HH, G.HO, g->hz,
-                   g->head_out, G.H, s, LLB_PROF_GIN_GEMM_HEAD, LLB_PROF_GIN_GEMM_HEAD));
+  // the caller's (B,H) rows come out of the internal (B,Hp) ones
+  if (pooled_or_null)
+    LLB_CUDA_OK(cudaMemcpy2DAsync(pooled_or_null, (size_t)G.H * 4, g->pooled, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
+  LLB_TRY(gin_mlp4(g, g->pooled_b, B, G.head0_w, G.head0_b, G.head_ln_w, G.head_ln_b, G.head4_w, G.head4_b, G.HH, G.HHt, G.HO, g->hz,
+                   g->head_out, G.Hp, s, LLB_PROF_GIN_GEMM_HEAD, LLB_PROF_GIN_GEMM_HEAD));
+  // L2 normalisation (the padded columns are 0 and add nothing): straight into the caller's rows when the row kernel can write
+  // H columns (H % 4 == 0), else in place at the padded width and a strided copy
+  const bool direct = G.H % 4 == 0;
   RowLnArgs a;
-  a.in = g->head_out, a.in_ld = G.H, a.rows = g->B, a.width = G.H, a.normalize = false, a.l2_normalize = true;
-  a.out_f32 = out, a.out_f32_ld = G.H;
+  a.in = g->head_out, a.in_ld = G.Hp, a.rows = B, a.width = direct ? G.H : G.Hp, a.normalize = false, a.l2_normalize = true;
+  a.out_f32 = direct ? out : g->head_out, a.out_f32_ld = direct ? G.H : G.Hp;
   a.prof_slot = LLB_PROF_GIN_MISC;
   LLB_TRY(launch_row_ln(a, s));
   g->launches++;
+  if (!direct)
+    LLB_CUDA_OK(cudaMemcpy2DAsync(out, (size_t)G.H * 4, g->head_out, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
   return LLB_OK;
 }
 
@@ -1499,10 +1536,10 @@ static int gin_head_hidden(llb_gin* g, cudaStream_t s) {
   // decoder.0 -> LayerNorm -> GELU, result (B,4H) bf16 in g->hz
   const GinLayout& G = g->G;
   g->ctr.slot = LLB_PROF_GIN_GEMM_HEAD;
-  LLB_TRY(gemm_bias_act(g->pooled_b, G.H, g->w<void>(G.head0_w), G.H, g->w<float>(G.head0_b), g->hz, G.HH, g->B, G.HH, G.H,
+  LLB_TRY(gemm_bias_act(g->pooled_b, G.Hp, g->w<void>(G.head0_w), G.Hp, g->w<float>(G.head0_b), g->hz, G.HH, g->B, G.HH, G.Hp,
                         LLB_ACT_NONE, false, s, &g->ctr));
   RowLnArgs a;
-  a.in = g->hz, a.in_ld = G.HH, a.in_bf16 = true, a.rows = g->B, a.width = G.HH;
+  a.in = g->hz, a.in_ld = G.HH, a.in_bf16 = true, a.rows = g->B, a.width = G.HH, a.valid = G.HHt;
   a.gamma = g->w<float>(G.head_ln_w), a.beta = g->w<float>(G.head_ln_b), a.act = LLB_ACT_GELU;
   a.out_bf16 = g->hz, a.out_bf16_ld = G.HH;
   a.prof_slot = LLB_PROF_GIN_ROWLN;

@@ -19,6 +19,7 @@ struct RowLnDev {
   int out_f32_ld;
   __nv_bfloat16* out_bf16;
   int out_bf16_ld, dup_rows, l2_normalize;
+  int valid;   // row_ln_kernel only (the register-resident kernel runs valid == width)
 };
 
 // Compile-time feature mask of the register-resident kernel.  F_RUNTIME keeps every test on the runtime
@@ -46,7 +47,8 @@ __device__ __forceinline__ float act_rt(float x, int act) {
   return x;
 }
 
-// Fallback for widths that are not a multiple of 128: one warp per row, three sweeps over L1/L2.
+// Fallback for widths that are not a multiple of 128, and for rows whose last width - valid columns are padding: one warp per row,
+// three sweeps over L1/L2.  Statistics over the first `valid` columns; the padding columns are written as 0.
 __global__ void __launch_bounds__(256) row_ln_kernel(RowLnDev a) {
   pdl_launch_dependents();
   pdl_wait();
@@ -54,25 +56,26 @@ __global__ void __launch_bounds__(256) row_ln_kernel(RowLnDev a) {
   const int lane = threadIdx.x & 31;
   if (row >= a.rows) return;
   const size_t in_off = (size_t)row * a.in_ld;
-  const int W = a.width;
+  const int W = a.width, V = a.valid;
   float mean = 0.f, rstd = 1.f;
   if (a.normalize || a.l2_normalize) {
     float s = 0.f;
     if (a.normalize) {
       for (int c = lane * 4; c < W; c += 128) {
         const float4 v = load4(a.in, a.in_bf16, in_off + c);
-        s += (v.x + v.y) + (v.z + v.w);
+        s += ((c < V ? v.x : 0.f) + (c + 1 < V ? v.y : 0.f)) + ((c + 2 < V ? v.z : 0.f) + (c + 3 < V ? v.w : 0.f));
       }
-      mean = warp_sum(s) / (float)W;
+      mean = warp_sum(s) / (float)V;
     }
     float q = 0.f;
     for (int c = lane * 4; c < W; c += 128) {
       const float4 v = load4(a.in, a.in_bf16, in_off + c);
-      const float d0 = v.x - mean, d1 = v.y - mean, d2 = v.z - mean, d3 = v.w - mean;
+      const float d0 = c < V ? v.x - mean : 0.f, d1 = c + 1 < V ? v.y - mean : 0.f;
+      const float d2 = c + 2 < V ? v.z - mean : 0.f, d3 = c + 3 < V ? v.w - mean : 0.f;
       q += (d0 * d0 + d1 * d1) + (d2 * d2 + d3 * d3);
     }
     q = warp_sum(q);
-    rstd = a.l2_normalize ? rsqrtf(q) : rsqrtf(q / (float)W + 1e-5f);
+    rstd = a.l2_normalize ? rsqrtf(q) : rsqrtf(q / (float)V + 1e-5f);
   }
   const int g = a.row_group ? a.row_group[row] : row;
   const float* sh = a.shift ? a.shift + (size_t)g * a.mod_ld : nullptr;
@@ -96,7 +99,7 @@ __global__ void __launch_bounds__(256) row_ln_kernel(RowLnDev a) {
       if (gt) x *= __ldg(gt + c + i);
       if (a.resid) x += r[i];
       if (av) x += __ldg(av + c + i);
-      v[i] = x;
+      v[i] = c + i < V ? x : 0.f;
     }
     if (a.out_f32) {
       const float4 o = make_float4(v[0], v[1], v[2], v[3]);
@@ -310,14 +313,17 @@ int launch_row_ln(const RowLnArgs& a, cudaStream_t stream) {
   LLB_CHECK_ARG((a.shift == nullptr) == (a.scale == nullptr), "row_ln: shift and scale come together");
   LLB_CHECK_ARG(a.in_parts >= 1 && (a.in_parts == 1 || (a.width % 128 == 0 && a.in_part_stride % 4 == 0)),
                 "row_ln: summed input parts need a width that is a multiple of 128 (width %d, parts %d)", a.width, a.in_parts);
+  const int valid = a.valid > 0 ? a.valid : a.width;
+  LLB_CHECK_ARG(valid <= a.width && (valid == a.width || a.in_parts == 1), "row_ln: valid=%d outside [1, width=%d] or with summed parts", valid,
+                a.width);
   RowLnDev d{a.in, a.in_ld, a.in_bf16 ? 1 : 0, a.rows, a.width, a.normalize ? 1 : 0, a.in_parts, a.in_part_stride, a.gamma, a.beta, a.row_group,
              a.shift, a.scale, a.gate, a.mod_ld, a.act, a.resid, a.resid_ld, a.addvec, a.addvec_ld, a.out_f32,
-             a.out_f32_ld, a.out_bf16, a.out_bf16_ld, a.dup_rows, a.l2_normalize ? 1 : 0};
+             a.out_f32_ld, a.out_bf16, a.out_bf16_ld, a.dup_rows, a.l2_normalize ? 1 : 0, valid};
   ProfScope prof(a.prof_slot, stream);
   const int grid = ceil_div(a.rows, 8);
   // all vector operands of the register path are read as float4
   const bool vec_ok = a.mod_ld % 4 == 0 && a.addvec_ld % 4 == 0 && a.resid_ld % 4 == 0 && a.out_f32_ld % 4 == 0 && a.out_bf16_ld % 4 == 0;
-  const int nch = (a.width % 128 == 0 && vec_ok) ? a.width / 128 : 0;
+  const int nch = (a.width % 128 == 0 && vec_ok && valid == a.width) ? a.width / 128 : 0;   // padded rows: row_ln_kernel
   unsigned f = 0;
   f |= a.in_bf16 ? F_IN_BF16 : 0, f |= a.normalize ? F_NORM : 0, f |= a.gamma ? F_GAMMA : 0, f |= a.scale ? F_MOD : 0;
   f |= a.act == LLB_ACT_GELU ? F_GELU : 0, f |= a.gate ? F_GATE : 0, f |= a.resid ? F_RESID : 0, f |= a.addvec ? F_ADDVEC : 0;

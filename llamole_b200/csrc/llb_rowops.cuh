@@ -14,6 +14,8 @@ struct RowLnArgs {
   int in_parts = 1;          // the input row is the sum of in_parts pieces, in_part_stride elements apart (split-K partials),
   int in_part_stride = 0;    // added in index order
   int rows = 0, width = 0;
+  int valid = 0;             // columns that carry data (0 = width): the statistics cover [0, valid), columns [valid, width) are
+                             // written as 0 (zero-padded operands of a wider internal width)
   bool normalize = true;
   const float* gamma = nullptr;
   const float* beta = nullptr;
