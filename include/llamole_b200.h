@@ -284,6 +284,25 @@ int llb_gin_predictor_forward(llb_gin* h, const float* c, float* logits, llb_str
  * materialising the logits for the caller.  topk_prob (B,k) fp32, topk_idx (B,k) int32, sorted descending. */
 int llb_gin_predictor_topk(llb_gin* h, const float* c, int k, float* topk_prob, int32_t* topk_idx,
                            llb_stream_t stream);
+/* Backward of GNNRetrosynthsizer.forward with respect to c (the text condition; the parameters are constants).
+ *   llb_gin_grad_packed_bytes / llb_gin_pack_grad_weights: a second, caller-owned blob of transposed bf16 copies of every
+ *     weight the backward multiplies by, built on the device from the handle's packed blob (the predictor head's copy is
+ *     out_dim x 4H: 1.1 GB at 180 576 templates and H = 768).  Only a caller that differentiates needs it.
+ *   llb_gin_saved_bytes / llb_gin_predictor_forward_saved: llb_gin_predictor_forward (the same kernels: bit-identical logits)
+ *     that also stores what the backward needs into the caller's `saved` buffer, including the batch bookkeeping, so a later
+ *     llb_gin_bind on the same handle does not change the gradient.  The buffer also holds the backward's scratch: one buffer
+ *     per forward whose gradient is wanted.
+ *   llb_gin_predictor_backward_c: dlogits (B,out_dim) fp32 -> dc (B,text_dim) fp32, for the forward that filled `saved` (pass
+ *     that forward's batch sizes).  c must be the forward's c; a NULL c is LLB_ERR_INVALID.  Run-to-run bit-identical.
+ * The *_bytes entries reject encoder configs. */
+int llb_gin_grad_packed_bytes(const llb_gin_config* cfg, size_t* bytes);
+int llb_gin_pack_grad_weights(llb_gin* h, void* grad_blob, size_t grad_bytes, llb_stream_t stream);
+int llb_gin_saved_bytes(const llb_gin_config* cfg, int num_nodes, int num_edges, int num_graphs, size_t* bytes);
+int llb_gin_predictor_forward_saved(llb_gin* h, const float* c, float* logits, void* saved, size_t saved_bytes,
+                                    llb_stream_t stream);
+int llb_gin_predictor_backward_c(llb_gin* h, int num_nodes, int num_edges, int num_graphs, const float* c,
+                                 const float* dlogits, void* saved, size_t saved_bytes, const void* grad_blob,
+                                 size_t grad_bytes, float* dc, llb_stream_t stream);
 int64_t llb_gin_launch_count(const llb_gin* h);
 /* Statistics of the last llb_gin_predictor_topk call on this handle: rows that went through the fused head + softmax + top-k
  * kernel, and how many of those fell back to the exact materialising path (expected: none). */

@@ -96,6 +96,11 @@ SIGNATURES = {
     "llb_gin_encoder_forward": (_I, [_P, _P, _P, _P]),
     "llb_gin_predictor_forward": (_I, [_P, _P, _P, _P]),
     "llb_gin_predictor_topk": (_I, [_P, _P, _I, _P, _P, _P]),
+    "llb_gin_grad_packed_bytes": (_I, [C.POINTER(GinConfig), C.POINTER(_SZ)]),
+    "llb_gin_pack_grad_weights": (_I, [_P, _P, _SZ, _P]),
+    "llb_gin_saved_bytes": (_I, [C.POINTER(GinConfig), _I, _I, _I, C.POINTER(_SZ)]),
+    "llb_gin_predictor_forward_saved": (_I, [_P, _P, _P, _P, _SZ, _P]),
+    "llb_gin_predictor_backward_c": (_I, [_P, _I, _I, _I, _P, _P, _P, _SZ, _P, _SZ, _P, _P]),
     "llb_gin_launch_count": (C.c_int64, [_P]),
     "llb_gin_stat": (C.c_int64, [_P, _I]),
     "llb_softmax_topk": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P]),

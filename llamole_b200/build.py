@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "_obj")
 LIB = os.path.join(HERE, "libllamole_b200.so")
-SOURCES = ["llb_runtime.cu", "llb_rowops.cu", "llb_gemm_ln.cu", "llb_dit.cu", "llb_gin.cu"]
+SOURCES = ["llb_runtime.cu", "llb_rowops.cu", "llb_gemm_ln.cu", "llb_dit.cu", "llb_gin.cu", "llb_gin_grad.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

@@ -107,6 +107,10 @@ struct Arena {
 // Device math
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752f)); }
+// d gelu_erf / dx = Phi(x) + x phi(x) (backward passes)
+__device__ __forceinline__ float gelu_erf_grad(float x) {
+  return 0.5f * (1.0f + erff(x * 0.70710678118654752f)) + x * 0.39894228040143268f * expf(-0.5f * x * x);
+}
 // Exact-erf GELU restated as gelu(x) = max(x, 0) - |x| * Phi(-|x|) with Phi(-a) = 2^P(a), P a degree-5 minimax fit
 // of log2(Phi(-a)) on [0, 6] (leading coefficient negative, so P -> -inf and the correction -> 0 beyond the fit range).
 // Max |error| against the fp64 erf form is 6.4e-7 over [-8, 8] (tools/fit_gelu.py), i.e. fp32 round-off of the

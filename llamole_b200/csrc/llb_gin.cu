@@ -8,10 +8,8 @@
 #include <math.h>
 #include <stdlib.h>
 
-#include <vector>
-
-#include "llb_gemm.cuh"
 #include "llb_gemm_ln.cuh"
+#include "llb_gin.cuh"
 #include "llb_rowops.cuh"
 
 namespace llb {
@@ -25,29 +23,7 @@ constexpr int HEAD_PILOT_COLS = 4096;         // strided sample of the templates
 constexpr int HEAD_CAND_CAP = 2048;           // candidates above the threshold kept per row
 constexpr int HEAD_ROW_CHUNK = 8192;          // rows per fused pass: 50 MB of head inputs stay L2-resident while the weight streams once
 
-// Widths.  H is the model's hidden size, any H >= 1.  Every H-wide operand and activation is stored with Hp = round_up(H, 64)
-// columns and every 4H-wide one with I = round_up(4H, 64); the padding of the parameters is zero, so the padded columns of every
-// activation stay exactly 0 through embeddings, GEMMs, biases, GELU (gelu(0) = 0), residuals, pooling and the virtual node.  The
-// only code that must know the true width is the LayerNorm statistics (divide by H / 4H) and the predictor's non-affine
-// LayerNorm, which would otherwise write -mean * rstd into the padded columns (row LayerNorms get `valid` = the true width).
-// When H % 64 == 0, Hp == H and I == 4H.  Below, "(4H,H)" etc. name the true shape and the stored shape is (I,Hp).
-struct GinLayout {
-  int H, Hp, I, L, predictor, out_dim, tdim;
-  int HH, HHt, HO;   // head: hidden width (padded, true), output width (padded: Hp for the encoder, out_dim for the predictor)
-  std::vector<size_t> mlp0_w, mlp4_w, vn0_w, vn4_w, adapter_w;   // bf16
-  std::vector<size_t> mlp_chol;                                    // bf16 (H,H): Cholesky factor of the node MLP's first linear (analytic LayerNorm)
-  std::vector<size_t> mlp_stat;                                    // fp32 [r (Hp, 0 past H) | c0 at Hp, 0, 0, 0]: bias column and constant of that factor
-  std::vector<size_t> mlp_bg;                                      // fp32 (4H): centred bias x LayerNorm gamma
-  size_t chol_scratch;                                             // fp64 (H+1, H+1) Gram matrix (true H), pack time only
-  size_t head0_w, head4_w;
-  size_t pilot_w, pilot_b;     // (pilot_cols, HH) bf16 / (pilot_cols) fp32: every pilot_stride-th template of the head (fused top-k)
-  int pilot_cols, pilot_stride;
-  size_t atom_emb, vn_emb, text_drop;                             // fp32
-  std::vector<size_t> eps, mlp0_b, mlp_ln_w, mlp_ln_b, mlp4_b, bond_emb, norm_w, norm_b;
-  std::vector<size_t> vn0_b, vn_ln_w, vn_ln_b, vn4_b, adapter_b;
-  size_t head0_b, head_ln_w, head_ln_b, head4_b;
-  size_t total;
-};
+}  // namespace
 
 int make_layout(const llb_gin_config& c, GinLayout& G) {
   LLB_CHECK_ARG(c.hidden > 0, "gin: hidden=%d must be positive", c.hidden);
@@ -105,6 +81,8 @@ int make_layout(const llb_gin_config& c, GinLayout& G) {
   G.total = align_up(off, 256);
   return LLB_OK;
 }
+
+namespace {
 
 // ---------------------------------------------------------------------------------------------
 // Graph preparation
@@ -204,6 +182,28 @@ __global__ void gin_sort_rows_kernel(const int32_t* __restrict__ rowptr, int32_t
     }
     eid[b + 1] = ke;
     col[b + 1] = kc;
+  }
+}
+
+// Source-sorted CSR for the predictor's backward (the transpose of the aggregation scatters along out-edges), built from the
+// destination-sorted one so that it holds exactly the edges the forward aggregated (input defects already resolved by
+// gin_fill_kernel).  One thread per destination row: FILL = 0 counts out-degrees, FILL = 1 places (destination, edge id) at
+// the source's rows; gin_sort_rows_kernel then orders every row by edge id.
+template <int FILL>
+__global__ void gin_csr_transpose_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ eid,
+                                         const int32_t* __restrict__ srowptr, int32_t* __restrict__ cnt, int32_t* __restrict__ sdst,
+                                         int32_t* __restrict__ seid, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (int p = rowptr[i]; p < rowptr[i + 1]; ++p) {
+    const int j = col[p];
+    if (FILL) {
+      const int pos = srowptr[j] + atomicAdd(&cnt[j], 1);
+      sdst[pos] = i;
+      seid[pos] = eid[p];
+    } else {
+      atomicAdd(&cnt[j], 1);
+    }
   }
 }
 
@@ -1043,54 +1043,6 @@ __global__ void cost_mlp_kernel(const float* __restrict__ w0, const float* __res
 
 using namespace llb;
 
-struct llb_gin {
-  llb_gin_config cfg;
-  GinLayout G;
-  const uint8_t* blob = nullptr;
-  GemmCounters ctr;
-  int64_t launches = 0;
-  int n = 0, e = 0, B = 0;
-  bool want_logits = false;
-  int32_t *x32 = nullptr, *batch32 = nullptr, *graph_ptr = nullptr, *rowptr = nullptr, *col = nullptr, *eid = nullptr;
-  int32_t *deg = nullptr, *blk = nullptr, *blk2 = nullptr;
-  int32_t* flags = nullptr;   // input-defect bits of the bound batch (LLB_GIN_BAD_*)
-  float* h = nullptr;
-  __nv_bfloat16* hb = nullptr;
-  __nv_bfloat16* agg = nullptr;
-  __nv_bfloat16* z = nullptr;
-  float* u = nullptr;
-  float* ln_part = nullptr;   // (n, ln_slots) partial |zc|^2 sums of the node MLP (analytic LayerNorm)
-  int ln_slots = 0;
-  std::vector<float> chol_c0;   // per layer: constant of the Cholesky factor (host copy)
-  float *vn_cur = nullptr, *vn_next = nullptr, *vu = nullptr;
-  __nv_bfloat16 *pool_b = nullptr, *vz = nullptr;
-  float* mod = nullptr;
-  __nv_bfloat16* ctext = nullptr;
-  float* pooled = nullptr;
-  __nv_bfloat16* pooled_b = nullptr;
-  __nv_bfloat16* hz = nullptr;
-  float* head_out = nullptr;
-  float* logits_ws = nullptr;
-  int32_t* topk_redo = nullptr;   // per row of a logits chunk: redo with the selection-pass kernel
-  // fused head + top-k
-  float* pilot_logits = nullptr;   // (fused rows, HEAD_PILOT_COLS)
-  float2* rowtau = nullptr;        // (fused rows)
-  float* head_part = nullptr;      // (fused rows, head_slots)
-  int head_slots = 0, fused_rows = 0;
-  float2* head_cand = nullptr;     // (fused rows, HEAD_CAND_CAP)
-  int32_t *head_cnt = nullptr, *head_flagged = nullptr, *head_nflag = nullptr;
-  __nv_bfloat16* redo_in = nullptr;   // (chunk_rows, HH) gathered head inputs of flagged rows
-  float* redo_v = nullptr;
-  int32_t* redo_i = nullptr;
-  int max_k = 0;
-  int64_t head_flagged_rows = 0, head_fused_rows = 0;   // statistics of the last llb_gin_predictor_topk call
-  uint32_t* pool_enc = nullptr;   // (B,H) per-graph maxima from the fused layer tail (encoded)
-  void* tail_sync = nullptr;      // statistics-exchange workspace of the fused layer tail
-  int chunk_rows = 0;
-  template <class T>
-  const T* w(size_t off) const { return reinterpret_cast<const T*>(blob + off); }
-};
-
 static const int TOPK_CHUNK = 4096;
 
 static int gin_carve(llb_gin* g, void* ws, size_t ws_bytes, int n, int e, int B, bool want_logits, size_t* need) {
@@ -1143,11 +1095,11 @@ static int gin_carve(llb_gin* g, void* ws, size_t ws_bytes, int n, int e, int B,
   return LLB_OK;
 }
 
-static int gin_scan(llb_gin* g, cudaStream_t s) {
+static int gin_scan(llb_gin* g, const int32_t* deg, int32_t* rowptr, cudaStream_t s) {
   // rowptr[0..n] = exclusive scan of deg[0..n] (deg[n] = 0)
   const int cnt = g->n + 1;
   const int nb = ceil_div(cnt, 1024);
-  scan_block_kernel<<<nb, 1024, 0, s>>>(g->deg, g->rowptr, g->blk, cnt);
+  scan_block_kernel<<<nb, 1024, 0, s>>>(deg, rowptr, g->blk, cnt);
   LLB_CUDA_OK(cudaGetLastError());
   if (nb > 1) {
     const int nb2 = ceil_div(nb, 1024);
@@ -1160,7 +1112,7 @@ static int gin_scan(llb_gin* g, cudaStream_t s) {
       LLB_CUDA_OK(cudaGetLastError());
       g->launches += 2;
     }
-    scan_add_kernel<<<nb, 1024, 0, s>>>(g->rowptr, g->blk, cnt);
+    scan_add_kernel<<<nb, 1024, 0, s>>>(rowptr, g->blk, cnt);
     LLB_CUDA_OK(cudaGetLastError());
     g->launches += 2;
   }
@@ -1168,29 +1120,35 @@ static int gin_scan(llb_gin* g, cudaStream_t s) {
   return LLB_OK;
 }
 
+namespace llb {
+int gin_node_mlp(llb_gin* g, const __nv_bfloat16* in, int rows, int l, float* ln_part, __nv_bfloat16* zbuf, float* u, int u_ld,
+                 bool first_half_only, int slot0, int slot4, cudaStream_t s) {
+  // node MLP with analytic LayerNorm statistics: statistics GEMM (no output matrix) -> first linear with LayerNorm + GELU in
+  // its epilogue -> second linear.  The un-normalised 4H-wide intermediate never exists.
+  const GinLayout& G = g->G;
+  const int H = G.Hp;
+  g->ctr.slot = LLB_PROF_GIN_GEMM_STATS;
+  EpiRowSq es{nullptr, 0, g->w<float>(G.mlp_stat[l]), ln_part, g->ln_slots};
+  LLB_TRY((launch_gemm<256>(in, H, g->w<void>(G.mlp_chol[l]), H, rows, H, H, es, s, &g->ctr)));
+  g->ctr.slot = slot0;
+  EpiLnGelu el{zbuf, G.I, g->w<float>(G.mlp_ln_w[l]), g->w<float>(G.mlp_bg[l]), g->w<float>(G.mlp_ln_b[l]), ln_part, g->ln_slots,
+               g->chol_c0[l], 1.0f / (float)(4 * G.H)};
+  LLB_TRY((launch_gemm<256>(in, H, g->w<void>(G.mlp0_w[l]), H, rows, G.I, H, el, s, &g->ctr)));
+  g->ctr.slot = slot4;
+  if (first_half_only) return LLB_OK;   // the caller fuses the second linear with the layer tail
+  GemmGroups f16;
+  f16.ab_f16 = true;   // fp16 intermediate x fp16 weight
+  return gemm_bias_act(zbuf, G.I, g->w<void>(G.mlp4_w[l]), G.I, g->w<float>(G.mlp4_b[l]), u, u_ld, rows, H, G.I, LLB_ACT_NONE, true, s, &g->ctr, f16);
+}
+}  // namespace llb
+
 static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, size_t b0, size_t lnw, size_t lnb, size_t w4, size_t b4,
                     int hidden, int hidden_true, int out_f, __nv_bfloat16* zbuf, float* out, int out_ld, cudaStream_t s,
                     int slot0 = LLB_PROF_GIN_MISC, int slot4 = LLB_PROF_GIN_MISC, int gram_layer = -1, bool first_half_only = false) {
   // Linear -> LayerNorm(hidden_true) -> GELU -> Linear  (the 4H MLP of GINConv / virtual node / heads); `hidden` is the padded
   // width of the intermediate, the input width is Hp
   const int H = g->G.Hp;
-  if (gram_layer >= 0) {
-    // node MLP with analytic LayerNorm statistics: statistics GEMM (no output matrix) -> first linear with LayerNorm + GELU in
-    // its epilogue -> second linear.  The un-normalised 4H-wide intermediate never exists.
-    const GinLayout& G = g->G;
-    g->ctr.slot = LLB_PROF_GIN_GEMM_STATS;
-    EpiRowSq es{nullptr, 0, g->w<float>(G.mlp_stat[gram_layer]), g->ln_part, g->ln_slots};
-    LLB_TRY((launch_gemm<256>(in, H, g->w<void>(G.mlp_chol[gram_layer]), H, rows, H, H, es, s, &g->ctr)));
-    g->ctr.slot = slot0;
-    EpiLnGelu el{zbuf, hidden, g->w<float>(lnw), g->w<float>(G.mlp_bg[gram_layer]), g->w<float>(lnb), g->ln_part, g->ln_slots,
-                 g->chol_c0[gram_layer], 1.0f / (float)hidden_true};
-    LLB_TRY((launch_gemm<256>(in, H, g->w<void>(w0), H, rows, hidden, H, el, s, &g->ctr)));
-    g->ctr.slot = slot4;
-    if (first_half_only) return LLB_OK;   // the caller fuses the second linear with the layer tail
-    GemmGroups f16;
-    f16.ab_f16 = true;   // fp16 intermediate x fp16 weight
-    return gemm_bias_act(zbuf, hidden, g->w<void>(w4), hidden, g->w<float>(b4), out, out_ld, rows, out_f, hidden, LLB_ACT_NONE, true, s, &g->ctr, f16);
-  }
+  if (gram_layer >= 0) return gin_node_mlp(g, in, rows, gram_layer, g->ln_part, zbuf, out, out_ld, first_half_only, slot0, slot4, s);
   g->ctr.slot = slot0;
   LLB_TRY(gemm_bias_act(in, H, g->w<void>(w0), H, g->w<float>(b0), zbuf, hidden, rows, hidden, H, LLB_ACT_NONE, false, s, &g->ctr));
   RowLnArgs a;
@@ -1204,8 +1162,9 @@ static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, si
   return gemm_bias_act(zbuf, hidden, g->w<void>(w4), hidden, g->w<float>(b4), out, out_ld, rows, out_f, hidden, LLB_ACT_NONE, true, s, &g->ctr);
 }
 
-// Trunk up to the pooled graph vector (B,H), stored (B,Hp).
-static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
+// Trunk up to the pooled graph vector (B,H), stored (B,Hp).  sv != null: also keep what the backward needs (GinSaved); the
+// copies read the buffers the unchanged forward writes, so the computation itself is the same either way.
+static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved* sv = nullptr) {
   const GinLayout& G = g->G;
   const int H = G.Hp, L = G.L, n = g->n, B = g->B;   // H: the padded width of every H-wide buffer here
   LLB_CHECK_ARG(n > 0 && B > 0, "gin: no graph batch bound");
@@ -1223,9 +1182,11 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
     for (int l = 0; l < L; ++l)
       LLB_TRY(gemm_bias_act(g->ctext, G.tdim, g->w<void>(G.adapter_w[l]), G.tdim, g->w<float>(G.adapter_b[l]),
                             g->mod + (size_t)l * B * 3 * H, 3 * H, B, 3 * H, G.tdim, LLB_ACT_NONE, true, s, &g->ctr));
+    if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->mod, g->mod, (size_t)L * B * 3 * H * 4, cudaMemcpyDeviceToDevice, s));
   }
   for (int l = 0; l < L; ++l) {
     const bool last = (l == L - 1);
+    if (sv && l > 0) LLB_CUDA_OK(cudaMemcpyAsync(sv->hin + (size_t)(l - 1) * n * H, g->h, (size_t)n * H * 4, cudaMemcpyDeviceToDevice, s));
     {
       ProfScope prof(LLB_PROF_GIN_AGGREGATE, s);
       const float* be = g->w<float>(G.bond_emb[l]);
@@ -1241,6 +1202,7 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
     }
     LLB_CUDA_OK(cudaGetLastError());
     g->launches++;
+    if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->agg + (size_t)l * n * H, g->agg, (size_t)n * H * 2, cudaMemcpyDeviceToDevice, s));
     // LLB_GIN_FUSED_TAIL=0: second linear + row kernel instead of the fused GEMM + layer-tail kernel (launch_gin_tail)
     static const bool tail_env_off = getenv("LLB_GIN_FUSED_TAIL") && getenv("LLB_GIN_FUSED_TAIL")[0] == '0';
     const bool fused_tail = !tail_env_off && G.H == G.Hp && gin_tail_supported(H, G.I);   // the fused tail has no column mask
@@ -1259,6 +1221,7 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
       }
       LLB_CUDA_OK(cudaGetLastError());
       g->launches++;
+      if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->pool + (size_t)l * B * H, g->pool_b, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
       LLB_TRY(gin_mlp4(g, g->pool_b, B, G.vn0_w[l], G.vn0_b[l], G.vn_ln_w[l], G.vn_ln_b[l], G.vn4_w[l], G.vn4_b[l], G.I, 4 * G.H, H,
                        g->vz, g->vu, H, s));
       RowLnArgs a;
@@ -1314,6 +1277,7 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s) {
   }
   LLB_CUDA_OK(cudaGetLastError());
   g->launches++;
+  if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->pooled_b, g->pooled_b, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
   return LLB_OK;
 }
 
@@ -1488,7 +1452,7 @@ int llb_gin_bind(llb_gin* g, void* workspace, size_t workspace_bytes, int num_no
     gin_degree_kernel<<<ceil_div(e, 256), 256, 0, s>>>(edge_index, edge_attr, g->deg, g->flags, e, n);
     LLB_CUDA_OK(cudaGetLastError());
   }
-  LLB_TRY(gin_scan(g, s));
+  LLB_TRY(gin_scan(g, g->deg, g->rowptr, s));
   LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
   if (e > 0) {
     gin_fill_kernel<<<ceil_div(e, 256), 256, 0, s>>>(edge_index, edge_attr, g->rowptr, g->deg, g->col, g->eid, e, n);
@@ -1555,6 +1519,44 @@ int llb_gin_predictor_forward(llb_gin* g, const float* c, float* logits, llb_str
   LLB_TRY(gin_trunk(g, c, s));
   LLB_TRY(gin_head_hidden(g, s));
   return gemm_bias_act(g->hz, G.HH, g->w<void>(G.head4_w), G.HH, g->w<float>(G.head4_b), logits, G.out_dim, g->B, G.out_dim, G.HH,
+                       LLB_ACT_NONE, true, s, &g->ctr);
+}
+
+int llb_gin_saved_bytes(const llb_gin_config* cfg, int num_nodes, int num_edges, int num_graphs, size_t* bytes) {
+  LLB_CHECK_ARG(cfg && bytes && num_nodes >= 1 && num_edges >= 0 && num_graphs >= 1, "llb_gin_saved_bytes: bad argument");
+  LLB_CHECK_ARG(cfg->predictor, "llb_gin_saved_bytes: only the predictor has a backward");
+  GinLayout G;
+  LLB_TRY(make_layout(*cfg, G));
+  gin_saved_carve(G, nullptr, num_nodes, num_edges, num_graphs, nullptr, bytes);
+  return LLB_OK;
+}
+
+int llb_gin_predictor_forward_saved(llb_gin* g, const float* c, float* logits, void* saved, size_t saved_bytes, llb_stream_t stream) {
+  LLB_CHECK_ARG(g && logits && saved && g->G.predictor, "llb_gin_predictor_forward_saved: needs a predictor handle and output buffers");
+  LLB_CHECK_ARG(g->n > 0 && g->B > 0, "gin: no graph batch bound");
+  cudaStream_t s = (cudaStream_t)stream;
+  const GinLayout& G = g->G;
+  const int n = g->n, e = g->e, B = g->B;
+  GinSaved sv;
+  size_t need = 0;
+  gin_saved_carve(G, saved, n, e, B, &sv, &need);
+  if (saved_bytes < need) return fail(LLB_ERR_WORKSPACE, "gin: saved buffer needs %zu bytes, got %zu", need, saved_bytes);
+  LLB_CUDA_OK(cudaMemcpyAsync(sv.graph_ptr, g->graph_ptr, (size_t)(B + 1) * 4, cudaMemcpyDeviceToDevice, s));
+  LLB_CUDA_OK(cudaMemcpyAsync(sv.batch32, g->batch32, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
+  // source-sorted CSR (the bound batch's degree scratch is free once llb_gin_bind has built the destination CSR)
+  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
+  gin_csr_transpose_kernel<0><<<ceil_div(n, 256), 256, 0, s>>>(g->rowptr, g->col, g->eid, nullptr, g->deg, nullptr, nullptr, n);
+  LLB_CUDA_OK(cudaGetLastError());
+  LLB_TRY(gin_scan(g, g->deg, sv.srowptr, s));
+  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
+  gin_csr_transpose_kernel<1><<<ceil_div(n, 256), 256, 0, s>>>(g->rowptr, g->col, g->eid, sv.srowptr, g->deg, sv.sdst, sv.seid, n);
+  gin_sort_rows_kernel<<<ceil_div(n, 256), 256, 0, s>>>(sv.srowptr, sv.sdst, sv.seid, n);
+  LLB_CUDA_OK(cudaGetLastError());
+  g->launches += 3;
+  // from here on exactly llb_gin_predictor_forward
+  LLB_TRY(gin_trunk(g, c, s, &sv));
+  LLB_TRY(gin_head_hidden(g, s));
+  return gemm_bias_act(g->hz, G.HH, g->w<void>(G.head4_w), G.HH, g->w<float>(G.head4_b), logits, G.out_dim, B, G.out_dim, G.HH,
                        LLB_ACT_NONE, true, s, &g->ctr);
 }
 

@@ -114,6 +114,65 @@ __global__ void __launch_bounds__(256) row_ln_kernel(RowLnDev a) {
   }
 }
 
+// Backward of row_ln_kernel (see RowLnBwdArgs).  Three sweeps over the row: statistics, the two sums of the LayerNorm backward,
+// output.  Any width; columns past `valid` are written as 0.
+__global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
+  const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= a.rows) return;
+  const int W = a.width, V = a.valid;
+  const size_t xo = (size_t)row * a.x_ld, yo = (size_t)row * a.dy_ld;
+  auto xv = [&](int c) {
+    return a.x_bf16 ? __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(a.x)[xo + c]) : reinterpret_cast<const float*>(a.x)[xo + c];
+  };
+  float s = 0.f;
+  for (int c = lane; c < V; c += 32) s += xv(c);
+  const float mean = warp_sum(s) / (float)V;
+  float q = 0.f;
+  for (int c = lane; c < V; c += 32) {
+    const float d = xv(c) - mean;
+    q += d * d;
+  }
+  const float rstd = rsqrtf(warp_sum(q) / (float)V + 1e-5f);
+  const int g = a.row_group ? a.row_group[row] : row;
+  const float* sh = a.shift ? a.shift + (size_t)g * a.mod_ld : nullptr;
+  const float* sc = a.scale ? a.scale + (size_t)g * a.mod_ld : nullptr;
+  const float* gt = a.gate ? a.gate + (size_t)g * a.mod_ld : nullptr;
+  // column c -> xh, dy, dt (gradient at t), and the factor d(t)/d(xh)
+  auto col = [&](int c, float& xh, float& dyv, float& t, float& dt, float& mul) {
+    xh = (xv(c) - mean) * rstd;
+    if (a.gamma) mul = __ldg(a.gamma + c), t = fmaf(xh, mul, __ldg(a.beta + c));
+    else if (sc) mul = 1.0f + __ldg(sc + c), t = fmaf(xh, mul, __ldg(sh + c));
+    else mul = 1.0f, t = xh;
+    dyv = a.dy[yo + c];
+    for (int p = 1; p < a.dy_parts; ++p) dyv += a.dy[yo + (size_t)p * a.dy_part_stride + c];
+    const float da = gt ? dyv * __ldg(gt + c) : dyv;
+    dt = a.gelu ? da * gelu_erf_grad(t) : da;
+  };
+  float s1 = 0.f, s2 = 0.f;
+  for (int c = lane; c < V; c += 32) {
+    float xh, dyv, t, dt, mul;
+    col(c, xh, dyv, t, dt, mul);
+    const float dxh = dt * mul;
+    s1 += dxh, s2 += dxh * xh;
+  }
+  s1 = warp_sum(s1) / (float)V, s2 = warp_sum(s2) / (float)V;
+  for (int c = lane; c < W; c += 32) {
+    float dx = 0.f, p0 = 0.f, p1 = 0.f, p2 = 0.f;
+    if (c < V) {
+      float xh, dyv, t, dt, mul;
+      col(c, xh, dyv, t, dt, mul);
+      dx = rstd * (dt * mul - s1 - xh * s2);
+      p0 = dt, p1 = dt * xh, p2 = dyv * (a.gelu ? gelu_erf(t) : t);
+    }
+    if (a.out_bf16) a.out_bf16[(size_t)row * a.out_ld + c] = __float2bfloat16(dx);
+    if (a.prod) {
+      float* pr = a.prod + (size_t)row * a.prod_ld + c;
+      pr[0] = p0, pr[W] = p1, pr[2 * W] = p2;
+    }
+  }
+}
+
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 
 // Register-resident variant: the row (NCH float4 per lane, width = 128 * NCH) is read from global exactly once.
@@ -347,6 +406,18 @@ int launch_row_ln(const RowLnArgs& a, cudaStream_t stream) {
   }
   if (!done && nch > 0) done = launch_reg<F_RUNTIME>(nch, grid, d, stream);
   if (!done) (void)launch_pdl(row_ln_kernel, dim3(grid), dim3(256), 0, stream, d);
+  LLB_CUDA_OK(cudaGetLastError());
+  return LLB_OK;
+}
+
+int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream) {
+  if (a.rows <= 0) return LLB_OK;
+  LLB_CHECK_ARG(a.x && a.dy && a.valid >= 1 && a.valid <= a.width && a.dy_parts >= 1, "row_ln_bwd: bad argument (width %d, valid %d)",
+                a.width, a.valid);
+  LLB_CHECK_ARG((a.shift == nullptr) == (a.scale == nullptr) && (a.gamma == nullptr) == (a.beta == nullptr) && !(a.gamma && a.scale),
+                "row_ln_bwd: gamma/beta or shift/scale, in pairs");
+  ProfScope prof(a.prof_slot, stream);
+  row_ln_bwd_kernel<<<ceil_div(a.rows, 8), 256, 0, stream>>>(a);
   LLB_CUDA_OK(cudaGetLastError());
   return LLB_OK;
 }

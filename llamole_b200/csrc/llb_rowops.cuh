@@ -39,6 +39,36 @@ struct RowLnArgs {
 };
 int launch_row_ln(const RowLnArgs& a, cudaStream_t stream);
 
+// Backward of the row LayerNorm above without residual / addvec (they pass the gradient through unchanged): with
+//   xh = LN(x) over the first `valid` columns,  t = xh * gamma + beta  or  xh * (1 + scale[g]) + shift[g],  out = gate[g] * act(t),
+// and dy = dL/d(out), writes dx = dL/dx (bf16, 0 in the padded columns) and, when `prod` is set, the per-row products whose
+// per-group sums are the gradients of [shift | scale | gate]: [dt | dt * xh | dy * act(t)] at columns 0, width, 2 width.
+// act is GELU (exact derivative of the erf form) or none.  One warp per row, sums in a fixed order: run-to-run deterministic.
+struct RowLnBwdArgs {
+  const void* x = nullptr;   // the forward's LayerNorm input
+  int x_ld = 0;
+  bool x_bf16 = false;
+  const float* dy = nullptr;
+  int dy_ld = 0;
+  int dy_parts = 1;          // dy is the sum of dy_parts pieces, dy_part_stride elements apart (split-K partials), added in index order
+  int dy_part_stride = 0;
+  int rows = 0, width = 0, valid = 0;
+  const float* gamma = nullptr;
+  const float* beta = nullptr;
+  const int32_t* row_group = nullptr;
+  const float* shift = nullptr;
+  const float* scale = nullptr;
+  const float* gate = nullptr;
+  int mod_ld = 0;
+  bool gelu = false;
+  float* prod = nullptr;
+  int prod_ld = 0;
+  __nv_bfloat16* out_bf16 = nullptr;
+  int out_ld = 0;
+  int prof_slot = LLB_PROF_GIN_ROWLN;
+};
+int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream);
+
 // fp32 (rows, cols) -> bf16 (rows, dst_ld) with zero padding up to pad_cols.
 int launch_f32_to_bf16(const float* src, int src_ld, __nv_bfloat16* dst, int dst_ld, int rows, int cols, int pad_cols,
                        cudaStream_t stream);

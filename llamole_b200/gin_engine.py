@@ -93,6 +93,8 @@ class GinEngine:
             self.handle = h
         self.workspace = None
         self.B = 0
+        self.n = self.e = 0
+        self.grad_blob = None   # transposed weights of the predictor's backward, packed on the first backward
 
     def __del__(self):
         try:
@@ -135,7 +137,7 @@ class GinEngine:
                              (4, "edge endpoint outside [0,num_nodes)"), (8, "bond type outside [0,5)"))
                     what = [msg for bit, msg in names if flags.value & bit]
                     raise IndexError("index out of range in the graph batch: " + "; ".join(what))
-        self.B = B
+        self.B, self.n, self.e = B, n, e
         return B
 
     def encoder_forward(self, want_pooled: bool = False):
@@ -155,6 +157,41 @@ class GinEngine:
             _cabi.check(self.lib.llb_gin_predictor_forward(self.handle, _cabi.ptr(c), _cabi.ptr(logits), _cabi.stream_ptr()),
                         "llb_gin_predictor_forward")
         return logits
+
+    def predictor_forward_saved(self, c: torch.Tensor):
+        """predictor_forward (bit-identical logits) that also returns what predictor_backward_c needs: the `saved` buffer and the
+        batch sizes it was filled for.  The buffer belongs to this call, so several forwards can be back-propagated in any order."""
+        c = c.to(self.device, torch.float32).contiguous()
+        assert c.shape == (self.B, self.text_dim), (c.shape, self.B, self.text_dim)
+        logits = torch.empty((self.B, self.out_dim), dtype=torch.float32, device=self.device)
+        dims = (self.n, self.e, self.B)
+        with torch.cuda.device(self.device):
+            need = C.c_size_t()
+            _cabi.check(self.lib.llb_gin_saved_bytes(C.byref(self.cfg), *dims, C.byref(need)), "llb_gin_saved_bytes")
+            saved = torch.empty(need.value, dtype=torch.uint8, device=self.device)
+            _cabi.check(self.lib.llb_gin_predictor_forward_saved(self.handle, _cabi.ptr(c), _cabi.ptr(logits), _cabi.ptr(saved), need.value,
+                                                                 _cabi.stream_ptr()), "llb_gin_predictor_forward_saved")
+        return logits, saved, dims
+
+    def predictor_backward_c(self, c: torch.Tensor, dlogits: torch.Tensor, saved: torch.Tensor, dims) -> torch.Tensor:
+        """dL/dc (B, text_dim) fp32 from dL/dlogits of the forward that filled `saved` (c: that forward's condition)."""
+        n, e, B = dims
+        c = c.to(self.device, torch.float32).contiguous()
+        dlogits = dlogits.to(self.device, torch.float32).contiguous()
+        assert dlogits.shape == (B, self.out_dim) and c.shape == (B, self.text_dim), (dlogits.shape, c.shape)
+        dc = torch.empty((B, self.text_dim), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            if self.grad_blob is None:
+                need = C.c_size_t()
+                _cabi.check(self.lib.llb_gin_grad_packed_bytes(C.byref(self.cfg), C.byref(need)), "llb_gin_grad_packed_bytes")
+                blob = torch.empty(need.value, dtype=torch.uint8, device=self.device)
+                _cabi.check(self.lib.llb_gin_pack_grad_weights(self.handle, _cabi.ptr(blob), need.value, _cabi.stream_ptr()),
+                            "llb_gin_pack_grad_weights")
+                self.grad_blob = blob
+            _cabi.check(self.lib.llb_gin_predictor_backward_c(self.handle, n, e, B, _cabi.ptr(c), _cabi.ptr(dlogits), _cabi.ptr(saved),
+                                                              saved.numel(), _cabi.ptr(self.grad_blob), self.grad_blob.numel(),
+                                                              _cabi.ptr(dc), _cabi.stream_ptr()), "llb_gin_predictor_backward_c")
+        return dc
 
     def predictor_topk(self, c: Optional[torch.Tensor], k: int):
         probs = torch.empty((self.B, k), dtype=torch.float32, device=self.device)

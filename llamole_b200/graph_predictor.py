@@ -6,10 +6,12 @@ from __future__ import annotations
 import ctypes as C
 import json
 import os
+import warnings
 from collections import defaultdict
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
 from .gin_engine import GinEngine, _Holder, gin_trunk_skeleton, mlp4
@@ -33,6 +35,24 @@ def _template_backend():
     return rdchiralRunText
 
 
+class _LogitsWrtCondition(torch.autograd.Function):
+    """Template logits as a function of c alone: forward = the engine's saved forward, backward = dc on the device."""
+
+    @staticmethod
+    def forward(ctx, c, eng, out_dtype):
+        logits, saved, dims = eng.predictor_forward_saved(c)
+        ctx.eng, ctx.saved, ctx.dims = eng, saved, dims   # the engine (and its blobs) stay alive until this graph is freed
+        ctx.save_for_backward(c)
+        return logits.to(out_dtype)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_logits):
+        (c,) = ctx.saved_tensors
+        dc = ctx.eng.predictor_backward_c(c, grad_logits.float(), ctx.saved, ctx.dims)
+        return dc.to(c.dtype), None, None
+
+
 class GraphPredictor(nn.Module):
     def __init__(self, num_layer, hidden_size, drop_ratio, out_dim, model_config, label_to_template, available=None):
         super().__init__()
@@ -52,6 +72,7 @@ class GraphPredictor(nn.Module):
         self.predictor = pred
         self.neural_cost = None
         self._engine = None
+        self._warned_param_grads = False
 
     # ------------------------------------------------------------------ files
     def init_model(self, model_path, verbose=False):
@@ -109,12 +130,26 @@ class GraphPredictor(nn.Module):
             self._engine.fingerprint = fp
         return self._engine
 
-    @torch.no_grad()
     def forward(self, x, edge_index, edge_attr, batch, c):
-        """Template logits (B,out_dim) (graph_predictor/model.py:306-353); c (B,768) or None."""
-        eng = self.engine()
-        eng.bind(x, edge_index, edge_attr, batch)
-        return eng.predictor_forward(c).to(next(self.predictor.parameters()).dtype)
+        """Template logits (B,out_dim) (graph_predictor/model.py:306-353); c (B,768) or None.
+
+        Differentiable with respect to c when c requires grad and grad mode is on (Llamole's SFT step back-propagates the retro
+        loss through the frozen predictor into the connector): the logits then carry a grad_fn whose backward runs on the
+        device.  The predictor's parameters never receive a gradient."""
+        dtype = next(self.predictor.parameters()).dtype
+        if c is None or not c.requires_grad or not torch.is_grad_enabled():
+            with torch.no_grad():
+                eng = self.engine()
+                eng.bind(x, edge_index, edge_attr, batch)
+                return eng.predictor_forward(c).to(dtype)
+        if not self._warned_param_grads and any(p.requires_grad for p in self.predictor.parameters()):
+            warnings.warn("GraphPredictor: gradients flow to c only; the predictor's parameters receive none "
+                          "(call disable_grads() to freeze them, as the reference loader does)", stacklevel=2)
+            self._warned_param_grads = True
+        with torch.no_grad():
+            eng = self.engine()
+            eng.bind(x, edge_index, edge_attr, batch)
+        return _LogitsWrtCondition.apply(c, eng, dtype)
 
     @torch.no_grad()
     def topk_templates(self, x, edge_index, edge_attr, batch, c, topk):
