@@ -194,6 +194,28 @@ int llb_dit_step(llb_dit* h, int t, uint64_t seed, const float* qX, const float*
 int llb_dit_sample(llb_dit* h, int t_first, int t_last, uint64_t seed, const float* qX_all, const float* qE_all,
                    llb_stream_t stream);
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
+/* Backward of the denoiser with respect to its condition vector c = t_emb + y_emb + txt_emb (B,H) (the SFT loss of
+ * GraphDiT.forward; the parameters are constants).  Uses a handle created with guide_scale == 1 (one pass, no unconditional
+ * half), so a sampler's handle, workspace and captured graph are never touched.
+ *   llb_dit_grad_packed_bytes / llb_dit_pack_grad_weights: a second, caller-owned blob of transposed bf16 copies of every
+ *     weight the backward multiplies by (qkv, proj, fc1, fc2, adaLN.2 of every block, the D+1 adaLN.0 weights stacked along K,
+ *     the output layer's fc1, fc2, adaLN.2), built on the device from the handle's packed blob (~1.1 GB at H = 1024, depth 28).
+ *   llb_dit_train_saved_bytes / llb_dit_denoise_c: one denoiser pass over the int8 states X (B,N), E (B,N,N) of the molecules of
+ *     n_nodes_host[b] atoms with the caller's fp32 c in place of the timestep table + conditions; writes the same masked dense
+ *     logits as llb_dit_denoise (logits_X (B,N,16), logits_E (B,N,N,5), zero outside each molecule; a molecule of 0 atoms is not
+ *     written).  t reaches the denoiser only through c: nothing indexes the schedule.  With `saved` (NULL: inference) it also
+ *     keeps the residual stream at every block-half boundary, the modulations, c and the batch bookkeeping, so a later call on
+ *     the handle cannot change this forward's gradient; the buffer also holds the backward's scratch (one per forward).
+ *   llb_dit_backward_c: dlogits (same shapes, fp32) -> dc (B,H) fp32 for the forward that filled `saved` (pass that forward's
+ *     B and atom total).  Run-to-run bit-identical. */
+int llb_dit_grad_packed_bytes(const llb_dit_config* cfg, size_t* bytes);
+int llb_dit_pack_grad_weights(llb_dit* h, void* grad_blob, size_t grad_bytes, llb_stream_t stream);
+int llb_dit_train_saved_bytes(const llb_dit_config* cfg, int B, int num_tokens, size_t* bytes);
+int llb_dit_denoise_c(llb_dit* h, void* workspace, size_t workspace_bytes, int B, const int32_t* n_nodes_host, const int8_t* X,
+                      const int8_t* E, const float* c, float* logits_X, float* logits_E, void* saved, size_t saved_bytes,
+                      llb_stream_t stream);
+int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t saved_bytes, const void* grad_blob, size_t grad_bytes,
+                       const float* dlogits_X, const float* dlogits_E, float* dc, llb_stream_t stream);
 int64_t llb_dit_launch_count(const llb_dit* h);
 /* Small batches (fewer than 2048 token rows, e.g. the reference's per-prompt batches of 6, modeling_llamole.py:653): from the
  * second denoiser pass of a batch binding on, the t-independent launches of a pass are replayed as one CUDA graph (a launch

@@ -83,6 +83,11 @@ SIGNATURES = {
     "llb_dit_denoise": (_I, [_P, _I, _I, _P, _P, _P]),
     "llb_dit_step": (_I, [_P, _I, C.c_uint64, _P, _P, _P, _P, _P]),
     "llb_dit_sample": (_I, [_P, _I, _I, C.c_uint64, _P, _P, _P]),
+    "llb_dit_grad_packed_bytes": (_I, [C.POINTER(DitConfig), C.POINTER(_SZ)]),
+    "llb_dit_pack_grad_weights": (_I, [_P, _P, _SZ, _P]),
+    "llb_dit_train_saved_bytes": (_I, [C.POINTER(DitConfig), _I, _I, C.POINTER(_SZ)]),
+    "llb_dit_denoise_c": (_I, [_P, _P, _SZ, _I, C.POINTER(C.c_int32), _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "llb_dit_backward_c": (_I, [_P, _I, _I, _P, _SZ, _P, _SZ, _P, _P, _P, _P]),
     "llb_dit_launch_count": (C.c_int64, [_P]),
     "llb_dit_graph_state": (C.c_int, [_P]),
     "llb_dit_posterior_sample": (_I, [_P, _I, _P, _P, _P, _P, C.c_uint64, _P, _P, _P, _P, _P]),

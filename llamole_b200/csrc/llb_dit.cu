@@ -12,31 +12,11 @@
 #define LLB_ATTN_DEFAULT 3
 #endif
 
-#include "llb_dit_kernels.cuh"
-#include "llb_gemm.cuh"
+#include "llb_dit.cuh"
 #include "llb_gemm_ln.cuh"
 #include "llb_rowops.cuh"
 
 namespace llb {
-
-namespace {
-
-struct DitLayout {
-  int H, D, heads, F, N, T, ydim, tdim, d0, K0, KC;
-  // bf16 matrices (byte offsets)
-  size_t x_embed_w, cond_w, ada0_w, out_fc1_w, out_fc2_w, out_ada2_w;
-  std::vector<size_t> qkv_w, proj_w, fc1_w, fc2_w, ada2_w;
-  // fp32 vectors
-  size_t x_ln_w, x_ln_b, ada0_b, out_fc1_b, out_fc2_b, out_ada2_b;
-  std::vector<size_t> qn_w, qn_b, kn_w, kn_b, proj_b, fc1_b, fc2_b, ada2_b;
-  size_t y_mlp0_w, y_mlp0_b, y_drop, txt_drop, txt_b;   // (ydim,H) x3, (H), (H)
-  size_t c1_table;   // (T+1, H): timestep embedding for t = 0..T
-  size_t c_unc;      // (H): sum of the drop embeddings
-  size_t tables;     // x_marg(16) e_marg(5) xe(80) ex(80)
-  size_t betas, abar;  // (T+1) each
-  size_t setup_scratch;  // (T+1, 256 + H) fp32, used by pack_weights only
-  size_t total;
-};
 
 int make_layout(const llb_dit_config& c, DitLayout& L) {
   LLB_CHECK_ARG(c.hidden > 0 && c.hidden % 64 == 0, "dit: hidden=%d must be a positive multiple of 64", c.hidden);
@@ -91,6 +71,8 @@ int make_layout(const llb_dit_config& c, DitLayout& L) {
   L.total = align_up(off, 256);
   return LLB_OK;
 }
+
+namespace {
 
 // timestep features on normalised t = i / T (conditions.py:33-51)
 __global__ void dit_tfeat_kernel(float* __restrict__ feat, int T) {
@@ -187,61 +169,6 @@ __global__ void dit_cond_fixup_kernel(float* __restrict__ cinv, const uint8_t* _
 
 using namespace llb;
 
-struct llb_dit {
-  llb_dit_config cfg;
-  DitLayout L;
-  const uint8_t* blob = nullptr;
-  std::vector<float> betas, abar;   // host copies of the schedule
-  DitTablesDev tables;
-  GemmCounters ctr;
-  int64_t launches = 0;
-  // batch binding
-  int B = 0, Mtok = 0, passes = 2;
-  int64_t mol_base = 0;
-  // workspace carve-up
-  float* x = nullptr;            // (M,H) residual stream fp32
-  __nv_bfloat16* xb = nullptr;   // (M,H) bf16 copy (GEMM A operand)
-  __nv_bfloat16* y = nullptr;    // (M,H)
-  __nv_bfloat16* qkv = nullptr;  // (M,3H)
-  __nv_bfloat16* attn = nullptr; // (M,H)
-  __nv_bfloat16* hbuf = nullptr; // (M,F)  (also fp32 scratch (Mtok,H) for the token embedding)
-  __nv_bfloat16* tok = nullptr;  // (Mtok,K0)
-  float* raw = nullptr;          // (M, raw_ld)
-  int raw_ld = 0;
-  __nv_bfloat16* cvec = nullptr; // (B+1,H)
-  __nv_bfloat16* hid = nullptr;  // (B+1,(D+1)H)
-  float* mod = nullptr;          // (D, B+1, 6H)
-  float* modout = nullptr;       // (B+1, 2 d0)
-  float* part = nullptr;         // (min(2M, 640), SPLITK, H) split-K partial products of fc2
-  float* cinv = nullptr;         // (B,H)
-  __nv_bfloat16* acond = nullptr;  // (B,KC)
-  uint8_t* missing = nullptr;    // (B, ydim+1)
-  int8_t* stX = nullptr;         // (B,N)
-  int8_t* stE = nullptr;         // (B,N,N)
-  int32_t* mol_off = nullptr;    // (B+1)
-  int32_t* row_mol = nullptr;    // (Mtok)
-  int32_t* row_group = nullptr;  // (M): modulation row of each token row
-  void* ln_sync = nullptr;       // statistics-exchange workspace of the CTA-pair GEMM + LayerNorm kernel
-  // Latency regime: everything of a denoiser pass that does not depend on t (all but the conditioning-vector kernel) is captured
-  // once per batch binding and replayed as ONE CUDA graph launch; the programmatic-dependent-launch edges are kept by the capture.
-  cudaGraphExec_t body_graph = nullptr;
-  cudaStream_t capture_stream = nullptr;
-  int graph_state = 0;           // 0 not built, 1 ready, -1 capture / instantiation failed for this binding (eager launches)
-  int passes_run = 0;            // denoiser passes since llb_dit_begin (the first one runs eagerly: lazy one-time set-up is not capturable)
-  int64_t graph_launches = 0;    // kernel launches one replay stands for
-  int64_t graph_kern[LLB_KERN_FAMILIES] = {};
-  void drop_graph() {
-    if (body_graph) cudaGraphExecDestroy(body_graph);
-    body_graph = nullptr, graph_state = 0, passes_run = 0;
-  }
-  ~llb_dit() {
-    drop_graph();
-    if (capture_stream) cudaStreamDestroy(capture_stream);
-  }
-  template <class T>
-  const T* w(size_t off) const { return reinterpret_cast<const T*>(blob + off); }
-};
-
 static size_t dit_step_smem(int N, int passes) {
   const int d0 = DIT_XC + DIT_EC * N;
   return (size_t)passes * N * d0 * 4 + (size_t)passes * N * sizeof(NodeStats) + (size_t)N * DIT_EC * 4 + ((N + 15) & ~15) +
@@ -312,6 +239,12 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
     LLB_TRY(launch_row_ln(a, s));
     h->launches++;
   }
+  // a saved pass (llb_dit_denoise_c) keeps the residual stream at every block-half boundary for its backward
+  auto save_x = [&](int k) -> int {
+    if (h->save_x) LLB_CUDA_OK(cudaMemcpyAsync(h->save_x + (size_t)k * M * H, h->x, (size_t)M * H * 4, cudaMemcpyDeviceToDevice, s));
+    return LLB_OK;
+  };
+  LLB_TRY(save_x(0));
   // 2. all adaLN modulations of this step from the conditioning vector
   ctr->slot = LLB_PROF_GEMM_ADALN;
   const int ldh = (D + 1) * H;
@@ -430,6 +363,7 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
       }
       h->launches++;
     }
+    LLB_TRY(save_x(2 * l + 1));
     ctr->slot = LLB_PROF_GEMM_FC1;
     LLB_TRY(gemm_bias_act(h->xb, H, h->w<void>(L.fc1_w[l]), H, h->w<float>(L.fc1_b[l]), h->hbuf, F, M, F, H, LLB_ACT_GELU, false, s, ctr));
     ctr->slot = LLB_PROF_GEMM_FC2;
@@ -465,6 +399,7 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
       }
       h->launches++;
     }
+    LLB_TRY(save_x(2 * l + 2));
   }
   // 4. output MLP (the LayerNorm / modulation / symmetrisation tail lives in the step kernel)
   ctr->slot = LLB_PROF_GEMM_OTHER;
@@ -571,6 +506,37 @@ static void dit_fill_step(llb_dit* h, DitStepArgs& a, int t) {
   a.guide_scale = h->cfg.guide_scale;
   a.stream_id = (uint32_t)(t - 1);
   a.mol_base = h->mol_base;
+}
+
+// Batch binding shared by llb_dit_begin and llb_dit_denoise_c: workspace carve-up and the varlen row bookkeeping.
+static int dit_bind(llb_dit* h, void* workspace, size_t workspace_bytes, int B, const int32_t* n_nodes_host, int64_t mol_index_base,
+                    cudaStream_t s) {
+  const DitLayout& L = h->L;
+  std::vector<int32_t> off(B + 1, 0);
+  for (int b = 0; b < B; ++b) {
+    LLB_CHECK_ARG(n_nodes_host[b] >= 0 && n_nodes_host[b] <= L.N, "dit: n_nodes[%d]=%d outside [0,%d]", b, n_nodes_host[b], L.N);
+    off[b + 1] = off[b] + n_nodes_host[b];
+  }
+  const int Mtok = off[B];
+  size_t need = 0;
+  LLB_TRY(dit_carve(h, workspace, workspace_bytes, B, Mtok, &need));
+  if (need > workspace_bytes) return fail(LLB_ERR_WORKSPACE, "dit: workspace needs %zu bytes, got %zu", need, workspace_bytes);
+  h->drop_graph();   // the captured launches carry the previous binding's pointers and sizes
+  h->B = B, h->Mtok = Mtok, h->mol_base = mol_index_base;
+  std::vector<int32_t> row_mol(Mtok > 0 ? Mtok : 1), row_group(h->passes * Mtok > 0 ? h->passes * Mtok : 1);
+  for (int b = 0; b < B; ++b)
+    for (int r = off[b]; r < off[b + 1]; ++r) {
+      row_mol[r] = b;
+      row_group[r] = b;
+      if (h->passes == 2) row_group[Mtok + r] = B;
+    }
+  LLB_CUDA_OK(cudaMemcpyAsync(h->mol_off, off.data(), (B + 1) * 4, cudaMemcpyHostToDevice, s));
+  if (Mtok > 0) {
+    LLB_CUDA_OK(cudaMemcpyAsync(h->row_mol, row_mol.data(), (size_t)Mtok * 4, cudaMemcpyHostToDevice, s));
+    LLB_CUDA_OK(cudaMemcpyAsync(h->row_group, row_group.data(), (size_t)h->passes * Mtok * 4, cudaMemcpyHostToDevice, s));
+  }
+  LLB_CUDA_OK(cudaMemsetAsync(h->ln_sync, 0, gemm_ln_pair_workspace_bytes(), s));   // mailbox tags start from a known state
+  return LLB_OK;
 }
 
 extern "C" {
@@ -709,30 +675,7 @@ int llb_dit_begin(llb_dit* h, void* workspace, size_t workspace_bytes, int B, co
   LLB_CHECK_ARG(h && workspace && n_nodes_host && props && txt && B >= 1, "llb_dit_begin: bad argument");
   cudaStream_t s = (cudaStream_t)stream;
   const DitLayout& L = h->L;
-  std::vector<int32_t> off(B + 1, 0);
-  for (int b = 0; b < B; ++b) {
-    LLB_CHECK_ARG(n_nodes_host[b] >= 0 && n_nodes_host[b] <= L.N, "llb_dit_begin: n_nodes[%d]=%d outside [0,%d]", b, n_nodes_host[b], L.N);
-    off[b + 1] = off[b] + n_nodes_host[b];
-  }
-  const int Mtok = off[B];
-  size_t need = 0;
-  LLB_TRY(dit_carve(h, workspace, workspace_bytes, B, Mtok, &need));
-  if (need > workspace_bytes) return fail(LLB_ERR_WORKSPACE, "dit: workspace needs %zu bytes, got %zu", need, workspace_bytes);
-  h->drop_graph();   // the captured launches carry the previous binding's pointers and sizes
-  h->B = B, h->Mtok = Mtok, h->mol_base = mol_index_base;
-  std::vector<int32_t> row_mol(Mtok > 0 ? Mtok : 1), row_group(h->passes * Mtok > 0 ? h->passes * Mtok : 1);
-  for (int b = 0; b < B; ++b)
-    for (int r = off[b]; r < off[b + 1]; ++r) {
-      row_mol[r] = b;
-      row_group[r] = b;
-      if (h->passes == 2) row_group[Mtok + r] = B;
-    }
-  LLB_CUDA_OK(cudaMemcpyAsync(h->mol_off, off.data(), (B + 1) * 4, cudaMemcpyHostToDevice, s));
-  if (Mtok > 0) {
-    LLB_CUDA_OK(cudaMemcpyAsync(h->row_mol, row_mol.data(), (size_t)Mtok * 4, cudaMemcpyHostToDevice, s));
-    LLB_CUDA_OK(cudaMemcpyAsync(h->row_group, row_group.data(), (size_t)h->passes * Mtok * 4, cudaMemcpyHostToDevice, s));
-  }
-  LLB_CUDA_OK(cudaMemsetAsync(h->ln_sync, 0, gemm_ln_pair_workspace_bytes(), s));   // mailbox tags start from a known state
+  LLB_TRY(dit_bind(h, workspace, workspace_bytes, B, n_nodes_host, mol_index_base, s));
   // the copies above read pageable host memory: they have been staged by the time cudaMemcpyAsync returns
   dit_cond_operand_kernel<<<dim3(B, L.ydim + 1), 256, 0, s>>>(props, txt, h->w<float>(L.y_mlp0_w), h->w<float>(L.y_mlp0_b), h->acond,
                                                               h->missing, L.ydim, L.tdim, L.H, L.KC);
@@ -781,6 +724,51 @@ int llb_dit_denoise(llb_dit* h, int t, int unconditioned, float* logits_X, float
   dit_fill_step(h, a, t);
   a.raw = h->raw, a.raw_ld = h->raw_ld, a.modout = h->modout;
   a.sample = 0, a.dump_logits = 1, a.dump_pass = unconditioned ? 1 : 0, a.dumpX = logits_X, a.dumpE = logits_E;
+  return dit_launch_step(h, a, s);
+}
+
+int llb_dit_denoise_c(llb_dit* h, void* workspace, size_t workspace_bytes, int B, const int32_t* n_nodes_host, const int8_t* X,
+                      const int8_t* E, const float* c, float* logits_X, float* logits_E, void* saved, size_t saved_bytes,
+                      llb_stream_t stream) {
+  LLB_CHECK_ARG(h && workspace && n_nodes_host && X && E && c && logits_X && logits_E && B >= 1, "llb_dit_denoise_c: bad argument");
+  LLB_CHECK_ARG(h->passes == 1, "llb_dit_denoise_c: needs a handle created with guide_scale == 1 (one pass)");
+  cudaStream_t s = (cudaStream_t)stream;
+  const DitLayout& L = h->L;
+  const int H = L.H;
+  LLB_TRY(dit_bind(h, workspace, workspace_bytes, B, n_nodes_host, 0, s));
+  const int Mtok = h->Mtok;
+  DitSaved sv{};
+  if (saved) {
+    size_t need = 0;
+    dit_saved_carve(L, saved, B, Mtok, &sv, &need);
+    if (saved_bytes < need) return fail(LLB_ERR_WORKSPACE, "dit: saved buffer needs %zu bytes, got %zu", need, saved_bytes);
+  }
+  LLB_CUDA_OK(cudaMemcpyAsync(h->stX, X, (size_t)B * L.N, cudaMemcpyDeviceToDevice, s));
+  LLB_CUDA_OK(cudaMemcpyAsync(h->stE, E, (size_t)B * L.N * L.N, cudaMemcpyDeviceToDevice, s));
+  // the caller's c replaces cinv + the timestep table; row B (the unconditional row of a guided pass) feeds nothing here
+  LLB_TRY(launch_f32_to_bf16(c, H, h->cvec, H, B, H, H, s));
+  LLB_CUDA_OK(cudaMemsetAsync(h->cvec + (size_t)B * H, 0, (size_t)H * 2, s));
+  h->launches++;
+  if (Mtok > 0) {
+    h->save_x = saved ? sv.xs : nullptr;
+    const int rc = dit_body(h, s);
+    h->save_x = nullptr;
+    LLB_TRY(rc);
+  }
+  if (saved) {
+    LLB_CUDA_OK(cudaMemcpyAsync(sv.mol_off, h->mol_off, (size_t)(B + 1) * 4, cudaMemcpyDeviceToDevice, s));
+    if (Mtok > 0) LLB_CUDA_OK(cudaMemcpyAsync(sv.row_mol, h->row_mol, (size_t)Mtok * 4, cudaMemcpyDeviceToDevice, s));
+    LLB_CUDA_OK(cudaMemcpyAsync(sv.cvec, h->cvec, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
+    LLB_CUDA_OK(cudaMemcpyAsync(sv.mod, h->mod, (size_t)B * L.D * 6 * H * 4, cudaMemcpyDeviceToDevice, s));
+    LLB_CUDA_OK(cudaMemcpyAsync(sv.modout, h->modout, (size_t)B * 2 * L.d0 * 4, cudaMemcpyDeviceToDevice, s));
+  }
+  // the step kernel's logits dump only (no schedule lookup: t reaches the denoiser through c alone)
+  DitStepArgs a{};
+  a.mol_off = h->mol_off;
+  a.B = B, a.N = L.N, a.Mtok = Mtok, a.passes = 1;
+  a.X = h->stX, a.E = h->stE;
+  a.raw = h->raw, a.raw_ld = h->raw_ld, a.modout = h->modout;
+  a.sample = 0, a.dump_logits = 1, a.dump_pass = 0, a.dumpX = logits_X, a.dumpE = logits_E;
   return dit_launch_step(h, a, s);
 }
 

@@ -1,6 +1,7 @@
 // Device kernels of the GraphDiT sampler that are not GEMMs: token one-hot builder, QKV epilogue (per-head
 // LayerNorm), small-sequence attention on mma.sync, and the fused per-molecule step kernel
 // (output-layer LN/modulate/symmetrise -> softmax -> closed-form posterior -> guidance -> categorical sample).
+// The non-template kernels are static: the sampler (llb_dit.cu) and the denoiser's backward (llb_dit_grad.cu) both include this.
 #pragma once
 #include "llb_common.cuh"
 
@@ -55,7 +56,7 @@ struct EpiQKV {
 // Token builder: one-hot joint rows [X_t | E_t row] for the valid tokens (transformer.py:94-95).
 // tok (Mtok, K0) bf16; one warp per token.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) dit_tokens_kernel(const int8_t* __restrict__ X, const int8_t* __restrict__ E,
+static __global__ void __launch_bounds__(256) dit_tokens_kernel(const int8_t* __restrict__ X, const int8_t* __restrict__ E,
                                                          const int32_t* __restrict__ mol_off, const int32_t* __restrict__ row_mol,
                                                          __nv_bfloat16* __restrict__ tok, int Mtok, int N, int K0) {
   const int r = blockIdx.x * 8 + (threadIdx.x >> 5);
@@ -81,7 +82,7 @@ __global__ void __launch_bounds__(256) dit_tokens_kernel(const int8_t* __restric
 }
 
 // c (B+1, H) bf16 = timestep table row t + step-invariant part (cond rows) / drop vector (last row).
-__global__ void dit_cvec_kernel(const float* __restrict__ c1_t, const float* __restrict__ cinv,
+static __global__ void dit_cvec_kernel(const float* __restrict__ c1_t, const float* __restrict__ cinv,
                                 const float* __restrict__ c_unc, __nv_bfloat16* __restrict__ cvec, int B, int H) {
   const int total = (B + 1) * H;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -123,7 +124,7 @@ constexpr int ATTT_TILE = 64 * DIT_DH * 2;   // one 64-row operand tile (8 KB)
 
 __device__ __forceinline__ uint32_t attt_swz(int row, int chunk) { return (uint32_t)(row * 128 + ((chunk ^ (row & 7)) << 4)); }
 
-__global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __grid_constant__ CUtensorMap tmQKV, __nv_bfloat16* __restrict__ out,
+static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __grid_constant__ CUtensorMap tmQKV, __nv_bfloat16* __restrict__ out,
                                                                 const int32_t* __restrict__ mol_off, int B, int Mtok, int H, int heads) {
   pdl_launch_dependents();
   LLB_STAMP(0x1A, 0, threadIdx.x == 0);
@@ -275,7 +276,7 @@ constexpr int ATT4_OFF_BARS = ATT4_STAGES * ATTU_STAGE_BYTES;
 constexpr int ATT4_SMEM = ATT4_OFF_BARS + 512 + 1024;
 constexpr int ATT4_THREADS = (4 * ATT4_GROUPS + 2) * 32;
 
-__global__ void __launch_bounds__(ATT4_THREADS, 1)
+static __global__ void __launch_bounds__(ATT4_THREADS, 1)
 dit_attention_umma4_kernel(const __grid_constant__ CUtensorMap tmQKV, __nv_bfloat16* __restrict__ out, const int32_t* __restrict__ mol_off,
                            int B, int Mtok, int H, int heads, int num_units) {
   extern __shared__ uint8_t att4_raw[];
@@ -526,7 +527,7 @@ __device__ __forceinline__ float post_term(float v, float ux, float p, float pu,
 // THREADS = 256 (two CTAs per SM at throughput batch sizes) or 512 (a handful of molecules: one CTA per molecule is all the
 // parallelism there is, so each gets more threads); every loop strides by blockDim.x.
 template <int THREADS>
-__global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a, const __grid_constant__ DitTablesDev tb) {
+static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a, const __grid_constant__ DitTablesDev tb) {
   LLB_STAMP(0x1C, 0, threadIdx.x == 0);
   extern __shared__ __align__(16) float sm[];
   const int b = blockIdx.x;
@@ -844,7 +845,7 @@ __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a, const 
 
 // z_T from the limit marginals (diffusion_utils.py:495-518): argmax(marg / q); strict upper triangle mirrored,
 // diagonal and masked entries hold no class (-1).
-__global__ void __launch_bounds__(256) dit_init_state_kernel(int8_t* __restrict__ X, int8_t* __restrict__ E,
+static __global__ void __launch_bounds__(256) dit_init_state_kernel(int8_t* __restrict__ X, int8_t* __restrict__ E,
                                                              const int32_t* __restrict__ mol_off, int N, const float* __restrict__ qX0,
                                                              const float* __restrict__ qE0, uint64_t seed, uint32_t stream_id,
                                                              int64_t mol_base, const __grid_constant__ DitTablesDev tb) {

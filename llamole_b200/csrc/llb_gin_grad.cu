@@ -16,6 +16,7 @@
 // is run-to-run bit-identical.  Padded columns (H % 64 != 0) stay exactly 0: the padded weights are 0 and the LayerNorm
 // backward writes 0 past the true width.
 #include "llb_gin.cuh"
+#include "llb_grad.cuh"
 #include "llb_rowops.cuh"
 
 namespace llb {
@@ -56,47 +57,12 @@ void make_grad_layout(const GinLayout& G, GinGradLayout& R) {
   R.total = align_up(off, 256);
 }
 
-__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
-__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
-
-// dst (cols, rows) bf16 with row stride ld_d  <-  src (rows, cols) with row stride ld_s; 32 x 32 tiles through shared memory
-template <class T>
-__global__ void __launch_bounds__(256) gin_grad_transpose_kernel(const T* __restrict__ src, int ld_s, int rows, int cols,
-                                                                 __nv_bfloat16* __restrict__ dst, int ld_d) {
-  __shared__ float tile[32][33];
-  const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32, tx = threadIdx.x, ty = threadIdx.y;
-  for (int k = ty; k < 32; k += 8) {
-    const int r = r0 + k, c = c0 + tx;
-    tile[k][tx] = (r < rows && c < cols) ? to_f32(src[(size_t)r * ld_s + c]) : 0.f;
-  }
-  __syncthreads();
-  for (int k = ty; k < 32; k += 8) {
-    const int c = c0 + k, r = r0 + tx;
-    if (c < cols && r < rows) dst[(size_t)c * ld_d + r] = __float2bfloat16(tile[tx][k]);
-  }
-}
-
 // out (n, W) = rows[batch[i]] (backward of the sum pool)
 __global__ void gin_grad_gather_kernel(const float* __restrict__ rows, const int32_t* __restrict__ batch32, int n, int W,
                                        float* __restrict__ out) {
   const size_t total = (size_t)n * W;
   for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x)
     out[idx] = rows[(size_t)batch32[idx / W] * W + idx % W];
-}
-
-// Per-graph sums over the contiguous node ranges, in node order: out[g] = add[g] + sum_{i in g} in[i] (fp32 and/or bf16 out;
-// add may alias out_f32).  grid (B, ceil(W/256)).
-__global__ void __launch_bounds__(256) gin_grad_segsum_kernel(const float* __restrict__ in, int in_ld, const int32_t* __restrict__ graph_ptr,
-                                                              int W, const float* add, float* out_f32, __nv_bfloat16* __restrict__ out_bf16,
-                                                              int out_ld) {
-  const int g = blockIdx.x;
-  const int c = blockIdx.y * 256 + threadIdx.x;
-  if (c >= W) return;
-  float acc = 0.f;
-  for (int i = graph_ptr[g], end = graph_ptr[g + 1]; i < end; ++i) acc += in[(size_t)i * in_ld + c];
-  if (add) acc += add[(size_t)g * out_ld + c];
-  if (out_f32) out_f32[(size_t)g * out_ld + c] = acc;
-  if (out_bf16) out_bf16[(size_t)g * out_ld + c] = __float2bfloat16(acc);
 }
 
 // Transpose of gin_aggregate_kernel: agg_i = (1 + eps) hb_i + sum_{j->i} gelu(hb_j + bond[e_ji]) with hb = bf16(h_in), so
@@ -224,7 +190,7 @@ int llb_gin_pack_grad_weights(llb_gin* g, void* grad_blob, size_t grad_bytes, ll
   uint8_t* base = (uint8_t*)grad_blob;
   auto dst = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(base + off); };
   auto tr = [&](const auto* src, int ld_s, int rows, int cols, __nv_bfloat16* d, int ld_d) {
-    gin_grad_transpose_kernel<<<dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s>>>(src, ld_s, rows, cols, d, ld_d);
+    grad_transpose_kernel<<<dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s>>>(src, ld_s, rows, cols, d, ld_d);
     g->launches++;
     return cudaGetLastError();
   };
@@ -301,7 +267,7 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
     const float* hin = l > 0 ? sv.hin + (size_t)(l - 1) * n * Hp : nullptr;
     if (!last) {
       // vn_{l+1} is added to every node of h_in_{l+1} and carried into vn_{l+2}
-      gin_grad_segsum_kernel<<<seg_grid_h, 256, 0, s>>>(sv.dh, Hp, sv.graph_ptr, Hp, l < L - 2 ? sv.dvn : nullptr, sv.dvn, sv.dvn_b, Hp);
+      grad_segsum_kernel<<<seg_grid_h, 256, 0, s>>>(sv.dh, Hp, sv.graph_ptr, Hp, l < L - 2 ? sv.dvn : nullptr, sv.dvn, sv.dvn_b, Hp);
       LLB_TRY(kdone());
       if (l > 0) {
         // vn_{l+1} = vn_l + MLP_l(maxpool(h_in_l)): back through the MLP to the pooled row (routed below)
@@ -334,7 +300,7 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
       if (l > 0) a.out_bf16 = sv.du_b, a.out_ld = Hp;
       LLB_TRY(launch_row_ln_bwd(a, s));
       LLB_TRY(kdone());
-      gin_grad_segsum_kernel<<<dim3(B, ceil_div(3 * Hp, 256)), 256, 0, s>>>(sv.prod, 3 * Hp, sv.graph_ptr, 3 * Hp, nullptr, nullptr,
+      grad_segsum_kernel<<<dim3(B, ceil_div(3 * Hp, 256)), 256, 0, s>>>(sv.prod, 3 * Hp, sv.graph_ptr, 3 * Hp, nullptr, nullptr,
                                                                            sv.dmod_b + (size_t)l * 3 * Hp, L * 3 * Hp);
       LLB_TRY(kdone());
     }

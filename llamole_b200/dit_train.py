@@ -1,6 +1,8 @@
 """GraphDiT.forward -- the SFT training loss of the graph decoder (diffusion_model.py:148-250, TrainLossDiscrete :402-438).
 
-NOT the accelerated path.  Training is outside the north-star hot path (SURVEY.md section 8f-4); this module exists so that
+The noisy state, the conditions and the cross-entropy always run here in eager PyTorch.  The denoiser runs on the sm_100a
+kernels (GraphDiT.denoise_on_device, differentiable with respect to the condition vector) when GraphDiT.device_denoiser_ok()
+holds -- a frozen decoder on a B200 -- and as the eager `denoiser_forward` below otherwise.  This module exists so that
 the drop-in class keeps the reference's whole surface: `GraphLLMForCausalMLM.forward` calls
 `graph_decoder(x, edge_index, edge_attr, graph_batch, properties, text_embedding, no_label_index)` during SFT
 (modeling_llamole.py:371-379) and must get the same scalar loss, differentiable with respect to the denoiser's parameters
@@ -194,6 +196,13 @@ def graphdit_loss(model, x, edge_index, edge_attr, graph_batch, properties, text
     X, E, node_mask = to_dense(data_x, edge_index, data_edge_attr, graph_batch, model.max_n_nodes)
     X_t, E_t, t = sample_noisy_state(model, X, E, node_mask)
     mc = model.model_config
-    pX, pE = denoiser_forward(model.denoiser, int(mc.num_heads), X_t.to(dt), E_t.to(dt), node_mask, properties.to(dt).clone(),
-                              text_embedding.to(dt), t, model.denoiser.training, False, float(mc.drop_condition))
+    den, train, drop = model.denoiser, model.denoiser.training, float(mc.drop_condition)
+    y, txt = properties.to(dt).clone(), text_embedding.to(dt)
+    if model.device_denoiser_ok():
+        # conditions in PyTorch (the token embedding before them draws nothing, so the RNG order is the eager path's), the
+        # denoiser c -> logits on the device
+        c = _conditions(den, y, txt, t, train, False, drop)
+        pX, pE = model.denoise_on_device(X_t.to(dt), E_t.to(dt), node_mask, c)
+    else:
+        pX, pE = denoiser_forward(den, int(mc.num_heads), X_t.to(dt), E_t.to(dt), node_mask, y, txt, t, train, False, drop)
     return train_loss(mc.lambda_train, pX, pE, X, E)

@@ -16,6 +16,7 @@ from typing import Callable, List, Optional, Tuple
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
 
@@ -181,12 +182,44 @@ class GraphDiT(nn.Module):
         raise ImportError("check_valid needs the reference's RDKit helpers (graph_decoder/molecule_utils.py)")
 
     def forward(self, x, edge_index, edge_attr, graph_batch, properties, text_embedding, no_label_index):
-        """SFT training loss (diffusion_model.py:148-172; called by modeling_llamole.py:371-379).  NOT accelerated: eager
-        PyTorch (llamole_b200/dit_train.py), differentiable, on the module's own device; same value as the reference for the
-        same torch.manual_seed.  The B200 kernels serve `generate` only (SURVEY.md section 8f-4)."""
+        """SFT training loss (diffusion_model.py:148-172; called by modeling_llamole.py:371-379); same value as the reference for
+        the same torch.manual_seed.  The noisy state, the conditions (dropout, property noise, the text linear) and the
+        cross-entropy are eager PyTorch (llamole_b200/dit_train.py), so torch's RNG is consumed in the reference's order.  The
+        denoiser c -> masked logits runs on the sm_100a kernels, differentiable with respect to c (so text_embedding, the
+        connector and the LLM get their gradient), when the module is on a B200 (`llb_arch_check`), the config is inside the
+        engine's limits and no denoiser parameter requires grad -- the frozen decoder Llamole trains with (`disable_grads()`).
+        Otherwise (CPU, other GPUs, unsupported shapes, a trainable decoder) the whole loss is eager PyTorch on the module's
+        device and the parameters get their gradients too."""
         from .dit_train import graphdit_loss
 
         return graphdit_loss(self, x, edge_index, edge_attr, graph_batch, properties, text_embedding, no_label_index)
+
+    def device_denoiser_ok(self) -> bool:
+        """Whether `forward` runs the denoiser on the sm_100a kernels (see `forward`)."""
+        params = list(self.denoiser.parameters())
+        dev = params[0].device
+        if dev.type != "cuda" or any(p.requires_grad for p in params):
+            return False
+        try:
+            lib = _cabi.lib()
+        except _cabi.LlamoleB200Error:
+            return False
+        idx = dev.index if dev.index is not None else torch.cuda.current_device()
+        nbytes = C.c_size_t()
+        return lib.llb_arch_check(idx) == _cabi.LLB_OK and \
+            lib.llb_dit_packed_bytes(C.byref(_dit_config(self)), C.byref(nbytes)) == _cabi.LLB_OK
+
+    def denoise_on_device(self, X_t, E_t, node_mask, c):
+        """Masked logits (B,N,16), (B,N,N,5) of the one-hot noisy state (X_t, E_t) at condition c (B,H), in the parameters'
+        dtype; differentiable with respect to c when c requires grad."""
+        eng = self.engine()
+        Xs, Es = state_from_onehot(X_t, E_t)
+        n_host = node_mask.sum(dim=1).to("cpu", torch.int32)
+        out_dtype = next(self.denoiser.parameters()).dtype
+        if torch.is_grad_enabled() and c.requires_grad:
+            return _DenoiserWrtCondition.apply(c, eng, Xs, Es, n_host, out_dtype)
+        lX, lE, _ = eng.denoise_c(Xs, Es, n_host, c.detach(), want_saved=False)
+        return lX.to(out_dtype), lE.to(out_dtype)
 
     @torch.no_grad()
     def generate(self, properties, text_embedding, no_label_index) -> List[Optional[str]]:
@@ -264,6 +297,35 @@ class GraphDiT(nn.Module):
         return X.long(), E.long(), n_nodes.to(dev)
 
 
+def _dit_config(model: GraphDiT, guide_scale: Optional[float] = None) -> _cabi.DitConfig:
+    mc = model.model_config
+    if guide_scale is None:
+        guide_scale = 1.0 if model.guide_scale is None else model.guide_scale
+    return _cabi.DitConfig(model.hidden_size, int(mc.depth), int(mc.num_heads), int(model.hidden_size * mc.mlp_ratio),
+                           model.max_n_nodes, model.T, Y_DIM, TEXT_DIM, float(guide_scale))
+
+
+class _DenoiserWrtCondition(torch.autograd.Function):
+    """Denoiser logits as a function of c alone: forward = the engine's saved pass, backward = dc on the device."""
+
+    @staticmethod
+    def forward(ctx, c, eng, Xs, Es, n_host, out_dtype):
+        lX, lE, saved = eng.denoise_c(Xs, Es, n_host, c.detach(), want_saved=True)
+        ctx.eng, ctx.saved, ctx.dims = eng, saved, (int(n_host.numel()), int(n_host.sum()))   # one buffer per forward
+        ctx.c_dtype = c.dtype
+        return lX.to(out_dtype), lE.to(out_dtype)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gX, gE):
+        B, N = ctx.dims[0], ctx.eng.N
+        dev = ctx.eng.device
+        gX = torch.zeros((B, N, X_CLASSES), device=dev) if gX is None else gX.float().contiguous()
+        gE = torch.zeros((B, N, N, E_CLASSES), device=dev) if gE is None else gE.float().contiguous()
+        dc = ctx.eng.backward_c(ctx.saved, ctx.dims, gX, gE)
+        return dc.to(ctx.c_dtype), None, None, None, None, None
+
+
 class _DitEngine:
     """Owns the packed weight blob, the workspace and the C handle for one device."""
 
@@ -274,11 +336,8 @@ class _DitEngine:
         self.device = device
         self.lib = _cabi.lib()
         self.model = model
-        mc = model.model_config
         self.N = model.max_n_nodes
-        self.cfg = _cabi.DitConfig(model.hidden_size, int(mc.depth), int(mc.num_heads), int(model.hidden_size * mc.mlp_ratio),
-                                   self.N, model.T, Y_DIM, TEXT_DIM,
-                                   float(1.0 if model.guide_scale is None else model.guide_scale))
+        self.cfg = _dit_config(model)
         with torch.cuda.device(device):
             _cabi.check(self.lib.llb_arch_check(device.index if device.index is not None else torch.cuda.current_device()),
                         "llb_arch_check")
@@ -291,11 +350,18 @@ class _DitEngine:
             self.handle = h
         self.workspace = None
         self.B = 0
+        # the SFT loss's denoiser (GraphDiT.forward): its own handle on the same blob with guide_scale = 1 (one pass), so the
+        # sampler's binding, workspace and captured graph are never touched; the transposed-weight blob is packed on first use
+        self.train_cfg = _dit_config(model, guide_scale=1.0)
+        self.train_handle = None
+        self.train_workspace = None
+        self.grad_blob = None
 
     def __del__(self):
         try:
-            if getattr(self, "handle", None):
-                self.lib.llb_dit_destroy(self.handle)
+            for h in (getattr(self, "handle", None), getattr(self, "train_handle", None)):
+                if h:
+                    self.lib.llb_dit_destroy(h)
         except Exception:
             pass
 
@@ -406,6 +472,56 @@ class _DitEngine:
                                                           _cabi.ptr(luE), int(seed), _cabi.ptr(qX), _cabi.ptr(qE), _cabi.ptr(pX),
                                                           _cabi.ptr(pE), _cabi.stream_ptr()), "llb_dit_posterior_sample")
         return pX, pE
+
+    def denoise_c(self, Xs: torch.Tensor, Es: torch.Tensor, n_host: torch.Tensor, c: torch.Tensor, want_saved: bool):
+        """Masked logits (fp32) of the int8 states Xs (B,N), Es (B,N,N) of molecules of n_host[b] atoms at condition c (B,H); with
+        want_saved also the buffer backward_c needs (None otherwise)."""
+        B = int(n_host.numel())
+        dev = self.device
+        Xs, Es = Xs.to(dev, torch.int8).contiguous(), Es.to(dev, torch.int8).contiguous()
+        c = c.to(dev, torch.float32).contiguous()
+        lX = torch.zeros((B, self.N, X_CLASSES), dtype=torch.float32, device=dev)
+        lE = torch.zeros((B, self.N, self.N, E_CLASSES), dtype=torch.float32, device=dev)
+        saved = None
+        with torch.cuda.device(dev):
+            if self.train_handle is None:
+                h = C.c_void_p()
+                _cabi.check(self.lib.llb_dit_create(C.byref(self.train_cfg), _cabi.ptr(self.blob), self.blob.numel(), C.byref(h)),
+                            "llb_dit_create")
+                self.train_handle = h
+            need = C.c_size_t()
+            _cabi.check(self.lib.llb_dit_workspace_bytes(C.byref(self.train_cfg), B, C.byref(need)), "llb_dit_workspace_bytes")
+            if self.train_workspace is None or self.train_workspace.numel() < need.value:
+                self.train_workspace = None
+                self.train_workspace = torch.empty(need.value, dtype=torch.uint8, device=dev)
+            if want_saved:
+                sb = C.c_size_t()
+                _cabi.check(self.lib.llb_dit_train_saved_bytes(C.byref(self.train_cfg), B, int(n_host.sum()), C.byref(sb)),
+                            "llb_dit_train_saved_bytes")
+                saved = torch.empty(sb.value, dtype=torch.uint8, device=dev)
+            n_arr = (C.c_int32 * B)(*n_host.tolist())
+            _cabi.check(self.lib.llb_dit_denoise_c(self.train_handle, _cabi.ptr(self.train_workspace), self.train_workspace.numel(), B,
+                                                   n_arr, _cabi.ptr(Xs), _cabi.ptr(Es), _cabi.ptr(c), _cabi.ptr(lX), _cabi.ptr(lE),
+                                                   _cabi.ptr(saved), 0 if saved is None else saved.numel(), _cabi.stream_ptr()),
+                        "llb_dit_denoise_c")
+        return lX, lE, saved
+
+    def backward_c(self, saved: torch.Tensor, dims, dlX: torch.Tensor, dlE: torch.Tensor) -> torch.Tensor:
+        """dL/dc (B,H) fp32 from dL/dlogits of the denoise_c call that filled `saved` (dims = (B, total atoms) of that call)."""
+        B, M = dims
+        dc = torch.empty((B, self.train_cfg.hidden), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            if self.grad_blob is None:
+                need = C.c_size_t()
+                _cabi.check(self.lib.llb_dit_grad_packed_bytes(C.byref(self.train_cfg), C.byref(need)), "llb_dit_grad_packed_bytes")
+                blob = torch.empty(need.value, dtype=torch.uint8, device=self.device)
+                _cabi.check(self.lib.llb_dit_pack_grad_weights(self.train_handle, _cabi.ptr(blob), need.value, _cabi.stream_ptr()),
+                            "llb_dit_pack_grad_weights")
+                self.grad_blob = blob
+            _cabi.check(self.lib.llb_dit_backward_c(self.train_handle, B, M, _cabi.ptr(saved), saved.numel(), _cabi.ptr(self.grad_blob),
+                                                    self.grad_blob.numel(), _cabi.ptr(dlX), _cabi.ptr(dlE), _cabi.ptr(dc),
+                                                    _cabi.stream_ptr()), "llb_dit_backward_c")
+        return dc
 
     def launch_count(self) -> int:
         return int(self.lib.llb_dit_launch_count(self.handle))
