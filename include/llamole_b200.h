@@ -216,6 +216,7 @@ int llb_dit_denoise_c(llb_dit* h, void* workspace, size_t workspace_bytes, int B
                       llb_stream_t stream);
 int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t saved_bytes, const void* grad_blob, size_t grad_bytes,
                        const float* dlogits_X, const float* dlogits_E, float* dc, llb_stream_t stream);
+/* Kernels this handle has issued since it was created, replayed graph nodes included (one replay counts every kernel it runs). */
 int64_t llb_dit_launch_count(const llb_dit* h);
 /* Small batches (fewer than 2048 token rows, e.g. the reference's per-prompt batches of 6, modeling_llamole.py:653): from the
  * second denoiser pass of a batch binding on, the t-independent launches of a pass are replayed as one CUDA graph (a launch
@@ -325,6 +326,7 @@ int llb_gin_predictor_forward_saved(llb_gin* h, const float* c, float* logits, v
 int llb_gin_predictor_backward_c(llb_gin* h, int num_nodes, int num_edges, int num_graphs, const float* c,
                                  const float* dlogits, void* saved, size_t saved_bytes, const void* grad_blob,
                                  size_t grad_bytes, float* dc, llb_stream_t stream);
+/* Kernels this handle has issued since it was created. */
 int64_t llb_gin_launch_count(const llb_gin* h);
 /* Statistics of the last llb_gin_predictor_topk call on this handle: rows that went through the fused head + softmax + top-k
  * kernel, and how many of those fell back to the exact materialising path (expected: none). */

@@ -41,14 +41,15 @@ int fail(int code, const char* fmt, ...);
 int num_sms();
 int require_sm100();  // LLB_OK or LLB_ERR_ARCH (no fallback by design)
 
-// Event bracket around one kernel launch (no-op unless llb_profile_enable(1)).
+// Event bracket around one kernel launch, or a group of them (no-op unless llb_profile_enable(1), and for NO_PROF).
+constexpr int NO_PROF = -1;   // a launch charged to no profiling slot
 bool profile_on();
 void profile_begin(int slot, cudaStream_t s);
 void profile_end(cudaStream_t s);
 struct ProfScope {
   cudaStream_t s;
   bool on;
-  ProfScope(int slot, cudaStream_t stream) : s(stream), on(profile_on()) {
+  ProfScope(int slot, cudaStream_t stream) : s(stream), on(slot != NO_PROF && profile_on()) {
     if (on) profile_begin(slot, s);
   }
   ~ProfScope() {
@@ -58,31 +59,54 @@ struct ProfScope {
 
 void note_kernel(int family, int64_t n = 1);   // llb_kernel_launches counters (n < 0: a stream capture issued nothing)
 
+// The kernels a handle issued (llb_*_launch_count), and the profiling slot its GEMM launchers charge.
+struct LaunchCounter {
+  int64_t launches = 0;
+  int slot = LLB_PROF_GEMM_OTHER;
+};
+
 // Programmatic dependent launch: the kernel may start while its predecessor in the stream still runs; whatever it does before
 // pdl_wait() (barrier init, TMEM allocation, descriptor prefetch, loads of WEIGHTS) overlaps the predecessor's tail.  Every access
 // to data a predecessor produced (or still reads) comes after pdl_wait(), which returns once all prerequisite grids have completed
 // and flushed.  Kernels launched the ordinary way execute both instructions as no-ops.
 bool pdl_enabled();   // LLB_PDL=0 launches everything the ordinary way (A-B comparison)
 template <class T>
-struct pdl_ident {
+struct kernel_arg {
   using type = T;
 };
-// Set to make the NEXT launch_pdl of this thread an ordinary launch (a full dependency on everything before it in the stream):
-// what some later kernel reads AHEAD of its own dependency wait must have been produced before such a launch.
+// Set to make the NEXT programmatic launch of this thread an ordinary launch (a full dependency on everything before it in the
+// stream): what some later kernel reads AHEAD of its own dependency wait must have been produced before such a launch.
 inline bool& pdl_full_barrier_next() {
   static thread_local bool flag = false;
   return flag;
 }
+// Raises the kernel's dynamic shared-memory limit to at least `smem` bytes (once per kernel and size).
+int reserve_dynamic_smem(const void* kern, size_t smem);
+// LLB_ERR_CUDA naming the kernel whose launch returned `e`.
+int launch_failed(const void* kern, cudaError_t e);
+
+// Every kernel of the library except the cooperative GEMM + LayerNorm launches (llb_gemm_ln.cu) goes through here: profiling
+// record (prof_slot), the programmatic-serialisation attribute (pdl: only for kernels that call pdl_wait() before touching their
+// predecessors' data), dynamic shared memory above the 48 KB default, the launch's status, and one count on ctr (may be null)
+// when it was issued.
 template <class... KArgs>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, typename pdl_ident<KArgs>::type... args) {
+int launch_kernel(LaunchCounter* ctr, int prof_slot, bool pdl, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
+                  typename kernel_arg<KArgs>::type... args) {
+  if (smem > 48 * 1024) LLB_TRY(reserve_dynamic_smem((const void*)kern, smem));
+  ProfScope prof(prof_slot, s);
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = s;
-  cfg.attrs = attr, cfg.numAttrs = (pdl_enabled() && !pdl_full_barrier_next()) ? 1 : 0;
-  pdl_full_barrier_next() = false;
-  return cudaLaunchKernelEx(&cfg, kern, args...);
+  cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = s, cfg.attrs = attr;
+  if (pdl) {
+    cfg.numAttrs = (pdl_enabled() && !pdl_full_barrier_next()) ? 1 : 0;
+    pdl_full_barrier_next() = false;
+  }
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+  if (e != cudaSuccess) return launch_failed((const void*)kern, e);
+  if (ctr) ctr->launches++;
+  return LLB_OK;
 }
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }

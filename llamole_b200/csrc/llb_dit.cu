@@ -218,14 +218,10 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
   const DitLayout& L = h->L;
   const int H = L.H, F = L.F, D = L.D, B = h->B, Mtok = h->Mtok;
   const int M = h->passes * Mtok;
-  GemmCounters* ctr = &h->ctr;
+  LaunchCounter* ctr = &h->ctr;
   // 1. tokens -> embedding -> LayerNorm (shared by both halves)
-  {
-    ProfScope prof(LLB_PROF_DIT_MISC, s);
-    dit_tokens_kernel<<<ceil_div(Mtok, 8), 256, 0, s>>>(h->stX, h->stE, h->mol_off, h->row_mol, h->tok, Mtok, L.N, L.K0);
-  }
-  LLB_CUDA_OK(cudaGetLastError());
-  h->launches++;
+  LLB_TRY(launch_kernel(ctr, LLB_PROF_DIT_MISC, false, dit_tokens_kernel, dim3(ceil_div(Mtok, 8)), dim3(256), 0, s, h->stX, h->stE, h->mol_off,
+                        h->row_mol, h->tok, Mtok, L.N, L.K0));
   ctr->slot = LLB_PROF_GEMM_OTHER;
   float* emb = reinterpret_cast<float*>(h->hbuf);
   LLB_TRY(gemm_bias_act(h->tok, L.K0, h->w<void>(L.x_embed_w), L.K0, nullptr, emb, H, Mtok, H, L.K0, LLB_ACT_NONE, true, s, ctr));
@@ -236,8 +232,7 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
     a.out_f32 = h->x, a.out_f32_ld = H, a.out_bf16 = h->xb, a.out_bf16_ld = H;
     a.dup_rows = h->passes == 2 ? Mtok : 0;
     a.prof_slot = LLB_PROF_DIT_MISC;
-    LLB_TRY(launch_row_ln(a, s));
-    h->launches++;
+    LLB_TRY(launch_row_ln(a, s, ctr));
   }
   // a saved pass (llb_dit_denoise_c) keeps the residual stream at every block-half boundary for its backward
   auto save_x = [&](int k) -> int {
@@ -279,17 +274,8 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
   // (other widths have no fused kernel: a full row must fit four pairs' tensor memory).
   // LLB_ATTN=2: tcgen05 attention (two heads per 128-row tile, P in tensor memory; needs an even head count); default: mma.sync
   // attention fed by TMA.
-  static int attn_env = -1;
-  if (attn_env < 0) {
-    const char* v = getenv("LLB_ATTN");
-    int mode = (v && v[0] == '2') ? 2 : 3;
-    if (mode == 2 && cudaFuncSetAttribute(dit_attention_umma4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT4_SMEM) != cudaSuccess) {
-      (void)cudaGetLastError();
-      mode = 3;
-    }
-    attn_env = mode;
-  }
-  const bool attn_umma = attn_env == 2 && L.heads % 2 == 0;
+  static const bool attn_umma_env = getenv("LLB_ATTN") && getenv("LLB_ATTN")[0] == '2';
+  const bool attn_umma = attn_umma_env && L.heads % 2 == 0;
   const bool fused_pair = fused_ln;
   const size_t part_rows = (size_t)(M < 640 ? M : 640) * LLB_DIT_SPLITK;   // rows x slices the split-K buffer h->part holds (dit_carve)
   const size_t ln_sync_bytes = gemm_ln_pair_workspace_bytes();
@@ -314,18 +300,15 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
       const int seqs = (share0 ? 1 : h->passes) * B;
       CUtensorMap tmQKV;
       LLB_TRY(make_tensor_map_2d(&tmQKV, h->qkv, 2, seqs / B * Mtok, 3 * H, 3 * H, DIT_DH, 64, 128));
-      ProfScope prof(LLB_PROF_ATTENTION, s);
       if (attn_umma) {
         const int units = seqs * (L.heads / 2);
-        dit_attention_umma4_kernel<<<units < num_sms() ? units : num_sms(), ATT4_THREADS, ATT4_SMEM, s>>>(tmQKV, h->attn, h->mol_off, B, Mtok, H,
-                                                                                                          L.heads, units);
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, false, dit_attention_umma4_kernel, dim3(units < num_sms() ? units : num_sms()),
+                              dim3(ATT4_THREADS), ATT4_SMEM, s, tmQKV, h->attn, h->mol_off, B, Mtok, H, L.heads, units));
       } else {
-        LLB_CUDA_OK(launch_pdl(dit_attention_tma_kernel, dim3((unsigned)(seqs * L.heads)), dim3(128), 0, s, tmQKV, h->attn, (const int32_t*)h->mol_off, B, Mtok, H,
-                               L.heads));
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel, dim3((unsigned)(seqs * L.heads)), dim3(128), 0, s, tmQKV,
+                              h->attn, h->mol_off, B, Mtok, H, L.heads));
       }
     }
-    LLB_CUDA_OK(cudaGetLastError());
-    h->launches++;
     // x += gate * (LN(linear(.)) (1 + scale) + shift): fused into the GEMM epilogue when a cluster can hold a full row
     RowLnArgs a;
     a.in = h->y, a.in_ld = H, a.in_bf16 = true, a.rows = M, a.width = H;
@@ -355,13 +338,12 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
         RowLnArgs ap = a;
         ap.in = h->part, ap.in_ld = 2 * H, ap.in_bf16 = false, ap.in_parts = 2, ap.in_part_stride = H;
         ap.shift = mod, ap.scale = mod + H, ap.gate = mod + 2 * H;
-        LLB_TRY(launch_row_ln(ap, s));
+        LLB_TRY(launch_row_ln(ap, s, ctr));
       } else {
         LLB_TRY(gemm_bias_act(h->attn, H, h->w<void>(L.proj_w[l]), H, h->w<float>(L.proj_b[l]), h->y, H, M, H, H, LLB_ACT_NONE, false, s, ctr));
         a.shift = mod, a.scale = mod + H, a.gate = mod + 2 * H;
-        LLB_TRY(launch_row_ln(a, s));
+        LLB_TRY(launch_row_ln(a, s, ctr));
       }
-      h->launches++;
     }
     LLB_TRY(save_x(2 * l + 1));
     ctr->slot = LLB_PROF_GEMM_FC1;
@@ -391,13 +373,12 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
         RowLnArgs ap = a;
         ap.in = h->part, ap.in_ld = parts * H, ap.in_bf16 = false, ap.in_parts = parts, ap.in_part_stride = H;
         ap.shift = mod + 3 * H, ap.scale = mod + 4 * H, ap.gate = mod + 5 * H;
-        LLB_TRY(launch_row_ln(ap, s));
+        LLB_TRY(launch_row_ln(ap, s, ctr));
       } else {
         LLB_TRY(gemm_bias_act(h->hbuf, F, h->w<void>(L.fc2_w[l]), F, h->w<float>(L.fc2_b[l]), h->y, H, M, H, F, LLB_ACT_NONE, false, s, ctr));
         a.shift = mod + 3 * H, a.scale = mod + 4 * H, a.gate = mod + 5 * H;
-        LLB_TRY(launch_row_ln(a, s));
+        LLB_TRY(launch_row_ln(a, s, ctr));
       }
-      h->launches++;
     }
     LLB_TRY(save_x(2 * l + 2));
   }
@@ -425,7 +406,7 @@ static int dit_build_graph(llb_dit* h) {
   }
   int64_t kern0[LLB_KERN_FAMILIES];
   for (int f = 0; f < LLB_KERN_FAMILIES; ++f) kern0[f] = llb_kernel_launches(f);
-  const int64_t own0 = h->launches, gemm0 = h->ctr.launches;
+  const int64_t launches0 = h->ctr.launches;
   if (cudaStreamBeginCapture(h->capture_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
     (void)cudaGetLastError();
     return LLB_OK;
@@ -433,9 +414,9 @@ static int dit_build_graph(llb_dit* h) {
   const int rc = dit_body(h, h->capture_stream);
   cudaGraph_t g = nullptr;
   const cudaError_t e = cudaStreamEndCapture(h->capture_stream, &g);
-  // the capture issued nothing: take its launches back out of the counters, replays add them
-  h->graph_launches = (h->launches - own0) + (h->ctr.launches - gemm0);
-  h->launches = own0, h->ctr.launches = gemm0;
+  // the capture issued nothing: take its launches back out of the counter, replays add them
+  h->graph_launches = h->ctr.launches - launches0;
+  h->ctr.launches = launches0;
   for (int f = 0; f < LLB_KERN_FAMILIES; ++f) {
     h->graph_kern[f] = llb_kernel_launches(f) - kern0[f];
     note_kernel(f, -h->graph_kern[f]);
@@ -460,19 +441,14 @@ static int dit_build_graph(llb_dit* h) {
 static int dit_forward(llb_dit* h, int t, cudaStream_t s) {
   const DitLayout& L = h->L;
   if (h->Mtok == 0) return LLB_OK;
-  {
-    ProfScope prof(LLB_PROF_DIT_MISC, s);
-    dit_cvec_kernel<<<ceil_div((h->B + 1) * L.H, 256), 256, 0, s>>>(h->w<float>(L.c1_table) + (size_t)t * L.H, h->cinv, h->w<float>(L.c_unc),
-                                                                  h->cvec, h->B, L.H);
-  }
-  LLB_CUDA_OK(cudaGetLastError());
-  h->launches++;
+  LLB_TRY(launch_kernel(&h->ctr, LLB_PROF_DIT_MISC, false, dit_cvec_kernel, dim3(ceil_div((h->B + 1) * L.H, 256)), dim3(256), 0, s,
+                        h->w<float>(L.c1_table) + (size_t)t * L.H, h->cinv, h->w<float>(L.c_unc), h->cvec, h->B, L.H));
   const bool want_graph = dit_latency_regime(h) && dit_graph_enabled() && !profile_on() && h->passes_run >= 1;
   h->passes_run++;
   if (want_graph && h->graph_state == 0) LLB_TRY(dit_build_graph(h));
   if (want_graph && h->graph_state == 1) {
     LLB_CUDA_OK(cudaGraphLaunch(h->body_graph, s));
-    h->launches += h->graph_launches;
+    h->ctr.launches += h->graph_launches;
     for (int f = 0; f < LLB_KERN_FAMILIES; ++f) note_kernel(f, h->graph_kern[f]);
     return LLB_OK;
   }
@@ -481,20 +457,9 @@ static int dit_forward(llb_dit* h, int t, cudaStream_t s) {
 
 static int dit_launch_step(llb_dit* h, DitStepArgs& a, cudaStream_t s) {
   const size_t smem = dit_step_smem(h->L.N, a.passes);
-  static size_t configured = 0;
-  if (smem > configured) {
-    LLB_CUDA_OK(cudaFuncSetAttribute(dit_step_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LLB_CUDA_OK(cudaFuncSetAttribute(dit_step_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
-  {
-    ProfScope prof(LLB_PROF_DIT_STEP, s);
-    if (h->B <= num_sms()) dit_step_kernel<512><<<h->B, 512, smem, s>>>(a, h->tables);   // fewer molecules than SMs: wider CTAs
-    else dit_step_kernel<256><<<h->B, 256, smem, s>>>(a, h->tables);
-  }
-  LLB_CUDA_OK(cudaGetLastError());
-  h->launches++;
-  return LLB_OK;
+  if (h->B <= num_sms())   // fewer molecules than SMs: wider CTAs
+    return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<512>, dim3(h->B), dim3(512), smem, s, a, h->tables);
+  return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<256>, dim3(h->B), dim3(256), smem, s, a, h->tables);
 }
 
 static void dit_fill_step(llb_dit* h, DitStepArgs& a, int t) {
@@ -564,18 +529,18 @@ int llb_dit_pack_weights(const llb_dit_config* cfg, const llb_dit_weights* w, vo
   auto cp = [&](size_t off, const float* src, size_t n) {
     return cudaMemcpyAsync(base + off, src, n * 4, cudaMemcpyDeviceToDevice, s);
   };
-  LLB_TRY(launch_f32_to_bf16(w->x_embed_w, L.d0, bf(L.x_embed_w), L.K0, H, L.d0, L.K0, s));
+  LLB_TRY(launch_f32_to_bf16(w->x_embed_w, L.d0, bf(L.x_embed_w), L.K0, H, L.d0, L.K0, s, nullptr));
   for (int d = 0; d < L.ydim; ++d)
-    LLB_TRY(launch_f32_to_bf16(w->y_mlp2_w[d], H, bf(L.cond_w) + (size_t)d * H, L.KC, H, H, H, s));
-  LLB_TRY(launch_f32_to_bf16(w->txt_w, L.tdim, bf(L.cond_w) + (size_t)L.ydim * H, L.KC, H, L.tdim, L.tdim, s));
+    LLB_TRY(launch_f32_to_bf16(w->y_mlp2_w[d], H, bf(L.cond_w) + (size_t)d * H, L.KC, H, H, H, s, nullptr));
+  LLB_TRY(launch_f32_to_bf16(w->txt_w, L.tdim, bf(L.cond_w) + (size_t)L.ydim * H, L.KC, H, L.tdim, L.tdim, s, nullptr));
   for (int l = 0; l < D; ++l) {
-    LLB_TRY(launch_f32_to_bf16(w->ada0_w[l], H, bf(L.ada0_w) + (size_t)l * H * H, H, H, H, H, s));
+    LLB_TRY(launch_f32_to_bf16(w->ada0_w[l], H, bf(L.ada0_w) + (size_t)l * H * H, H, H, H, H, s, nullptr));
     LLB_CUDA_OK(cp(L.ada0_b + (size_t)l * H * 4, w->ada0_b[l], H));
-    LLB_TRY(launch_f32_to_bf16(w->qkv_w[l], H, bf(L.qkv_w[l]), H, 3 * H, H, H, s));
-    LLB_TRY(launch_f32_to_bf16(w->proj_w[l], H, bf(L.proj_w[l]), H, H, H, H, s));
-    LLB_TRY(launch_f32_to_bf16(w->fc1_w[l], H, bf(L.fc1_w[l]), H, F, H, H, s));
-    LLB_TRY(launch_f32_to_bf16(w->fc2_w[l], F, bf(L.fc2_w[l]), F, H, F, F, s));
-    LLB_TRY(launch_f32_to_bf16(w->ada2_w[l], H, bf(L.ada2_w[l]), H, 6 * H, H, H, s));
+    LLB_TRY(launch_f32_to_bf16(w->qkv_w[l], H, bf(L.qkv_w[l]), H, 3 * H, H, H, s, nullptr));
+    LLB_TRY(launch_f32_to_bf16(w->proj_w[l], H, bf(L.proj_w[l]), H, H, H, H, s, nullptr));
+    LLB_TRY(launch_f32_to_bf16(w->fc1_w[l], H, bf(L.fc1_w[l]), H, F, H, H, s, nullptr));
+    LLB_TRY(launch_f32_to_bf16(w->fc2_w[l], F, bf(L.fc2_w[l]), F, H, F, F, s, nullptr));
+    LLB_TRY(launch_f32_to_bf16(w->ada2_w[l], H, bf(L.ada2_w[l]), H, 6 * H, H, H, s, nullptr));
     LLB_CUDA_OK(cp(L.qn_w[l], w->q_norm_w[l], DIT_DH));
     LLB_CUDA_OK(cp(L.qn_b[l], w->q_norm_b[l], DIT_DH));
     LLB_CUDA_OK(cp(L.kn_w[l], w->k_norm_w[l], DIT_DH));
@@ -587,11 +552,11 @@ int llb_dit_pack_weights(const llb_dit_config* cfg, const llb_dit_weights* w, vo
     LLB_CUDA_OK(cudaMemsetAsync(static_cast<uint8_t*>(packed) + L.fc2_b[l] + H * 4, 0, (size_t)(LLB_DIT_SPLITK - 1) * H * 4, s));
     LLB_CUDA_OK(cp(L.ada2_b[l], w->ada2_b[l], 6 * H));
   }
-  LLB_TRY(launch_f32_to_bf16(w->out_ada0_w, H, bf(L.ada0_w) + (size_t)D * H * H, H, H, H, H, s));
+  LLB_TRY(launch_f32_to_bf16(w->out_ada0_w, H, bf(L.ada0_w) + (size_t)D * H * H, H, H, H, H, s, nullptr));
   LLB_CUDA_OK(cp(L.ada0_b + (size_t)D * H * 4, w->out_ada0_b, H));
-  LLB_TRY(launch_f32_to_bf16(w->out_fc1_w, H, bf(L.out_fc1_w), H, H, H, H, s));
-  LLB_TRY(launch_f32_to_bf16(w->out_fc2_w, H, bf(L.out_fc2_w), H, L.d0, H, H, s));
-  LLB_TRY(launch_f32_to_bf16(w->out_ada2_w, H, bf(L.out_ada2_w), H, 2 * L.d0, H, H, s));
+  LLB_TRY(launch_f32_to_bf16(w->out_fc1_w, H, bf(L.out_fc1_w), H, H, H, H, s, nullptr));
+  LLB_TRY(launch_f32_to_bf16(w->out_fc2_w, H, bf(L.out_fc2_w), H, L.d0, H, H, s, nullptr));
+  LLB_TRY(launch_f32_to_bf16(w->out_ada2_w, H, bf(L.out_ada2_w), H, 2 * L.d0, H, H, s, nullptr));
   LLB_CUDA_OK(cp(L.out_fc1_b, w->out_fc1_b, H));
   LLB_CUDA_OK(cp(L.out_fc2_b, w->out_fc2_b, L.d0));
   LLB_CUDA_OK(cp(L.out_ada2_b, w->out_ada2_b, 2 * L.d0));
@@ -614,14 +579,12 @@ int llb_dit_pack_weights(const llb_dit_config* cfg, const llb_dit_weights* w, vo
   {
     float* feat = f32(L.setup_scratch);                  // (T+1,256)
     float* hidden = feat + (size_t)(L.T + 1) * 256;      // (T+1,H)
-    dit_tfeat_kernel<<<L.T + 1, 128, 0, s>>>(feat, L.T);
-    LLB_CUDA_OK(cudaGetLastError());
-    LLB_TRY(launch_linear_f32(feat, 256, w->t_mlp0_w, 256, w->t_mlp0_b, hidden, H, L.T + 1, H, 256, LLB_ACT_SILU, s));
-    LLB_TRY(launch_linear_f32(hidden, H, w->t_mlp2_w, H, w->t_mlp2_b, f32(L.c1_table), H, L.T + 1, H, H, LLB_ACT_NONE, s));
+    LLB_TRY(launch_kernel(nullptr, NO_PROF, false, dit_tfeat_kernel, dim3(L.T + 1), dim3(128), 0, s, feat, L.T));
+    LLB_TRY(launch_linear_f32(feat, 256, w->t_mlp0_w, 256, w->t_mlp0_b, hidden, H, L.T + 1, H, 256, LLB_ACT_SILU, s, nullptr));
+    LLB_TRY(launch_linear_f32(hidden, H, w->t_mlp2_w, H, w->t_mlp2_b, f32(L.c1_table), H, L.T + 1, H, H, LLB_ACT_NONE, s, nullptr));
   }
-  dit_cunc_kernel<<<ceil_div(H, 256), 256, 0, s>>>(w->y_drop, w->txt_drop, f32(L.c_unc), L.ydim, H);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_kernel(nullptr, NO_PROF, false, dit_cunc_kernel, dim3(ceil_div(H, 256)), dim3(256), 0, s, w->y_drop, w->txt_drop, f32(L.c_unc),
+                       L.ydim, H);
 }
 
 int llb_dit_create(const llb_dit_config* cfg, const void* packed, size_t packed_bytes, llb_dit** out) {
@@ -677,15 +640,11 @@ int llb_dit_begin(llb_dit* h, void* workspace, size_t workspace_bytes, int B, co
   const DitLayout& L = h->L;
   LLB_TRY(dit_bind(h, workspace, workspace_bytes, B, n_nodes_host, mol_index_base, s));
   // the copies above read pageable host memory: they have been staged by the time cudaMemcpyAsync returns
-  dit_cond_operand_kernel<<<dim3(B, L.ydim + 1), 256, 0, s>>>(props, txt, h->w<float>(L.y_mlp0_w), h->w<float>(L.y_mlp0_b), h->acond,
-                                                              h->missing, L.ydim, L.tdim, L.H, L.KC);
-  LLB_CUDA_OK(cudaGetLastError());
+  LLB_TRY(launch_kernel(&h->ctr, NO_PROF, false, dit_cond_operand_kernel, dim3(B, L.ydim + 1), dim3(256), 0, s, props, txt,
+                        h->w<float>(L.y_mlp0_w), h->w<float>(L.y_mlp0_b), h->acond, h->missing, L.ydim, L.tdim, L.H, L.KC));
   LLB_TRY(gemm_bias_act(h->acond, L.KC, h->w<void>(L.cond_w), L.KC, nullptr, h->cinv, L.H, B, L.H, L.KC, LLB_ACT_NONE, true, s, &h->ctr));
-  dit_cond_fixup_kernel<<<ceil_div(B * L.H, 256), 256, 0, s>>>(h->cinv, h->missing, h->w<float>(L.y_drop), h->w<float>(L.txt_drop),
-                                                              h->w<float>(L.txt_b), B, L.ydim, L.H);
-  LLB_CUDA_OK(cudaGetLastError());
-  h->launches += 2;
-  return LLB_OK;
+  return launch_kernel(&h->ctr, NO_PROF, false, dit_cond_fixup_kernel, dim3(ceil_div(B * L.H, 256)), dim3(256), 0, s, h->cinv, h->missing,
+                       h->w<float>(L.y_drop), h->w<float>(L.txt_drop), h->w<float>(L.txt_b), B, L.ydim, L.H);
 }
 
 int llb_dit_set_state(llb_dit* h, const int8_t* X, const int8_t* E, llb_stream_t stream) {
@@ -707,11 +666,8 @@ int llb_dit_get_state(llb_dit* h, int8_t* X, int8_t* E, llb_stream_t stream) {
 int llb_dit_init_state(llb_dit* h, uint64_t seed, const float* qX0, const float* qE0, llb_stream_t stream) {
   LLB_CHECK_ARG(h && h->B > 0, "llb_dit_init_state: no batch bound");
   LLB_CHECK_ARG((qX0 == nullptr) == (qE0 == nullptr), "llb_dit_init_state: pass both noise tensors or neither");
-  dit_init_state_kernel<<<h->B, 256, 0, (cudaStream_t)stream>>>(h->stX, h->stE, h->mol_off, h->L.N, qX0, qE0, seed,
-                                                               (uint32_t)h->L.T, h->mol_base, h->tables);
-  LLB_CUDA_OK(cudaGetLastError());
-  h->launches++;
-  return LLB_OK;
+  return launch_kernel(&h->ctr, NO_PROF, false, dit_init_state_kernel, dim3(h->B), dim3(256), 0, (cudaStream_t)stream, h->stX, h->stE, h->mol_off,
+                       h->L.N, qX0, qE0, seed, (uint32_t)h->L.T, h->mol_base, h->tables);
 }
 
 int llb_dit_denoise(llb_dit* h, int t, int unconditioned, float* logits_X, float* logits_E, llb_stream_t stream) {
@@ -746,9 +702,8 @@ int llb_dit_denoise_c(llb_dit* h, void* workspace, size_t workspace_bytes, int B
   LLB_CUDA_OK(cudaMemcpyAsync(h->stX, X, (size_t)B * L.N, cudaMemcpyDeviceToDevice, s));
   LLB_CUDA_OK(cudaMemcpyAsync(h->stE, E, (size_t)B * L.N * L.N, cudaMemcpyDeviceToDevice, s));
   // the caller's c replaces cinv + the timestep table; row B (the unconditional row of a guided pass) feeds nothing here
-  LLB_TRY(launch_f32_to_bf16(c, H, h->cvec, H, B, H, H, s));
+  LLB_TRY(launch_f32_to_bf16(c, H, h->cvec, H, B, H, H, s, &h->ctr));
   LLB_CUDA_OK(cudaMemsetAsync(h->cvec + (size_t)B * H, 0, (size_t)H * 2, s));
-  h->launches++;
   if (Mtok > 0) {
     h->save_x = saved ? sv.xs : nullptr;
     const int rc = dit_body(h, s);
@@ -799,7 +754,7 @@ int llb_dit_sample(llb_dit* h, int t_first, int t_last, uint64_t seed, const flo
   return LLB_OK;
 }
 
-int64_t llb_dit_launch_count(const llb_dit* h) { return h ? h->launches + h->ctr.launches : 0; }
+int64_t llb_dit_launch_count(const llb_dit* h) { return h ? h->ctr.launches : 0; }
 
 int llb_dit_graph_state(const llb_dit* h) { return h ? h->graph_state : 0; }
 

@@ -69,8 +69,7 @@ struct llb_dit {
   const uint8_t* blob = nullptr;
   std::vector<float> betas, abar;   // host copies of the schedule
   llb::DitTablesDev tables;
-  llb::GemmCounters ctr;
-  int64_t launches = 0;
+  llb::LaunchCounter ctr;
   // batch binding
   int B = 0, Mtok = 0, passes = 2;
   int64_t mol_base = 0;

@@ -370,23 +370,22 @@ int llb_dit_pack_grad_weights(llb_dit* h, void* grad_blob, size_t grad_bytes, ll
   uint8_t* base = (uint8_t*)grad_blob;
   auto dst = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(base + off); };
   auto tr = [&](size_t src, int rows, int cols, __nv_bfloat16* d, int ld_d) {
-    grad_transpose_kernel<<<dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s>>>(h->w<__nv_bfloat16>(src), cols, rows, cols, d, ld_d);
-    h->launches++;
-    return cudaGetLastError();
+    return launch_kernel(&h->ctr, NO_PROF, false, grad_transpose_kernel<__nv_bfloat16>, dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s,
+                         h->w<__nv_bfloat16>(src), cols, rows, cols, d, ld_d);
   };
   const int H = L.H, F = L.F, D = L.D;
   LLB_CUDA_OK(cudaMemsetAsync(base, 0, R.total, s));   // the K padding of the out-layer and condition operands is zero
   for (int l = 0; l < D; ++l) {
-    LLB_CUDA_OK(tr(L.qkv_w[l], 3 * H, H, dst(R.qkvt[l]), 3 * H));
-    LLB_CUDA_OK(tr(L.proj_w[l], H, H, dst(R.projt[l]), H));
-    LLB_CUDA_OK(tr(L.fc1_w[l], F, H, dst(R.fc1t[l]), F));
-    LLB_CUDA_OK(tr(L.fc2_w[l], H, F, dst(R.fc2t[l]), H));
-    LLB_CUDA_OK(tr(L.ada2_w[l], 6 * H, H, dst(R.ada2t) + (size_t)l * H * 6 * H, 6 * H));
+    LLB_TRY(tr(L.qkv_w[l], 3 * H, H, dst(R.qkvt[l]), 3 * H));
+    LLB_TRY(tr(L.proj_w[l], H, H, dst(R.projt[l]), H));
+    LLB_TRY(tr(L.fc1_w[l], F, H, dst(R.fc1t[l]), F));
+    LLB_TRY(tr(L.fc2_w[l], H, F, dst(R.fc2t[l]), H));
+    LLB_TRY(tr(L.ada2_w[l], 6 * H, H, dst(R.ada2t) + (size_t)l * H * 6 * H, 6 * H));
   }
-  LLB_CUDA_OK(tr(L.ada0_w, (D + 1) * H, H, dst(R.ada0t), dit_grad_ka(L)));
-  LLB_CUDA_OK(tr(L.out_fc1_w, H, H, dst(R.out_fc1t), H));
-  LLB_CUDA_OK(tr(L.out_fc2_w, L.d0, H, dst(R.out_fc2t), dit_grad_k0o(L)));
-  LLB_CUDA_OK(tr(L.out_ada2_w, 2 * L.d0, H, dst(R.out_ada2t), dit_grad_ko(L)));
+  LLB_TRY(tr(L.ada0_w, (D + 1) * H, H, dst(R.ada0t), dit_grad_ka(L)));
+  LLB_TRY(tr(L.out_fc1_w, H, H, dst(R.out_fc1t), H));
+  LLB_TRY(tr(L.out_fc2_w, L.d0, H, dst(R.out_fc2t), dit_grad_k0o(L)));
+  LLB_TRY(tr(L.out_ada2_w, 2 * L.d0, H, dst(R.out_ada2t), dit_grad_ko(L)));
   return LLB_OK;
 }
 
@@ -408,36 +407,28 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
   const int raw_ld = (int)align_up(d0, 4);
   const uint8_t* gb = (const uint8_t*)grad_blob;
   auto gw = [&](size_t off) { return (const void*)(gb + off); };
-  GemmCounters* ctr = &h->ctr;
+  LaunchCounter* ctr = &h->ctr;
   ctr->slot = LLB_PROF_GEMM_OTHER;
-  auto kdone = [&]() -> int {
-    LLB_CUDA_OK(cudaGetLastError());
-    h->launches++;
-    return LLB_OK;
-  };
   auto gemm = [&](const void* A, int lda, const void* W, int ldw, const float* bias, void* C, int ldc, int rows, int N, int K, int act,
                   bool f32, GemmGroups grp = GemmGroups()) {
     return gemm_bias_act(A, lda, W, ldw, bias, C, ldc, rows, N, K, act, f32, s, ctr, grp);
   };
   auto to_bf16 = [&](const float* x) -> int {   // sv.xb = bf16(x), the forward's GEMM operand of that residual row
-    LLB_TRY(launch_f32_to_bf16(x, H, sv.xb, H, M, H, H, s));
-    return kdone();
+    return launch_f32_to_bf16(x, H, sv.xb, H, M, H, H, s, ctr);
   };
   auto gelu_bwd = [&](const float* g, const float* pre, __nv_bfloat16* out, size_t total) -> int {
-    dit_grad_gelu_kernel<<<grid_for(total), 256, 0, s>>>(g, pre, out, total);
-    return kdone();
+    return launch_kernel(ctr, NO_PROF, false, dit_grad_gelu_kernel, grid_for(total), dim3(256), 0, s, g, pre, out, total);
   };
   auto add_dx = [&](const float* v) -> int {
-    dit_grad_add_kernel<<<grid_for((size_t)M * H), 256, 0, s>>>(sv.dx, v, (size_t)M * H);
-    return kdone();
+    return launch_kernel(ctr, NO_PROF, false, dit_grad_add_kernel, grid_for((size_t)M * H), dim3(256), 0, s, sv.dx, v, (size_t)M * H);
   };
   if (M > 0) {
     // ---- output layer
     LLB_TRY(to_bf16(sv.xs + (size_t)2 * D * M * H));
     LLB_TRY(gemm(sv.xb, H, h->w<void>(L.out_fc1_w), H, h->w<float>(L.out_fc1_b), sv.hb, H, M, H, H, LLB_ACT_GELU, false));
     LLB_TRY(gemm(sv.hb, H, h->w<void>(L.out_fc2_w), H, h->w<float>(L.out_fc2_b), sv.raw, raw_ld, M, d0, H, LLB_ACT_NONE, true));
-    dit_grad_out_tail_kernel<<<B, 256, 0, s>>>(sv.raw, raw_ld, sv.modout, sv.mol_off, dlogits_X, dlogits_E, L.N, sv.db, K0o, sv.dmodout);
-    LLB_TRY(kdone());
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, dit_grad_out_tail_kernel, dim3(B), dim3(256), 0, s, sv.raw, raw_ld, sv.modout, sv.mol_off, dlogits_X,
+                          dlogits_E, L.N, sv.db, K0o, sv.dmodout));
     LLB_TRY(gemm(sv.db, K0o, gw(R.out_fc2t), K0o, nullptr, sv.tmp, H, M, H, K0o, LLB_ACT_NONE, true));
     LLB_TRY(gemm(sv.xb, H, h->w<void>(L.out_fc1_w), H, h->w<float>(L.out_fc1_b), sv.pre, H, M, H, H, LLB_ACT_NONE, true));
     LLB_TRY(gelu_bwd(sv.tmp, sv.pre, sv.dvec, (size_t)M * H));
@@ -464,11 +455,10 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
       {
         RowLnBwdArgs a = t;
         a.shift = mod + 3 * H, a.scale = mod + 4 * H, a.gate = mod + 5 * H;
-        LLB_TRY(launch_row_ln_bwd(a, s));
-        LLB_TRY(kdone());
+        LLB_TRY(launch_row_ln_bwd(a, s, ctr));
       }
-      grad_segsum_kernel<<<seg_grid, 256, 0, s>>>(sv.prod, 3 * H, sv.mol_off, 3 * H, nullptr, sv.dmod + (size_t)l * 6 * H + 3 * H, nullptr, ldm);
-      LLB_TRY(kdone());
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, grad_segsum_kernel, seg_grid, dim3(256), 0, s, sv.prod, 3 * H, sv.mol_off, 3 * H, nullptr,
+                            sv.dmod + (size_t)l * 6 * H + 3 * H, nullptr, ldm));
       ctr->slot = LLB_PROF_GEMM_FC2;
       LLB_TRY(gemm(sv.dvec, H, gw(R.fc2t[l]), H, nullptr, sv.tmp, F, M, F, H, LLB_ACT_NONE, true));
       ctr->slot = LLB_PROF_GEMM_FC1;
@@ -485,37 +475,26 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
       {
         CUtensorMap tmQKV;
         LLB_TRY(make_tensor_map_2d(&tmQKV, sv.qkv, 2, M, 3 * H, 3 * H, DIT_DH, 64, 128));
-        ProfScope prof(LLB_PROF_ATTENTION, s);
-        LLB_CUDA_OK(launch_pdl(dit_attention_tma_kernel, dim3((unsigned)(B * L.heads)), dim3(128), 0, s, tmQKV, sv.attn,
-                               (const int32_t*)sv.mol_off, B, M, H, L.heads));
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel, dim3((unsigned)(B * L.heads)), dim3(128), 0, s, tmQKV, sv.attn,
+                              sv.mol_off, B, M, H, L.heads));
       }
-      LLB_TRY(kdone());
       ctr->slot = LLB_PROF_GEMM_PROJ;
       LLB_TRY(gemm(sv.attn, H, h->w<void>(L.proj_w[l]), H, h->w<float>(L.proj_b[l]), sv.y, H, M, H, H, LLB_ACT_NONE, true));
       {
         RowLnBwdArgs a = t;
         a.shift = mod, a.scale = mod + H, a.gate = mod + 2 * H;
         if (l == 0) a.out_bf16 = nullptr;
-        LLB_TRY(launch_row_ln_bwd(a, s));
-        LLB_TRY(kdone());
+        LLB_TRY(launch_row_ln_bwd(a, s, ctr));
       }
-      grad_segsum_kernel<<<seg_grid, 256, 0, s>>>(sv.prod, 3 * H, sv.mol_off, 3 * H, nullptr, sv.dmod + (size_t)l * 6 * H, nullptr, ldm);
-      LLB_TRY(kdone());
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, grad_segsum_kernel, seg_grid, dim3(256), 0, s, sv.prod, 3 * H, sv.mol_off, 3 * H, nullptr,
+                            sv.dmod + (size_t)l * 6 * H, nullptr, ldm));
       if (l == 0) break;   // block 0's input is the token embedding: nothing upstream depends on c
       LLB_TRY(gemm(sv.dvec, H, gw(R.projt[l]), H, nullptr, sv.attn, H, M, H, H, LLB_ACT_NONE, false));   // dO (bf16)
       ctr->slot = LLB_PROF_GEMM_QKV;
       LLB_TRY(gemm(sv.xb, H, h->w<void>(L.qkv_w[l]), H, nullptr, sv.qkv_raw, 3 * H, M, 3 * H, H, LLB_ACT_NONE, true));
-      {
-        static bool configured = false;
-        if (!configured) {
-          LLB_CUDA_OK(cudaFuncSetAttribute(dit_grad_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AG_SMEM));
-          configured = true;
-        }
-        ProfScope prof(LLB_PROF_ATTENTION, s);
-        dit_grad_attention_kernel<<<B * L.heads, 256, AG_SMEM, s>>>(sv.qkv_raw, sv.qkv, sv.attn, sv.mol_off, H, L.heads, h->w<float>(L.qn_w[l]),
-                                                                   h->w<float>(L.qn_b[l]), h->w<float>(L.kn_w[l]), h->w<float>(L.kn_b[l]), sv.db);
-      }
-      LLB_TRY(kdone());
+      LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, false, dit_grad_attention_kernel, dim3(B * L.heads), dim3(256), AG_SMEM, s, sv.qkv_raw, sv.qkv,
+                            sv.attn, sv.mol_off, H, L.heads, h->w<float>(L.qn_w[l]), h->w<float>(L.qn_b[l]), h->w<float>(L.kn_w[l]),
+                            h->w<float>(L.kn_b[l]), sv.db));
       LLB_TRY(gemm(sv.db, 3 * H, gw(R.qkvt[l]), 3 * H, nullptr, sv.y, H, M, H, 3 * H, LLB_ACT_NONE, true));
       LLB_TRY(add_dx(sv.y));
     }
@@ -526,28 +505,25 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
   // ---- condition
   ctr->slot = LLB_PROF_GEMM_ADALN;
   const size_t nmod = (size_t)B * ldm;
-  dit_grad_softsign_kernel<<<grid_for(nmod), 256, 0, s>>>(sv.dmod, sv.mod, sv.dz_b, nmod);
-  LLB_TRY(kdone());
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, dit_grad_softsign_kernel, grid_for(nmod), dim3(256), 0, s, sv.dmod, sv.mod, sv.dz_b, nmod));
   const int ldh = (D + 1) * H;
   {
     GemmGroups grp;
     grp.group_n = H, grp.group_k = 6 * H;
     LLB_TRY(gemm(sv.dz_b, ldm, gw(R.ada2t), 6 * H, nullptr, sv.dhid, ldh, B, D * H, 6 * H, LLB_ACT_NONE, true, grp));
   }
-  LLB_TRY(launch_f32_to_bf16(sv.dmodout, 2 * d0, sv.dmodout_b, KO, B, 2 * d0, KO, s));
-  LLB_TRY(kdone());
+  LLB_TRY(launch_f32_to_bf16(sv.dmodout, 2 * d0, sv.dmodout_b, KO, B, 2 * d0, KO, s, ctr));
   LLB_TRY(gemm(sv.dmodout_b, KO, gw(R.out_ada2t), KO, nullptr, sv.dhid + (size_t)D * H, ldh, B, H, KO, LLB_ACT_NONE, true));
   LLB_TRY(gemm(sv.cvec, H, h->w<void>(L.ada0_w), H, h->w<float>(L.ada0_b), sv.pre0, ldh, B, ldh, H, LLB_ACT_NONE, true));
-  dit_grad_silu_kernel<<<grid_for((size_t)B * KA), 256, 0, s>>>(sv.dhid, sv.pre0, ldh, sv.dpre_b, KA, B);
-  LLB_TRY(kdone());
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, dit_grad_silu_kernel, grid_for((size_t)B * KA), dim3(256), 0, s, sv.dhid, sv.pre0, ldh, sv.dpre_b, KA,
+                        B));
   {
     const int S = sv.split, ks = KA / S;
     GemmGroups split;
     split.group_n = H, split.group_k = ks, split.split_k = true;
     LLB_TRY(gemm(sv.dpre_b, KA, gw(R.ada0t), KA, nullptr, sv.dc_parts, S * H, B, S * H, ks, LLB_ACT_NONE, true, split));
-    dit_grad_sum_slices_kernel<<<grid_for((size_t)B * H), 256, 0, s>>>(sv.dc_parts, S, H, B, dc);
+    return launch_kernel(ctr, NO_PROF, false, dit_grad_sum_slices_kernel, grid_for((size_t)B * H), dim3(256), 0, s, sv.dc_parts, S, H, B, dc);
   }
-  return kdone();
 }
 
 }  // extern "C"

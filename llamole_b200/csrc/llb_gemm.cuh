@@ -670,14 +670,9 @@ struct GemmGroups {
   bool m_fastest = false;   // tile order: consecutive CTAs share a W tile (narrow A resident in L2, wide W streamed from HBM once)
 };
 
-struct GemmCounters {
-  int64_t launches = 0;
-  int slot = LLB_PROF_GEMM_OTHER;  // profiling slot charged for the next launches
-};
-
 template <int BN, class Epi>
 int launch_gemm(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const Epi& epi,
-                cudaStream_t stream, GemmCounters* ctr = nullptr, GemmGroups grp = GemmGroups()) {
+                cudaStream_t stream, LaunchCounter* ctr = nullptr, GemmGroups grp = GemmGroups()) {
   using Cfg = GemmCfg<BN>;
   if (M <= 0 || N <= 0) return LLB_OK;
   LLB_CHECK_ARG(K > 0 && lda % 8 == 0 && ldw % 8 == 0, "gemm: K=%d lda=%d ldw=%d (ld must be a multiple of 8)", K, lda, ldw);
@@ -701,45 +696,32 @@ int launch_gemm(const void* A, int lda, const void* W, int ldw, int M, int N, in
   // m-fastest automatically when A fits the L2 comfortably and W does not (the predictor head: 50 MB of activations against a
   // 1.1 GB weight, which the n-fastest walk would stream from HBM once per 256-row block); never for grouped launches
   const bool m_fast = grp.group_n == 0 && (grp.m_fastest || ((size_t)M * K * 2 <= ((size_t)64 << 20) && (size_t)N * K * 2 >= ((size_t)256 << 20)));
-  static bool configured[4] = {false, false, false, false};  // per template instantiation
   // CTA-pair kernel: wide problems whose 256 x 256 pair-tiles fill the machine
   const int pair_tiles = ceil_div(M, 2 * GEMM_BM) * ceil_div(N, 256);
   // (not for a single row block: the pair's second CTA would multiply nothing but padding, and a skinny GEMM -- the adaLN
   // modulations of a handful of molecules, 352 MB of weights against 7 rows -- wants every SM streaming its own weight tiles)
   const bool use_pair = BN == 256 && M > GEMM_BM && pair_tiles >= num_sms() / 2 && grp.group_n % 256 == 0;
+  const int slot = ctr ? ctr->slot : LLB_PROF_GEMM_OTHER;
+  const int flags = (grp.ab_f16 ? 1 : 0) | (m_fast ? 2 : 0);
   if (use_pair) {
+    // the cluster shape is the kernel's __cluster_dims__; an ordinary launch
     CUtensorMap tmBh;
     LLB_TRY(make_tensor_map_2d(&tmBh, W, 2, w_rows, w_cols, ldw, GEMM_BK, 128, 128));
-    auto launch2 = [&](auto kern, int which) -> int {
-      if (!configured[which]) {
-        LLB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Gemm2Cfg::SMEM_BYTES));
-        configured[which] = true;
-      }
-      const int pairs = pair_tiles < num_sms() / 2 ? pair_tiles : num_sms() / 2;
-      ProfScope prof(ctr ? ctr->slot : LLB_PROF_GEMM_OTHER, stream);
-      kern<<<2 * pairs, GEMM_THREADS, Gemm2Cfg::SMEM_BYTES, stream>>>(tmA, tmBh, tmC, M, N, K, epi, grp.group_n, grp.group_k, grp.split_k ? 1 : 0, (grp.ab_f16 ? 1 : 0) | (m_fast ? 2 : 0));
-      note_kernel(LLB_KERN_GEMM_2CTA);
-      return LLB_OK;
+    const int pairs = pair_tiles < num_sms() / 2 ? pair_tiles : num_sms() / 2;
+    auto launch2 = [&](auto kern) -> int {
+      return launch_kernel(ctr, slot, false, kern, dim3(2 * pairs), dim3(GEMM_THREADS), (size_t)Gemm2Cfg::SMEM_BYTES, stream, tmA, tmBh, tmC, M, N,
+                           K, epi, grp.group_n, grp.group_k, grp.split_k ? 1 : 0, flags);
     };
-    if (tma_store) LLB_TRY(launch2(gemm_tcgen05_2cta_kernel<true, Epi>, 2));
-    else LLB_TRY(launch2(gemm_tcgen05_2cta_kernel<false, Epi>, 3));
-  } else {
-    auto launch = [&](auto kern, int which) -> int {
-      if (!configured[which]) {
-        LLB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        configured[which] = true;
-      }
-      ProfScope prof(ctr ? ctr->slot : LLB_PROF_GEMM_OTHER, stream);
-      LLB_CUDA_OK(launch_pdl(kern, dim3(grid), dim3(GEMM_THREADS), (size_t)Cfg::SMEM_BYTES, stream, tmA, tmB, tmC, M, N, K, epi, grp.group_n, grp.group_k,
-                             grp.split_k ? 1 : 0, (grp.ab_f16 ? 1 : 0) | (m_fast ? 2 : 0)));
-      note_kernel(LLB_KERN_GEMM_1CTA);
-      return LLB_OK;
-    };
-    if (tma_store) LLB_TRY(launch(gemm_tcgen05_kernel<BN, true, Epi>, 0));
-    else LLB_TRY(launch(gemm_tcgen05_kernel<BN, false, Epi>, 1));
+    LLB_TRY(tma_store ? launch2(gemm_tcgen05_2cta_kernel<true, Epi>) : launch2(gemm_tcgen05_2cta_kernel<false, Epi>));
+    note_kernel(LLB_KERN_GEMM_2CTA);
+    return LLB_OK;
   }
-  LLB_CUDA_OK(cudaGetLastError());
-  if (ctr) ctr->launches++;
+  auto launch1 = [&](auto kern) -> int {
+    return launch_kernel(ctr, slot, true, kern, dim3(grid), dim3(GEMM_THREADS), (size_t)Cfg::SMEM_BYTES, stream, tmA, tmB, tmC, M, N, K, epi,
+                         grp.group_n, grp.group_k, grp.split_k ? 1 : 0, flags);
+  };
+  LLB_TRY(tma_store ? launch1(gemm_tcgen05_kernel<BN, true, Epi>) : launch1(gemm_tcgen05_kernel<BN, false, Epi>));
+  note_kernel(LLB_KERN_GEMM_1CTA);
   return LLB_OK;
 }
 
@@ -789,6 +771,6 @@ struct EpiBiasAct {
 
 // Generic runtime-dispatched GEMM used by the small / non-critical linears.
 int gemm_bias_act(const void* A, int lda, const void* W, int ldw, const float* bias, void* C, int ldc, int M, int N,
-                  int K, int act, bool out_f32, cudaStream_t stream, GemmCounters* ctr = nullptr, GemmGroups grp = GemmGroups());
+                  int K, int act, bool out_f32, cudaStream_t stream, LaunchCounter* ctr = nullptr, GemmGroups grp = GemmGroups());
 
 }  // namespace llb

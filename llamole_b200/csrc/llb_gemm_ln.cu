@@ -749,7 +749,7 @@ size_t gemm_ln_pair_workspace_bytes() {
 }
 
 int launch_gemm_ln_pair(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const GemmLnArgs& e, void* sync_ws,
-                        size_t sync_bytes, cudaStream_t stream, GemmCounters* ctr) {
+                        size_t sync_bytes, cudaStream_t stream, LaunchCounter* ctr) {
   if (M <= 0) return LLB_OK;
   LLB_CHECK_ARG(N == 4 * GLN_BN && K % 8 == 0, "gemm_ln_pair: N=%d must be 1024 and K=%d a multiple of 8", N, K);
   LLB_CHECK_ARG(lda % 8 == 0 && ldw % 8 == 0 && e.ldx % 4 == 0 && e.ldxb % 8 == 0 && e.mod_ld % 4 == 0,
@@ -827,7 +827,7 @@ int launch_gemm_ln_pair(const void* A, int lda, const void* W, int ldw, int M, i
 
 template <int NS>
 static int launch_gin_tail_ns(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const GinTailArgs& t, void* sync_ws,
-                              cudaStream_t stream, GemmCounters* ctr) {
+                              cudaStream_t stream, LaunchCounter* ctr) {
   CUtensorMap tmA, tmBh, tmX, tmXb, tmXpf;
   LLB_TRY(make_tensor_map_2d(&tmA, A, 2, M, K, lda, GEMM_BK, GEMM_BM, 128));
   LLB_TRY(make_tensor_map_2d(&tmBh, W, 2, N, K, ldw, GEMM_BK, GLN_BN / 2, 128));
@@ -892,7 +892,7 @@ static int launch_gin_tail_ns(const void* A, int lda, const void* W, int ldw, in
 }
 
 int launch_gin_tail(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const GinTailArgs& t, void* sync_ws, size_t sync_bytes,
-                    cudaStream_t stream, GemmCounters* ctr) {
+                    cudaStream_t stream, LaunchCounter* ctr) {
   if (M <= 0) return LLB_OK;
   LLB_CHECK_ARG(gin_tail_supported(N, K), "gin_tail: N=%d must be 768 or 1024 and K=%d a multiple of 8", N, K);
   LLB_CHECK_ARG(lda % 8 == 0 && ldw % 8 == 0 && t.ldx % 4 == 0 && t.ldxb % 8 == 0 && t.mod_ld % 4 == 0 && t.addvec_ld % 4 == 0,

@@ -71,7 +71,7 @@ struct GinTailArgs {
 // N = 768 (three CTA pairs per 256-row block) or 1024 (four); needs the same exchange workspace as launch_gemm_ln_pair.
 inline bool gin_tail_supported(int N, int K) { return (N == 3 * GLN_BN || N == 4 * GLN_BN) && K % 8 == 0; }
 int launch_gin_tail(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const GinTailArgs& t, void* sync_ws, size_t sync_bytes,
-                    cudaStream_t stream, GemmCounters* ctr);
+                    cudaStream_t stream, LaunchCounter* ctr);
 // order-preserving encoding of a float for unsigned atomicMax (0 = below every float)
 __host__ __device__ inline uint32_t float_order_enc(uint32_t bits) { return (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u); }
 __host__ __device__ inline uint32_t float_order_dec(uint32_t e) { return (e & 0x80000000u) ? (e & 0x7fffffffu) : ~e; }
@@ -80,6 +80,6 @@ __host__ __device__ inline uint32_t float_order_dec(uint32_t e) { return (e & 0x
 // clears its counters with a stream-ordered memset) that no other launch uses concurrently.
 size_t gemm_ln_pair_workspace_bytes();
 int launch_gemm_ln_pair(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const GemmLnArgs& e, void* sync_ws,
-                        size_t sync_bytes, cudaStream_t stream, GemmCounters* ctr);
+                        size_t sync_bytes, cudaStream_t stream, LaunchCounter* ctr);
 
 }  // namespace llb

@@ -838,19 +838,21 @@ __global__ void __launch_bounds__(1024) gin_topk_thresh_kernel(const float* __re
   if (tid == 0) redo_flag[blockIdx.x] = 0;
 }
 
-// Rows per launch -> (threshold kernel | per-thread-list kernel) -> selection-pass kernel for whatever is still flagged.
-static void launch_softmax_topk(const float* logits, int rows, int W, int ld, int k, float* topv, int32_t* topi, int32_t* flags,
-                                cudaStream_t s) {
+// Rows per launch -> (threshold kernel | per-thread-list kernel) -> selection-pass kernel for whatever is still flagged; the two or
+// three kernels form one profiling record of prof_slot.
+static int launch_softmax_topk(const float* logits, int rows, int W, int ld, int k, float* topv, int32_t* topi, int32_t* flags,
+                               cudaStream_t s, LaunchCounter* ctr, int prof_slot) {
   const bool vec = (ld % 4 == 0) && ((reinterpret_cast<uintptr_t>(logits) & 15) == 0);
   const long long r_need = ((long long)7 * k * 4096 + W - 1) / W;
   const int R = r_need < 4 ? 4 : (int)r_need;
+  ProfScope prof(prof_slot, s);
   if (vec && W >= 16384 && R <= 32) {
-    gin_topk_thresh_kernel<<<rows, 1024, 0, s>>>(logits, ld, W, k, R, topv, topi, flags);
-    gin_topk_stream_kernel<<<rows, 1024, 0, s>>>(logits, ld, W, k, topv, topi, flags, 1);
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_topk_thresh_kernel, dim3(rows), dim3(1024), 0, s, logits, ld, W, k, R, topv, topi, flags));
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_topk_stream_kernel, dim3(rows), dim3(1024), 0, s, logits, ld, W, k, topv, topi, flags, 1));
   } else {
-    gin_topk_stream_kernel<<<rows, 1024, 0, s>>>(logits, ld, W, k, topv, topi, flags, 0);
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_topk_stream_kernel, dim3(rows), dim3(1024), 0, s, logits, ld, W, k, topv, topi, flags, 0));
   }
-  gin_topk_kernel<<<rows, 1024, 0, s>>>(logits, ld, W, k, topv, topi, flags);
+  return launch_kernel(ctr, NO_PROF, false, gin_topk_kernel, dim3(rows), dim3(1024), 0, s, logits, ld, W, k, topv, topi, flags);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1099,24 +1101,18 @@ static int gin_scan(llb_gin* g, const int32_t* deg, int32_t* rowptr, cudaStream_
   // rowptr[0..n] = exclusive scan of deg[0..n] (deg[n] = 0)
   const int cnt = g->n + 1;
   const int nb = ceil_div(cnt, 1024);
-  scan_block_kernel<<<nb, 1024, 0, s>>>(deg, rowptr, g->blk, cnt);
-  LLB_CUDA_OK(cudaGetLastError());
+  LaunchCounter* ctr = &g->ctr;
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, scan_block_kernel, dim3(nb), dim3(1024), 0, s, deg, rowptr, g->blk, cnt));
   if (nb > 1) {
     const int nb2 = ceil_div(nb, 1024);
     LLB_CHECK_ARG(nb2 <= 1024, "gin: too many nodes (%d)", g->n);
-    scan_block_kernel<<<nb2, 1024, 0, s>>>(g->blk, g->blk, g->blk2, nb);
-    LLB_CUDA_OK(cudaGetLastError());
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, scan_block_kernel, dim3(nb2), dim3(1024), 0, s, g->blk, g->blk, g->blk2, nb));
     if (nb2 > 1) {
-      scan_block_kernel<<<1, 1024, 0, s>>>(g->blk2, g->blk2, nullptr, nb2);
-      scan_add_kernel<<<nb2, 1024, 0, s>>>(g->blk, g->blk2, nb);
-      LLB_CUDA_OK(cudaGetLastError());
-      g->launches += 2;
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, scan_block_kernel, dim3(1), dim3(1024), 0, s, g->blk2, g->blk2, nullptr, nb2));
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, scan_add_kernel, dim3(nb2), dim3(1024), 0, s, g->blk, g->blk2, nb));
     }
-    scan_add_kernel<<<nb, 1024, 0, s>>>(rowptr, g->blk, cnt);
-    LLB_CUDA_OK(cudaGetLastError());
-    g->launches += 2;
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, scan_add_kernel, dim3(nb), dim3(1024), 0, s, rowptr, g->blk, cnt));
   }
-  g->launches++;
   return LLB_OK;
 }
 
@@ -1156,8 +1152,7 @@ static int gin_mlp4(llb_gin* g, const __nv_bfloat16* in, int rows, size_t w0, si
   a.gamma = g->w<float>(lnw), a.beta = g->w<float>(lnb), a.act = LLB_ACT_GELU;
   a.out_bf16 = zbuf, a.out_bf16_ld = hidden;
   a.prof_slot = LLB_PROF_GIN_ROWLN;
-  LLB_TRY(launch_row_ln(a, s));
-  g->launches++;
+  LLB_TRY(launch_row_ln(a, s, &g->ctr));
   g->ctr.slot = slot4;
   return gemm_bias_act(zbuf, hidden, g->w<void>(w4), hidden, g->w<float>(b4), out, out_ld, rows, out_f, hidden, LLB_ACT_NONE, true, s, &g->ctr);
 }
@@ -1168,16 +1163,15 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
   const GinLayout& G = g->G;
   const int H = G.Hp, L = G.L, n = g->n, B = g->B;   // H: the padded width of every H-wide buffer here
   LLB_CHECK_ARG(n > 0 && B > 0, "gin: no graph batch bound");
+  LaunchCounter* ctr = &g->ctr;
   const int eb = (int)(((size_t)n * (H / 4) + 255) / 256 < 8192 ? ((size_t)n * (H / 4) + 255) / 256 : 8192);
-  gin_embed_kernel<<<eb, 256, 0, s>>>(g->x32, g->w<float>(G.atom_emb), g->w<float>(G.vn_emb), g->h, g->hb, n, H);
-  gin_broadcast_rows_kernel<<<ceil_div(B * H, 256) < 4096 ? ceil_div(B * H, 256) : 4096, 256, 0, s>>>(g->w<float>(G.vn_emb), g->vn_cur, B, H);
-  LLB_CUDA_OK(cudaGetLastError());
-  g->launches += 2;
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_embed_kernel, dim3(eb), dim3(256), 0, s, g->x32, g->w<float>(G.atom_emb), g->w<float>(G.vn_emb),
+                        g->h, g->hb, n, H));
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_broadcast_rows_kernel, dim3(ceil_div(B * H, 256) < 4096 ? ceil_div(B * H, 256) : 4096), dim3(256),
+                        0, s, g->w<float>(G.vn_emb), g->vn_cur, B, H));
   if (G.predictor) {
-    gin_text_operand_kernel<<<ceil_div(B * G.tdim, 256) < 4096 ? ceil_div(B * G.tdim, 256) : 4096, 256, 0, s>>>(
-        c, g->w<float>(G.text_drop), g->ctext, B, G.tdim);
-    LLB_CUDA_OK(cudaGetLastError());
-    g->launches++;
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_text_operand_kernel, dim3(ceil_div(B * G.tdim, 256) < 4096 ? ceil_div(B * G.tdim, 256) : 4096),
+                          dim3(256), 0, s, c, g->w<float>(G.text_drop), g->ctext, B, G.tdim));
     g->ctr.slot = LLB_PROF_GIN_MISC;
     for (int l = 0; l < L; ++l)
       LLB_TRY(gemm_bias_act(g->ctext, G.tdim, g->w<void>(G.adapter_w[l]), G.tdim, g->w<float>(G.adapter_b[l]),
@@ -1188,20 +1182,18 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
     const bool last = (l == L - 1);
     if (sv && l > 0) LLB_CUDA_OK(cudaMemcpyAsync(sv->hin + (size_t)(l - 1) * n * H, g->h, (size_t)n * H * 4, cudaMemcpyDeviceToDevice, s));
     {
-      ProfScope prof(LLB_PROF_GIN_AGGREGATE, s);
       const float* be = g->w<float>(G.bond_emb[l]);
       const float* ep = g->w<float>(G.eps[l]);
-      const unsigned blocks = (unsigned)ceil_div(n, 8);
-      switch (H) {   // width-specialised (neighbour-outer) kernel for the widths the checkpoints and fixtures use
-        case 256: gin_aggregate_wide_kernel<1><<<blocks, 256, 0, s>>>(g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n); break;
-        case 512: gin_aggregate_wide_kernel<2><<<blocks, 256, 0, s>>>(g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n); break;
-        case 768: gin_aggregate_wide_kernel<3><<<blocks, 256, 0, s>>>(g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n); break;
-        case 1024: gin_aggregate_wide_kernel<4><<<blocks, 256, 0, s>>>(g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n); break;
-        default: gin_aggregate_kernel<<<blocks, 256, 0, s>>>(g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n, H);
-      }
+      const dim3 blocks(ceil_div(n, 8));
+      // width-specialised (neighbour-outer) kernel for the widths the checkpoints and fixtures use
+      auto wide = H == 256 ? gin_aggregate_wide_kernel<1> : H == 512 ? gin_aggregate_wide_kernel<2> : H == 768 ? gin_aggregate_wide_kernel<3>
+                  : H == 1024 ? gin_aggregate_wide_kernel<4> : nullptr;
+      if (wide)
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_AGGREGATE, false, wide, blocks, dim3(256), 0, s, g->hb, g->rowptr, g->col, g->eid, be, ep, g->agg, n));
+      else
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_AGGREGATE, false, gin_aggregate_kernel, blocks, dim3(256), 0, s, g->hb, g->rowptr, g->col, g->eid, be,
+                              ep, g->agg, n, H));
     }
-    LLB_CUDA_OK(cudaGetLastError());
-    g->launches++;
     if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->agg + (size_t)l * n * H, g->agg, (size_t)n * H * 2, cudaMemcpyDeviceToDevice, s));
     // LLB_GIN_FUSED_TAIL=0: second linear + row kernel instead of the fused GEMM + layer-tail kernel (launch_gin_tail)
     static const bool tail_env_off = getenv("LLB_GIN_FUSED_TAIL") && getenv("LLB_GIN_FUSED_TAIL")[0] == '0';
@@ -1209,18 +1201,18 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
     if (!last) {
       // virtual node of the next layer from the max-pool of this layer's INPUT (model.py:148 / :343): the fused tail of the
       // previous layer has already accumulated it while it wrote that input; layer 0 (and the unfused path) pool explicitly
-      {
-        ProfScope prof(LLB_PROF_GIN_POOL, s);
-        if (fused_tail && l > 0) {
-          const size_t total = (size_t)B * H;
-          gin_pool_decode_kernel<<<(unsigned)(ceil_div((int)(total / 4), 256) < 2048 ? ceil_div((int)(total / 4), 256) : 2048), 256, 0, s>>>(g->pool_enc, g->pool_b, total);
-        } else {
-          if (H % 2 == 0) gin_pool_max_bf16_kernel<<<dim3(B, ceil_div(H, 512)), 256, 0, s>>>(g->hb, g->graph_ptr, H, g->pool_b);
-          else gin_pool_kernel<<<dim3(B, ceil_div(H, 256)), 256, 0, s>>>(nullptr, g->hb, g->graph_ptr, H, 1, nullptr, g->pool_b);
-        }
+      if (fused_tail && l > 0) {
+        const size_t total = (size_t)B * H;
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_POOL, false, gin_pool_decode_kernel,
+                              dim3(ceil_div((int)(total / 4), 256) < 2048 ? ceil_div((int)(total / 4), 256) : 2048), dim3(256), 0, s, g->pool_enc,
+                              g->pool_b, total));
+      } else if (H % 2 == 0) {
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_POOL, false, gin_pool_max_bf16_kernel, dim3(B, ceil_div(H, 512)), dim3(256), 0, s, g->hb, g->graph_ptr,
+                              H, g->pool_b));
+      } else {
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_POOL, false, gin_pool_kernel, dim3(B, ceil_div(H, 256)), dim3(256), 0, s, nullptr, g->hb, g->graph_ptr,
+                              H, 1, nullptr, g->pool_b));
       }
-      LLB_CUDA_OK(cudaGetLastError());
-      g->launches++;
       if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->pool + (size_t)l * B * H, g->pool_b, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
       LLB_TRY(gin_mlp4(g, g->pool_b, B, G.vn0_w[l], G.vn0_b[l], G.vn_ln_w[l], G.vn_ln_b[l], G.vn4_w[l], G.vn4_b[l], G.I, 4 * G.H, H,
                        g->vz, g->vu, H, s));
@@ -1228,8 +1220,7 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
       a.in = g->vu, a.in_ld = H, a.rows = B, a.width = H, a.normalize = false;
       a.resid = g->vn_cur, a.resid_ld = H, a.out_f32 = g->vn_next, a.out_f32_ld = H;
       a.prof_slot = LLB_PROF_GIN_MISC;
-      LLB_TRY(launch_row_ln(a, s));
-      g->launches++;
+      LLB_TRY(launch_row_ln(a, s, ctr));
     }
     // LayerNorm + GELU of the node MLP in the first linear's epilogue, from analytic row statistics (see EpiRowSq); the
     // intermediate is fp16 and the second linear multiplies it by the fp16 copy of its weight
@@ -1266,17 +1257,12 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
       if (!last) a.addvec = g->vn_next, a.addvec_ld = H;
       a.out_f32 = g->h, a.out_f32_ld = H, a.out_bf16 = g->hb, a.out_bf16_ld = H;
       a.prof_slot = LLB_PROF_GIN_ROWLN;
-      LLB_TRY(launch_row_ln(a, s));
-      g->launches++;
+      LLB_TRY(launch_row_ln(a, s, ctr));
     }
     if (!last) std::swap(g->vn_cur, g->vn_next);
   }
-  {
-    ProfScope prof(LLB_PROF_GIN_POOL, s);
-    gin_pool_kernel<<<dim3(B, ceil_div(H, 256)), 256, 0, s>>>(g->h, nullptr, g->graph_ptr, H, 0, g->pooled, g->pooled_b);
-  }
-  LLB_CUDA_OK(cudaGetLastError());
-  g->launches++;
+  LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_POOL, false, gin_pool_kernel, dim3(B, ceil_div(H, 256)), dim3(256), 0, s, g->h, nullptr, g->graph_ptr, H, 0,
+                        g->pooled, g->pooled_b));
   if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->pooled_b, g->pooled_b, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
   return LLB_OK;
 }
@@ -1312,8 +1298,8 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
   LLB_CUDA_OK(cp_rows(G.atom_emb, Hp, w->atom_emb, ATOM_VOCAB, H));
   LLB_CUDA_OK(cp(G.vn_emb, w->vn_emb, H));
   for (int l = 0; l < G.L; ++l) {
-    gin_f32_to_f16_kernel<<<1024, 256, 0, s>>>(w->mlp4_w[l], 4 * H, reinterpret_cast<__half*>(base + G.mlp4_w[l]), I, H, 4 * H);   // fp16: see EpiLnGelu
-    LLB_CUDA_OK(cudaGetLastError());
+    LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_f32_to_f16_kernel, dim3(1024), dim3(256), 0, s, w->mlp4_w[l], 4 * H,
+                          reinterpret_cast<__half*>(base + G.mlp4_w[l]), I, H, 4 * H));   // fp16: see EpiLnGelu
     LLB_CUDA_OK(cp(G.eps[l], w->eps[l], 1));
     LLB_CUDA_OK(cp(G.mlp_ln_w[l], w->mlp_ln_w[l], 4 * H));
     LLB_CUDA_OK(cp(G.mlp_ln_b[l], w->mlp_ln_b[l], 4 * H));
@@ -1325,14 +1311,14 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
     // (not centred), and a padded Gram matrix would be singular.
     {
       float* wbar = reinterpret_cast<float*>(base + G.chol_scratch);   // scratch doubles as the column-mean buffer first
-      gin_colmean_kernel<<<ceil_div(H, 256), 256, 0, s>>>(w->mlp0_w[l], 4 * H, H, wbar);
-      gin_center_weight_kernel<<<1024, 256, 0, s>>>(w->mlp0_w[l], wbar, 4 * H, H, bf(G.mlp0_w[l]), Hp);
-      gin_center_bias_kernel<<<1, 1024, 0, s>>>(w->mlp0_b[l], w->mlp_ln_w[l], 4 * H, reinterpret_cast<float*>(base + G.mlp0_b[l]),
-                                                 reinterpret_cast<float*>(base + G.mlp_bg[l]));
+      LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_colmean_kernel, dim3(ceil_div(H, 256)), dim3(256), 0, s, w->mlp0_w[l], 4 * H, H, wbar));
+      LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_center_weight_kernel, dim3(1024), dim3(256), 0, s, w->mlp0_w[l], wbar, 4 * H, H,
+                            bf(G.mlp0_w[l]), Hp));
+      LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_center_bias_kernel, dim3(1), dim3(1024), 0, s, w->mlp0_b[l], w->mlp_ln_w[l], 4 * H,
+                            reinterpret_cast<float*>(base + G.mlp0_b[l]), reinterpret_cast<float*>(base + G.mlp_bg[l])));
       double* Gd = reinterpret_cast<double*>(base + G.chol_scratch);
-      gin_gram64_kernel<<<dim3(ceil_div(H + 1, 16), ceil_div(H + 1, 16)), 256, 0, s>>>(bf(G.mlp0_w[l]), Hp, reinterpret_cast<const float*>(base + G.mlp0_b[l]),
-                                                                                      4 * H, H, Gd);
-      LLB_CUDA_OK(cudaGetLastError());
+      LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_gram64_kernel, dim3(ceil_div(H + 1, 16), ceil_div(H + 1, 16)), dim3(256), 0, s,
+                            bf(G.mlp0_w[l]), Hp, reinterpret_cast<const float*>(base + G.mlp0_b[l]), 4 * H, H, Gd));
       const int n1 = H + 1;
       std::vector<double> Gh((size_t)n1 * n1), Lh;
       LLB_CUDA_OK(cudaMemcpyAsync(Gh.data(), Gd, Gh.size() * 8, cudaMemcpyDeviceToHost, s));
@@ -1358,8 +1344,8 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
       LLB_CUDA_OK(cp(G.norm_b[l], w->norm_b[l], H));
     }
     if (l < G.L - 1) {
-      LLB_TRY(launch_f32_to_bf16(w->vn0_w[l], H, bf(G.vn0_w[l]), Hp, 4 * H, H, Hp, s));
-      LLB_TRY(launch_f32_to_bf16(w->vn4_w[l], 4 * H, bf(G.vn4_w[l]), I, H, 4 * H, I, s));
+      LLB_TRY(launch_f32_to_bf16(w->vn0_w[l], H, bf(G.vn0_w[l]), Hp, 4 * H, H, Hp, s, nullptr));
+      LLB_TRY(launch_f32_to_bf16(w->vn4_w[l], 4 * H, bf(G.vn4_w[l]), I, H, 4 * H, I, s, nullptr));
       LLB_CUDA_OK(cp(G.vn0_b[l], w->vn0_b[l], 4 * H));
       LLB_CUDA_OK(cp(G.vn_ln_w[l], w->vn_ln_w[l], 4 * H));
       LLB_CUDA_OK(cp(G.vn_ln_b[l], w->vn_ln_b[l], 4 * H));
@@ -1369,24 +1355,22 @@ int llb_gin_pack_weights(const llb_gin_config* cfg, const llb_gin_weights* w, vo
       // [shift | scale | gate] as three row blocks of Hp rows: the forward reads them at mod, mod + Hp, mod + 2 Hp
       for (int b = 0; b < 3; ++b) {
         LLB_TRY(launch_f32_to_bf16(w->adapter_w[l] + (size_t)b * H * G.tdim, G.tdim, bf(G.adapter_w[l]) + (size_t)b * Hp * G.tdim, G.tdim, H,
-                                   G.tdim, G.tdim, s));
+                                   G.tdim, G.tdim, s, nullptr));
         LLB_CUDA_OK(cp(G.adapter_b[l] + (size_t)b * Hp * 4, w->adapter_b[l] + (size_t)b * H, H));
       }
     }
   }
   if (G.predictor) LLB_CUDA_OK(cp(G.text_drop, w->text_dropping, G.tdim));
   const int HOt = G.predictor ? G.out_dim : H;   // true output width of the head
-  LLB_TRY(launch_f32_to_bf16(w->head0_w, H, bf(G.head0_w), Hp, G.HHt, H, Hp, s));
-  LLB_TRY(launch_f32_to_bf16(w->head4_w, G.HHt, bf(G.head4_w), G.HH, HOt, G.HHt, G.HH, s));
+  LLB_TRY(launch_f32_to_bf16(w->head0_w, H, bf(G.head0_w), Hp, G.HHt, H, Hp, s, nullptr));
+  LLB_TRY(launch_f32_to_bf16(w->head4_w, G.HHt, bf(G.head4_w), G.HH, HOt, G.HHt, G.HH, s, nullptr));
   LLB_CUDA_OK(cp(G.head0_b, w->head0_b, G.HHt));
   LLB_CUDA_OK(cp(G.head_ln_w, w->head_ln_w, G.HHt));
   LLB_CUDA_OK(cp(G.head_ln_b, w->head_ln_b, G.HHt));
   LLB_CUDA_OK(cp(G.head4_b, w->head4_b, HOt));
-  if (G.pilot_cols > 0) {
-    gin_pilot_pack_kernel<<<G.pilot_cols, 256, 0, s>>>(w->head4_w, w->head4_b, G.HHt, G.pilot_stride, G.pilot_cols, bf(G.pilot_w), G.HH,
-                                                       reinterpret_cast<float*>(base + G.pilot_b));
-    LLB_CUDA_OK(cudaGetLastError());
-  }
+  if (G.pilot_cols > 0)
+    LLB_TRY(launch_kernel(nullptr, NO_PROF, false, gin_pilot_pack_kernel, dim3(G.pilot_cols), dim3(256), 0, s, w->head4_w, w->head4_b, G.HHt,
+                          G.pilot_stride, G.pilot_cols, bf(G.pilot_w), G.HH, reinterpret_cast<float*>(base + G.pilot_b)));
   return LLB_OK;
 }
 
@@ -1445,21 +1429,20 @@ int llb_gin_bind(llb_gin* g, void* workspace, size_t workspace_bytes, int num_no
   g->n = num_nodes, g->e = num_edges, g->B = num_graphs;
   const int n = num_nodes, e = num_edges;
   LLB_CUDA_OK(cudaMemsetAsync(g->flags, 0, 16, s));
-  gin_prep_nodes_kernel<<<ceil_div(n, 256), 256, 0, s>>>(x, batch, g->x32, g->batch32, g->graph_ptr, g->flags, n, num_graphs);
-  LLB_CUDA_OK(cudaGetLastError());
+  LaunchCounter* ctr = &g->ctr;
+  LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_prep_nodes_kernel, dim3(ceil_div(n, 256)), dim3(256), 0, s, x, batch, g->x32, g->batch32, g->graph_ptr,
+                        g->flags, n, num_graphs));
   LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
-  if (e > 0) {
-    gin_degree_kernel<<<ceil_div(e, 256), 256, 0, s>>>(edge_index, edge_attr, g->deg, g->flags, e, n);
-    LLB_CUDA_OK(cudaGetLastError());
-  }
+  if (e > 0)
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_degree_kernel, dim3(ceil_div(e, 256)), dim3(256), 0, s, edge_index, edge_attr, g->deg, g->flags, e,
+                          n));
   LLB_TRY(gin_scan(g, g->deg, g->rowptr, s));
   LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
   if (e > 0) {
-    gin_fill_kernel<<<ceil_div(e, 256), 256, 0, s>>>(edge_index, edge_attr, g->rowptr, g->deg, g->col, g->eid, e, n);
-    gin_sort_rows_kernel<<<ceil_div(n, 256), 256, 0, s>>>(g->rowptr, g->col, g->eid, n);
-    LLB_CUDA_OK(cudaGetLastError());
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_fill_kernel, dim3(ceil_div(e, 256)), dim3(256), 0, s, edge_index, edge_attr, g->rowptr, g->deg,
+                          g->col, g->eid, e, n));
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_sort_rows_kernel, dim3(ceil_div(n, 256)), dim3(256), 0, s, g->rowptr, g->col, g->eid, n));
   }
-  g->launches += 4;
   return LLB_OK;
 }
 
@@ -1489,8 +1472,7 @@ int llb_gin_encoder_forward(llb_gin* g, float* out, float* pooled_or_null, llb_s
   a.in = g->head_out, a.in_ld = G.Hp, a.rows = B, a.width = direct ? G.H : G.Hp, a.normalize = false, a.l2_normalize = true;
   a.out_f32 = direct ? out : g->head_out, a.out_f32_ld = direct ? G.H : G.Hp;
   a.prof_slot = LLB_PROF_GIN_MISC;
-  LLB_TRY(launch_row_ln(a, s));
-  g->launches++;
+  LLB_TRY(launch_row_ln(a, s, &g->ctr));
   if (!direct)
     LLB_CUDA_OK(cudaMemcpy2DAsync(out, (size_t)G.H * 4, g->head_out, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
   return LLB_OK;
@@ -1507,9 +1489,7 @@ static int gin_head_hidden(llb_gin* g, cudaStream_t s) {
   a.gamma = g->w<float>(G.head_ln_w), a.beta = g->w<float>(G.head_ln_b), a.act = LLB_ACT_GELU;
   a.out_bf16 = g->hz, a.out_bf16_ld = G.HH;
   a.prof_slot = LLB_PROF_GIN_ROWLN;
-  LLB_TRY(launch_row_ln(a, s));
-  g->launches++;
-  return LLB_OK;
+  return launch_row_ln(a, s, &g->ctr);
 }
 
 int llb_gin_predictor_forward(llb_gin* g, const float* c, float* logits, llb_stream_t stream) {
@@ -1545,14 +1525,14 @@ int llb_gin_predictor_forward_saved(llb_gin* g, const float* c, float* logits, v
   LLB_CUDA_OK(cudaMemcpyAsync(sv.batch32, g->batch32, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
   // source-sorted CSR (the bound batch's degree scratch is free once llb_gin_bind has built the destination CSR)
   LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
-  gin_csr_transpose_kernel<0><<<ceil_div(n, 256), 256, 0, s>>>(g->rowptr, g->col, g->eid, nullptr, g->deg, nullptr, nullptr, n);
-  LLB_CUDA_OK(cudaGetLastError());
+  const dim3 node_blocks(ceil_div(n, 256));
+  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<0>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, nullptr, g->deg,
+                        nullptr, nullptr, n));
   LLB_TRY(gin_scan(g, g->deg, sv.srowptr, s));
   LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
-  gin_csr_transpose_kernel<1><<<ceil_div(n, 256), 256, 0, s>>>(g->rowptr, g->col, g->eid, sv.srowptr, g->deg, sv.sdst, sv.seid, n);
-  gin_sort_rows_kernel<<<ceil_div(n, 256), 256, 0, s>>>(sv.srowptr, sv.sdst, sv.seid, n);
-  LLB_CUDA_OK(cudaGetLastError());
-  g->launches += 3;
+  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<1>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, sv.srowptr,
+                        g->deg, sv.sdst, sv.seid, n));
+  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_sort_rows_kernel, node_blocks, dim3(256), 0, s, sv.srowptr, sv.sdst, sv.seid, n));
   // from here on exactly llb_gin_predictor_forward
   LLB_TRY(gin_trunk(g, c, s, &sv));
   LLB_TRY(gin_head_hidden(g, s));
@@ -1576,10 +1556,8 @@ int llb_gin_predictor_topk(llb_gin* g, const float* c, int k, float* topk_prob, 
       g->ctr.slot = LLB_PROF_GIN_GEMM_HEAD;
       LLB_TRY(gemm_bias_act(in + (size_t)r0 * G.HH, G.HH, g->w<void>(G.head4_w), G.HH, g->w<float>(G.head4_b), g->logits_ws, G.out_dim, rows,
                             G.out_dim, G.HH, LLB_ACT_NONE, true, s, &g->ctr));
-      ProfScope prof(LLB_PROF_GIN_TOPK, s);
-      launch_softmax_topk(g->logits_ws, rows, G.out_dim, G.out_dim, k, outv + (size_t)r0 * k, outi + (size_t)r0 * k, g->topk_redo, s);
-      LLB_CUDA_OK(cudaGetLastError());
-      g->launches += 3;
+      LLB_TRY(launch_softmax_topk(g->logits_ws, rows, G.out_dim, G.out_dim, k, outv + (size_t)r0 * k, outi + (size_t)r0 * k, g->topk_redo, s, &g->ctr,
+                                  LLB_PROF_GIN_TOPK));
     }
     return LLB_OK;
   };
@@ -1596,22 +1574,13 @@ int llb_gin_predictor_topk(llb_gin* g, const float* c, int k, float* topk_prob, 
     g->ctr.slot = LLB_PROF_GIN_GEMM_HEAD;
     LLB_TRY(gemm_bias_act(in, G.HH, g->w<void>(G.pilot_w), G.HH, g->w<float>(G.pilot_b), g->pilot_logits, HEAD_PILOT_COLS, rows, HEAD_PILOT_COLS,
                           G.HH, LLB_ACT_NONE, true, s, &g->ctr));
-    {
-      ProfScope prof(LLB_PROF_GIN_TOPK, s);
-      gin_head_pilot_kernel<<<rows, 1024, 0, s>>>(g->pilot_logits, R, g->rowtau);
-    }
-    LLB_CUDA_OK(cudaGetLastError());
+    LLB_TRY(launch_kernel(&g->ctr, LLB_PROF_GIN_TOPK, false, gin_head_pilot_kernel, dim3(rows), dim3(1024), 0, s, g->pilot_logits, R, g->rowtau));
     EpiHeadTopk eh{nullptr, 0, g->w<float>(G.head4_b), g->rowtau, g->head_part, g->head_slots, g->head_cand, g->head_cnt};
     g->ctr.slot = LLB_PROF_GIN_GEMM_HEAD;
     LLB_TRY((launch_gemm<256>(in, G.HH, g->w<void>(G.head4_w), G.HH, rows, G.out_dim, G.HH, eh, s, &g->ctr)));
     note_kernel(LLB_KERN_HEAD_TOPK);
-    {
-      ProfScope prof(LLB_PROF_GIN_TOPK, s);
-      gin_head_select_kernel<<<rows, 256, 0, s>>>(g->head_part, g->head_slots, g->rowtau, g->head_cand, g->head_cnt, k, topk_prob + (size_t)r0 * k,
-                                                  topk_idx + (size_t)r0 * k, g->head_flagged, g->head_nflag);
-    }
-    LLB_CUDA_OK(cudaGetLastError());
-    g->launches += 2;
+    LLB_TRY(launch_kernel(&g->ctr, LLB_PROF_GIN_TOPK, false, gin_head_select_kernel, dim3(rows), dim3(256), 0, s, g->head_part, g->head_slots, g->rowtau,
+                          g->head_cand, g->head_cnt, k, topk_prob + (size_t)r0 * k, topk_idx + (size_t)r0 * k, g->head_flagged, g->head_nflag));
     // the one host synchronisation of this entry: did any row fall outside the threshold scheme's guarantees?
     int32_t nflag = 0;
     LLB_CUDA_OK(cudaMemcpyAsync(&nflag, g->head_nflag, 4, cudaMemcpyDeviceToHost, s));
@@ -1619,18 +1588,16 @@ int llb_gin_predictor_topk(llb_gin* g, const float* c, int k, float* topk_prob, 
     g->head_flagged_rows += nflag, g->head_fused_rows += rows;
     for (int f0 = 0; f0 < nflag; f0 += g->chunk_rows) {
       const int fr = nflag - f0 < g->chunk_rows ? nflag - f0 : g->chunk_rows;
-      gin_gather_rows_kernel<<<fr, 128, 0, s>>>(in, g->head_flagged + f0, G.HH, g->redo_in);
-      LLB_CUDA_OK(cudaGetLastError());
+      LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_gather_rows_kernel, dim3(fr), dim3(128), 0, s, in, g->head_flagged + f0, G.HH, g->redo_in));
       LLB_TRY(materialise(g->redo_in, fr, g->redo_v, g->redo_i));
-      gin_scatter_topk_kernel<<<fr, 64, 0, s>>>(g->redo_v, g->redo_i, g->head_flagged + f0, k, topk_prob + (size_t)r0 * k, topk_idx + (size_t)r0 * k);
-      LLB_CUDA_OK(cudaGetLastError());
-      g->launches += 2;
+      LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_scatter_topk_kernel, dim3(fr), dim3(64), 0, s, g->redo_v, g->redo_i, g->head_flagged + f0, k,
+                            topk_prob + (size_t)r0 * k, topk_idx + (size_t)r0 * k));
     }
   }
   return LLB_OK;
 }
 
-int64_t llb_gin_launch_count(const llb_gin* g) { return g ? g->launches + g->ctr.launches : 0; }
+int64_t llb_gin_launch_count(const llb_gin* g) { return g ? g->ctr.launches : 0; }
 
 int64_t llb_gin_stat(const llb_gin* g, int which) {
   if (!g) return -1;
@@ -1647,18 +1614,15 @@ int llb_softmax_topk(const float* logits, int rows, int W, int ld, int k, float*
   LLB_CHECK_ARG(logits && topk_prob && topk_idx && scratch && rows >= 1 && W >= 1 && ld >= W && k >= 1 && k <= W,
                 "llb_softmax_topk: bad argument (rows=%d W=%d ld=%d k=%d)", rows, W, ld, k);
   cudaStream_t s = (cudaStream_t)stream;
-  launch_softmax_topk(logits, rows, W, ld, k, topk_prob, topk_idx, scratch, s);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_softmax_topk(logits, rows, W, ld, k, topk_prob, topk_idx, scratch, s, nullptr, NO_PROF);
 }
 
 int llb_cost_mlp(const float* w0, const float* b0, const float* w1, const float* b1, const float* fps, int n, int fp_dim,
                  int latent, float* out, llb_stream_t stream) {
   LLB_TRY(require_sm100());
   LLB_CHECK_ARG(w0 && b0 && w1 && b1 && fps && out && n >= 1 && fp_dim >= 1 && latent >= 1 && latent <= 4096, "llb_cost_mlp: bad argument");
-  cost_mlp_kernel<<<n, 256, latent * sizeof(float), (cudaStream_t)stream>>>(w0, b0, w1, b1, fps, fp_dim, latent, out);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_kernel(nullptr, NO_PROF, false, cost_mlp_kernel, dim3(n), dim3(256), latent * sizeof(float), (cudaStream_t)stream, w0, b0, w1, b1, fps,
+                       fp_dim, latent, out);
 }
 
 }  // extern "C"

@@ -81,8 +81,7 @@ struct llb_gin {
   llb_gin_config cfg;
   llb::GinLayout G;
   const uint8_t* blob = nullptr;
-  llb::GemmCounters ctr;
-  int64_t launches = 0;
+  llb::LaunchCounter ctr;
   int n = 0, e = 0, B = 0;
   bool want_logits = false;
   int32_t *x32 = nullptr, *batch32 = nullptr, *graph_ptr = nullptr, *rowptr = nullptr, *col = nullptr, *eid = nullptr;

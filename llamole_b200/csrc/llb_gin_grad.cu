@@ -190,24 +190,24 @@ int llb_gin_pack_grad_weights(llb_gin* g, void* grad_blob, size_t grad_bytes, ll
   uint8_t* base = (uint8_t*)grad_blob;
   auto dst = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(base + off); };
   auto tr = [&](const auto* src, int ld_s, int rows, int cols, __nv_bfloat16* d, int ld_d) {
-    grad_transpose_kernel<<<dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s>>>(src, ld_s, rows, cols, d, ld_d);
-    g->launches++;
-    return cudaGetLastError();
+    using T = std::remove_const_t<std::remove_pointer_t<decltype(src)>>;
+    return launch_kernel(&g->ctr, NO_PROF, false, grad_transpose_kernel<T>, dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s, src,
+                         ld_s, rows, cols, d, ld_d);
   };
   const int Hp = G.Hp, I = G.I, HH = G.HH;
   LLB_CUDA_OK(cudaMemsetAsync(base, 0, R.total, s));   // the head's K padding past out_dim is zero
-  LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.head4_w), HH, G.out_dim, HH, dst(R.head4t), R.kp));
-  LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.head0_w), Hp, HH, Hp, dst(R.head0t), HH));
+  LLB_TRY(tr(g->w<__nv_bfloat16>(G.head4_w), HH, G.out_dim, HH, dst(R.head4t), R.kp));
+  LLB_TRY(tr(g->w<__nv_bfloat16>(G.head0_w), Hp, HH, Hp, dst(R.head0t), HH));
   for (int l = 1; l < G.L; ++l) {
-    LLB_CUDA_OK(tr(g->w<__half>(G.mlp4_w[l]), I, Hp, I, dst(R.mlp4t[l]), Hp));   // the forward's copy is fp16 (see EpiLnGelu)
-    LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.mlp0_w[l]), Hp, I, Hp, dst(R.mlp0t[l]), I));
+    LLB_TRY(tr(g->w<__half>(G.mlp4_w[l]), I, Hp, I, dst(R.mlp4t[l]), Hp));   // the forward's copy is fp16 (see EpiLnGelu)
+    LLB_TRY(tr(g->w<__nv_bfloat16>(G.mlp0_w[l]), Hp, I, Hp, dst(R.mlp0t[l]), I));
     if (l < G.L - 1) {
-      LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.vn4_w[l]), I, Hp, I, dst(R.vn4t[l]), Hp));
-      LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.vn0_w[l]), Hp, I, Hp, dst(R.vn0t[l]), I));
+      LLB_TRY(tr(g->w<__nv_bfloat16>(G.vn4_w[l]), I, Hp, I, dst(R.vn4t[l]), Hp));
+      LLB_TRY(tr(g->w<__nv_bfloat16>(G.vn0_w[l]), Hp, I, Hp, dst(R.vn0t[l]), I));
     }
   }
   for (int l = 0; l < G.L; ++l)
-    LLB_CUDA_OK(tr(g->w<__nv_bfloat16>(G.adapter_w[l]), G.tdim, 3 * Hp, G.tdim, dst(R.adaptert) + (size_t)l * 3 * Hp, G.L * 3 * Hp));
+    LLB_TRY(tr(g->w<__nv_bfloat16>(G.adapter_w[l]), G.tdim, 3 * Hp, G.tdim, dst(R.adaptert) + (size_t)l * 3 * Hp, G.L * 3 * Hp));
   return LLB_OK;
 }
 
@@ -229,18 +229,13 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
   cudaStream_t s = (cudaStream_t)stream;
   const uint8_t* gb = (const uint8_t*)grad_blob;
   auto gw = [&](size_t off) { return (const void*)(gb + off); };
-  g->ctr.slot = LLB_PROF_GIN_MISC;
-  auto kdone = [&]() -> int {
-    LLB_CUDA_OK(cudaGetLastError());
-    g->launches++;
-    return LLB_OK;
-  };
+  LaunchCounter* ctr = &g->ctr;
+  ctr->slot = LLB_PROF_GIN_MISC;
 
   // ---- head: dhz = dlogits . W4 as head_split K slices (M = B is one or two row blocks; one slice would run on a few CTAs)
   {
     const int kp = R.kp, S = sv.head_split, kslice = kp / S;
-    LLB_TRY(launch_f32_to_bf16(dlogits, G.out_dim, sv.dlog_b, kp, B, G.out_dim, kp, s));
-    LLB_TRY(kdone());
+    LLB_TRY(launch_f32_to_bf16(dlogits, G.out_dim, sv.dlog_b, kp, B, G.out_dim, kp, s, ctr));
     GemmGroups split;
     split.group_n = HH, split.group_k = kslice, split.split_k = true;
     g->ctr.slot = LLB_PROF_GIN_GEMM_HEAD;
@@ -254,11 +249,10 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
     a.rows = B, a.width = HH, a.valid = G.HHt;
     a.gamma = g->w<float>(G.head_ln_w), a.beta = g->w<float>(G.head_ln_b), a.gelu = true;
     a.out_bf16 = sv.dhz_pre, a.out_ld = HH;
-    LLB_TRY(launch_row_ln_bwd(a, s));
-    LLB_TRY(kdone());
+    LLB_TRY(launch_row_ln_bwd(a, s, ctr));
     LLB_TRY(gemm_bias_act(sv.dhz_pre, HH, gw(R.head0t), HH, nullptr, sv.dpooled, Hp, B, Hp, HH, LLB_ACT_NONE, true, s, &g->ctr));
-    gin_grad_gather_kernel<<<grid_for((size_t)n * Hp), 256, 0, s>>>(sv.dpooled, sv.batch32, n, Hp, sv.dh);
-    LLB_TRY(kdone());
+    LLB_TRY(launch_kernel(ctr, NO_PROF, false, gin_grad_gather_kernel, grid_for((size_t)n * Hp), dim3(256), 0, s, sv.dpooled, sv.batch32, n, Hp,
+                          sv.dh));
   }
   // ---- layers, last to first; sv.dh holds dL/d(output of layer l) = dL/d(h_in_{l+1}) on entry
   const dim3 seg_grid_h(B, ceil_div(Hp, 256));
@@ -267,8 +261,8 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
     const float* hin = l > 0 ? sv.hin + (size_t)(l - 1) * n * Hp : nullptr;
     if (!last) {
       // vn_{l+1} is added to every node of h_in_{l+1} and carried into vn_{l+2}
-      grad_segsum_kernel<<<seg_grid_h, 256, 0, s>>>(sv.dh, Hp, sv.graph_ptr, Hp, l < L - 2 ? sv.dvn : nullptr, sv.dvn, sv.dvn_b, Hp);
-      LLB_TRY(kdone());
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, grad_segsum_kernel, seg_grid_h, dim3(256), 0, s, sv.dh, Hp, sv.graph_ptr, Hp,
+                            l < L - 2 ? sv.dvn : nullptr, sv.dvn, sv.dvn_b, Hp));
       if (l > 0) {
         // vn_{l+1} = vn_l + MLP_l(maxpool(h_in_l)): back through the MLP to the pooled row (routed below)
         g->ctr.slot = LLB_PROF_GIN_MISC;
@@ -280,8 +274,7 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
         a.rows = B, a.width = I, a.valid = 4 * G.H;
         a.gamma = g->w<float>(G.vn_ln_w[l]), a.beta = g->w<float>(G.vn_ln_b[l]), a.gelu = true;
         a.out_bf16 = sv.dvz_b, a.out_ld = I;
-        LLB_TRY(launch_row_ln_bwd(a, s));
-        LLB_TRY(kdone());
+        LLB_TRY(launch_row_ln_bwd(a, s, ctr));
         LLB_TRY(gemm_bias_act(sv.dvz_b, I, gw(R.vn0t[l]), I, nullptr, sv.dpool, Hp, B, Hp, I, LLB_ACT_NONE, true, s, &g->ctr));
       }
     }
@@ -298,11 +291,9 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
       a.gelu = !last;
       a.prod = sv.prod, a.prod_ld = 3 * Hp;
       if (l > 0) a.out_bf16 = sv.du_b, a.out_ld = Hp;
-      LLB_TRY(launch_row_ln_bwd(a, s));
-      LLB_TRY(kdone());
-      grad_segsum_kernel<<<dim3(B, ceil_div(3 * Hp, 256)), 256, 0, s>>>(sv.prod, 3 * Hp, sv.graph_ptr, 3 * Hp, nullptr, nullptr,
-                                                                           sv.dmod_b + (size_t)l * 3 * Hp, L * 3 * Hp);
-      LLB_TRY(kdone());
+      LLB_TRY(launch_row_ln_bwd(a, s, ctr));
+      LLB_TRY(launch_kernel(ctr, NO_PROF, false, grad_segsum_kernel, dim3(B, ceil_div(3 * Hp, 256)), dim3(256), 0, s, sv.prod, 3 * Hp, sv.graph_ptr,
+                            3 * Hp, nullptr, nullptr, sv.dmod_b + (size_t)l * 3 * Hp, L * 3 * Hp));
     }
     if (l == 0) break;   // nothing upstream of layer 0's tail depends on c
     // node MLP: du -> dz = du . W4 -> GELU' + LayerNorm(4H) backward on the centred first linear's output -> da = dz_c . W0c
@@ -317,29 +308,22 @@ int llb_gin_predictor_backward_c(llb_gin* g, int num_nodes, int num_edges, int n
       a.rows = n, a.width = I, a.valid = 4 * G.H;
       a.gamma = g->w<float>(G.mlp_ln_w[l]), a.beta = g->w<float>(G.mlp_ln_b[l]), a.gelu = true;
       a.out_bf16 = sv.dzpre_b, a.out_ld = I;
-      LLB_TRY(launch_row_ln_bwd(a, s));
-      LLB_TRY(kdone());
+      LLB_TRY(launch_row_ln_bwd(a, s, ctr));
     }
     g->ctr.slot = LLB_PROF_GIN_GEMM_MLP0;
     LLB_TRY(gemm_bias_act(sv.dzpre_b, I, gw(R.mlp0t[l]), I, nullptr, sv.da, Hp, n, Hp, I, LLB_ACT_NONE, true, s, &g->ctr));
-    {
-      ProfScope prof(LLB_PROF_GIN_AGGREGATE, s);
-      gin_grad_aggregate_kernel<<<ceil_div(n, 8), 256, 0, s>>>(hin, sv.da, sv.srowptr, sv.sdst, sv.seid, g->w<float>(G.bond_emb[l]),
-                                                               g->w<float>(G.eps[l]), sv.dh, n, Hp);
-    }
-    LLB_TRY(kdone());
-    if (!last) {
-      ProfScope prof(LLB_PROF_GIN_POOL, s);
-      gin_grad_route_max_kernel<<<seg_grid_h, 256, 0, s>>>(hin, sv.graph_ptr, sv.dpool, sv.dh, Hp);
-      LLB_TRY(kdone());
-    }
+    LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_AGGREGATE, false, gin_grad_aggregate_kernel, dim3(ceil_div(n, 8)), dim3(256), 0, s, hin, sv.da, sv.srowptr,
+                          sv.sdst, sv.seid, g->w<float>(G.bond_emb[l]), g->w<float>(G.eps[l]), sv.dh, n, Hp));
+    if (!last)
+      LLB_TRY(launch_kernel(ctr, LLB_PROF_GIN_POOL, false, gin_grad_route_max_kernel, seg_grid_h, dim3(256), 0, s, hin, sv.graph_ptr, sv.dpool, sv.dh,
+                            Hp));
   }
   // ---- condition: dctext = [dmod_0 | ... | dmod_{L-1}] . [W_adapter_0 | ... ]^T, dc = dctext * silu'(c)
   g->ctr.slot = LLB_PROF_GIN_MISC;
   LLB_TRY(gemm_bias_act(sv.dmod_b, L * 3 * Hp, gw(R.adaptert), L * 3 * Hp, nullptr, sv.dctext, G.tdim, B, G.tdim, L * 3 * Hp, LLB_ACT_NONE, true,
                         s, &g->ctr));
-  gin_grad_silu_kernel<<<grid_for((size_t)B * G.tdim), 256, 0, s>>>(c, sv.dctext, dc, (size_t)B * G.tdim);
-  return kdone();
+  return launch_kernel(ctr, NO_PROF, false, gin_grad_silu_kernel, grid_for((size_t)B * G.tdim), dim3(256), 0, s, c, sv.dctext, dc,
+                       (size_t)B * G.tdim);
 }
 
 }  // extern "C"

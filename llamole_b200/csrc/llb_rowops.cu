@@ -318,20 +318,22 @@ __global__ void __launch_bounds__(256) row_ln_reg_kernel(RowLnDev a) {
   }
 }
 
+using RowLnKernel = void (*)(RowLnDev);
+// The register-resident kernel of `nch` 128-column chunks, or null when there is no such variant.
 template <unsigned F>
-bool launch_reg(int nch, int grid, const RowLnDev& d, cudaStream_t stream) {
+RowLnKernel reg_variant(int nch) {
   switch (nch) {
-    case 1: return launch_pdl(row_ln_reg_kernel<1, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 2: return launch_pdl(row_ln_reg_kernel<2, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 4: return launch_pdl(row_ln_reg_kernel<4, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 6: return launch_pdl(row_ln_reg_kernel<6, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 8: return launch_pdl(row_ln_reg_kernel<8, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 12: return launch_pdl(row_ln_reg_kernel<12, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 16: return launch_pdl(row_ln_reg_kernel<16, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 24: return launch_pdl(row_ln_reg_kernel<24, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
-    case 32: return launch_pdl(row_ln_reg_kernel<32, F>, dim3(grid), dim3(256), 0, stream, d) == cudaSuccess;
+    case 1: return row_ln_reg_kernel<1, F>;
+    case 2: return row_ln_reg_kernel<2, F>;
+    case 4: return row_ln_reg_kernel<4, F>;
+    case 6: return row_ln_reg_kernel<6, F>;
+    case 8: return row_ln_reg_kernel<8, F>;
+    case 12: return row_ln_reg_kernel<12, F>;
+    case 16: return row_ln_reg_kernel<16, F>;
+    case 24: return row_ln_reg_kernel<24, F>;
+    case 32: return row_ln_reg_kernel<32, F>;
   }
-  return false;
+  return nullptr;
 }
 
 __global__ void f32_to_bf16_kernel(const float* __restrict__ src, int src_ld, __nv_bfloat16* __restrict__ dst, int dst_ld,
@@ -366,7 +368,7 @@ __global__ void __launch_bounds__(256) linear_f32_kernel(const float* __restrict
 
 }  // namespace
 
-int launch_row_ln(const RowLnArgs& a, cudaStream_t stream) {
+int launch_row_ln(const RowLnArgs& a, cudaStream_t stream, LaunchCounter* ctr) {
   if (a.rows <= 0) return LLB_OK;
   LLB_CHECK_ARG(a.width % 4 == 0 && a.in_ld % 4 == 0, "row_ln: width %d / ld %d must be multiples of 4", a.width, a.in_ld);
   LLB_CHECK_ARG((a.shift == nullptr) == (a.scale == nullptr), "row_ln: shift and scale come together");
@@ -378,7 +380,6 @@ int launch_row_ln(const RowLnArgs& a, cudaStream_t stream) {
   RowLnDev d{a.in, a.in_ld, a.in_bf16 ? 1 : 0, a.rows, a.width, a.normalize ? 1 : 0, a.in_parts, a.in_part_stride, a.gamma, a.beta, a.row_group,
              a.shift, a.scale, a.gate, a.mod_ld, a.act, a.resid, a.resid_ld, a.addvec, a.addvec_ld, a.out_f32,
              a.out_f32_ld, a.out_bf16, a.out_bf16_ld, a.dup_rows, a.l2_normalize ? 1 : 0, valid};
-  ProfScope prof(a.prof_slot, stream);
   const int grid = ceil_div(a.rows, 8);
   // all vector operands of the register path are read as float4
   const bool vec_ok = a.mod_ld % 4 == 0 && a.addvec_ld % 4 == 0 && a.resid_ld % 4 == 0 && a.out_f32_ld % 4 == 0 && a.out_bf16_ld % 4 == 0;
@@ -395,50 +396,43 @@ int launch_row_ln(const RowLnArgs& a, cudaStream_t stream) {
   constexpr unsigned V_ENC_LAST = F_NORM | F_GAMMA | F_RESID | F_OUT_F32 | F_OUT_BF16;
   constexpr unsigned V_PRED = F_NORM | F_MOD | F_GELU | F_GATE | F_RESID | F_ADDVEC | F_OUT_F32 | F_OUT_BF16;  // GIN predictor layer tail
   constexpr unsigned V_PRED_LAST = F_NORM | F_MOD | F_GATE | F_RESID | F_OUT_F32 | F_OUT_BF16;
-  bool done = false;
+  RowLnKernel kern = nullptr;
   if (nch > 0 && plain) {
-    if (f == V_DIT) done = launch_reg<V_DIT>(nch, grid, d, stream);
-    else if (f == V_MLP) done = launch_reg<V_MLP>(nch, grid, d, stream);
-    else if (f == V_ENC) done = launch_reg<V_ENC>(nch, grid, d, stream);
-    else if (f == V_ENC_LAST) done = launch_reg<V_ENC_LAST>(nch, grid, d, stream);
-    else if (f == V_PRED) done = launch_reg<V_PRED>(nch, grid, d, stream);
-    else if (f == V_PRED_LAST) done = launch_reg<V_PRED_LAST>(nch, grid, d, stream);
+    if (f == V_DIT) kern = reg_variant<V_DIT>(nch);
+    else if (f == V_MLP) kern = reg_variant<V_MLP>(nch);
+    else if (f == V_ENC) kern = reg_variant<V_ENC>(nch);
+    else if (f == V_ENC_LAST) kern = reg_variant<V_ENC_LAST>(nch);
+    else if (f == V_PRED) kern = reg_variant<V_PRED>(nch);
+    else if (f == V_PRED_LAST) kern = reg_variant<V_PRED_LAST>(nch);
   }
-  if (!done && nch > 0) done = launch_reg<F_RUNTIME>(nch, grid, d, stream);
-  if (!done) (void)launch_pdl(row_ln_kernel, dim3(grid), dim3(256), 0, stream, d);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  if (!kern && nch > 0) kern = reg_variant<F_RUNTIME>(nch);
+  if (!kern) kern = row_ln_kernel;   // no register variant for this width
+  return launch_kernel(ctr, a.prof_slot, true, kern, dim3(grid), dim3(256), 0, stream, d);
 }
 
-int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream) {
+int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream, LaunchCounter* ctr) {
   if (a.rows <= 0) return LLB_OK;
   LLB_CHECK_ARG(a.x && a.dy && a.valid >= 1 && a.valid <= a.width && a.dy_parts >= 1, "row_ln_bwd: bad argument (width %d, valid %d)",
                 a.width, a.valid);
   LLB_CHECK_ARG((a.shift == nullptr) == (a.scale == nullptr) && (a.gamma == nullptr) == (a.beta == nullptr) && !(a.gamma && a.scale),
                 "row_ln_bwd: gamma/beta or shift/scale, in pairs");
-  ProfScope prof(a.prof_slot, stream);
-  row_ln_bwd_kernel<<<ceil_div(a.rows, 8), 256, 0, stream>>>(a);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_kernel(ctr, a.prof_slot, false, row_ln_bwd_kernel, dim3(ceil_div(a.rows, 8)), dim3(256), 0, stream, a);
 }
 
 int launch_f32_to_bf16(const float* src, int src_ld, __nv_bfloat16* dst, int dst_ld, int rows, int cols, int pad_cols,
-                       cudaStream_t stream) {
+                       cudaStream_t stream, LaunchCounter* ctr) {
   if (rows <= 0) return LLB_OK;
   const size_t total = (size_t)rows * pad_cols;
   const int blocks = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-  f32_to_bf16_kernel<<<blocks, 256, 0, stream>>>(src, src_ld, dst, dst_ld, rows, cols, pad_cols);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_kernel(ctr, NO_PROF, false, f32_to_bf16_kernel, dim3(blocks), dim3(256), 0, stream, src, src_ld, dst, dst_ld, rows, cols, pad_cols);
 }
 
 int launch_linear_f32(const float* in, int in_ld, const float* W, int w_ld, const float* b, float* out, int out_ld,
-                      int rows, int out_f, int in_f, int act, cudaStream_t stream) {
+                      int rows, int out_f, int in_f, int act, cudaStream_t stream, LaunchCounter* ctr) {
   if (rows <= 0) return LLB_OK;
   const size_t warps = (size_t)rows * out_f;
-  linear_f32_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, stream>>>(in, in_ld, W, w_ld, b, out, out_ld, rows, out_f, in_f, act);
-  LLB_CUDA_OK(cudaGetLastError());
-  return LLB_OK;
+  return launch_kernel(ctr, NO_PROF, false, linear_f32_kernel, dim3((unsigned)((warps + 7) / 8)), dim3(256), 0, stream, in, in_ld, W, w_ld, b, out,
+                       out_ld, rows, out_f, in_f, act);
 }
 
 }  // namespace llb

@@ -1,4 +1,5 @@
-// Row-wise fused kernels shared by the GraphDiT and GIN paths (HBM-bound; one warp per row).
+// Row-wise fused kernels shared by the GraphDiT and GIN paths (HBM-bound; one warp per row).  Each launcher issues at most one
+// kernel (none for rows <= 0) and counts it on ctr, which may be null.
 #pragma once
 #include "llb_common.cuh"
 
@@ -37,7 +38,7 @@ struct RowLnArgs {
   bool l2_normalize = false;  // out = v / ||v|| instead of LN (GraphCLIP head)
   int prof_slot = LLB_PROF_LN_MOD_RES;
 };
-int launch_row_ln(const RowLnArgs& a, cudaStream_t stream);
+int launch_row_ln(const RowLnArgs& a, cudaStream_t stream, LaunchCounter* ctr);
 
 // Backward of the row LayerNorm above without residual / addvec (they pass the gradient through unchanged): with
 //   xh = LN(x) over the first `valid` columns,  t = xh * gamma + beta  or  xh * (1 + scale[g]) + shift[g],  out = gate[g] * act(t),
@@ -67,13 +68,13 @@ struct RowLnBwdArgs {
   int out_ld = 0;
   int prof_slot = LLB_PROF_GIN_ROWLN;
 };
-int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream);
+int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream, LaunchCounter* ctr);
 
 // fp32 (rows, cols) -> bf16 (rows, dst_ld) with zero padding up to pad_cols.
 int launch_f32_to_bf16(const float* src, int src_ld, __nv_bfloat16* dst, int dst_ld, int rows, int cols, int pad_cols,
-                       cudaStream_t stream);
+                       cudaStream_t stream, LaunchCounter* ctr);
 // out[r, o] = act(sum_k in[r,k] W[o,k] + b[o]) in fp32 on CUDA cores (tiny set-up linears only).
 int launch_linear_f32(const float* in, int in_ld, const float* W, int w_ld, const float* b, float* out, int out_ld,
-                      int rows, int out_f, int in_f, int act, cudaStream_t stream);
+                      int rows, int out_f, int in_f, int act, cudaStream_t stream, LaunchCounter* ctr);
 
 }  // namespace llb

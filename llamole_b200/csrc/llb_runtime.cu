@@ -4,6 +4,7 @@
 #include <stdlib.h>
 
 #include <mutex>
+#include <unordered_map>
 #include <vector>
 
 #include "llb_gemm.cuh"
@@ -71,6 +72,28 @@ void profile_begin(int slot, cudaStream_t s) {
   g_prof_recs.push_back(r);
 }
 void profile_end(cudaStream_t s) { cudaEventRecord(g_prof_recs.back().b, s); }
+
+int launch_failed(const void* kern, cudaError_t e) {
+  (void)cudaGetLastError();   // the launch's error is reported here, not by a later status check
+  const char* name = nullptr;
+  if (cudaFuncGetName(&name, kern) != cudaSuccess || !name) {
+    (void)cudaGetLastError();
+    name = "?";
+  }
+  return fail(LLB_ERR_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
+}
+
+int reserve_dynamic_smem(const void* kern, size_t smem) {
+  static std::mutex mu;
+  static std::unordered_map<const void*, size_t> reserved;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& have = reserved[kern];
+  if (smem <= have) return LLB_OK;
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return launch_failed(kern, e);
+  have = smem;
+  return LLB_OK;
+}
 
 bool pdl_enabled() {
   static int on = -1;
@@ -200,7 +223,7 @@ static int pick_bn(int M, int N, int K, int group_n = 0) {
 
 template <int ACT, bool F32>
 static int gemm_dispatch_bn(const void* A, int lda, const void* W, int ldw, const float* bias, void* C, int ldc, int M,
-                            int N, int K, cudaStream_t stream, GemmCounters* ctr, GemmGroups grp) {
+                            int N, int K, cudaStream_t stream, LaunchCounter* ctr, GemmGroups grp) {
   LLB_CHECK_ARG(bias == nullptr || (reinterpret_cast<uintptr_t>(bias) & 15) == 0, "gemm: bias must be 16-byte aligned");
   EpiBiasAct<ACT, F32> epi{C, ldc, bias};
   switch (pick_bn(M, N, K, grp.group_n)) {
@@ -212,7 +235,7 @@ static int gemm_dispatch_bn(const void* A, int lda, const void* W, int ldw, cons
 
 template <bool F32>
 static int gemm_dispatch_act(const void* A, int lda, const void* W, int ldw, const float* bias, void* C, int ldc, int M,
-                             int N, int K, int act, cudaStream_t stream, GemmCounters* ctr, GemmGroups grp) {
+                             int N, int K, int act, cudaStream_t stream, LaunchCounter* ctr, GemmGroups grp) {
   switch (act) {
     case LLB_ACT_NONE: return gemm_dispatch_bn<LLB_ACT_NONE, F32>(A, lda, W, ldw, bias, C, ldc, M, N, K, stream, ctr, grp);
     case LLB_ACT_GELU: return gemm_dispatch_bn<LLB_ACT_GELU, F32>(A, lda, W, ldw, bias, C, ldc, M, N, K, stream, ctr, grp);
@@ -224,7 +247,7 @@ static int gemm_dispatch_act(const void* A, int lda, const void* W, int ldw, con
 }
 
 int gemm_bias_act(const void* A, int lda, const void* W, int ldw, const float* bias, void* C, int ldc, int M, int N,
-                  int K, int act, bool out_f32, cudaStream_t stream, GemmCounters* ctr, GemmGroups grp) {
+                  int K, int act, bool out_f32, cudaStream_t stream, LaunchCounter* ctr, GemmGroups grp) {
   return out_f32 ? gemm_dispatch_act<true>(A, lda, W, ldw, bias, C, ldc, M, N, K, act, stream, ctr, grp)
                  : gemm_dispatch_act<false>(A, lda, W, ldw, bias, C, ldc, M, N, K, act, stream, ctr, grp);
 }
