@@ -101,7 +101,7 @@ typedef struct {
   int32_t depth;       /* transformer blocks */
   int32_t heads;       /* H / heads must be 64 */
   int32_t mlp_hidden;  /* int(H * mlp_ratio), multiple of 64 */
-  int32_t max_nodes;   /* N <= 64; joint token width d0 = 16 + 5 N */
+  int32_t max_nodes;   /* N <= 128 for sampling, <= 64 for the training entries below; joint token width d0 = 16 + 5 N */
   int32_t timesteps;   /* T */
   int32_t y_dim;       /* 10 */
   int32_t text_dim;    /* 768 */
@@ -207,7 +207,9 @@ int llb_dit_sample(llb_dit* h, int t_first, int t_last, uint64_t seed, const flo
  *     keeps the residual stream at every block-half boundary, the modulations, c and the batch bookkeeping, so a later call on
  *     the handle cannot change this forward's gradient; the buffer also holds the backward's scratch (one per forward).
  *   llb_dit_backward_c: dlogits (same shapes, fp32) -> dc (B,H) fp32 for the forward that filled `saved` (pass that forward's
- *     B and atom total).  Run-to-run bit-identical. */
+ *     B and atom total).  Run-to-run bit-identical.
+ * These entries (and llb_dit_denoise_c with a `saved` buffer) need max_nodes <= 64; llb_dit_denoise_c without one takes
+ * max_nodes up to 128, like the sampler. */
 int llb_dit_grad_packed_bytes(const llb_dit_config* cfg, size_t* bytes);
 int llb_dit_pack_grad_weights(llb_dit* h, void* grad_blob, size_t grad_bytes, llb_stream_t stream);
 int llb_dit_train_saved_bytes(const llb_dit_config* cfg, int B, int num_tokens, size_t* bytes);

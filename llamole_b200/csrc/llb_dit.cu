@@ -169,10 +169,22 @@ __global__ void dit_cond_fixup_kernel(float* __restrict__ cinv, const uint8_t* _
 
 using namespace llb;
 
-static size_t dit_step_smem(int N, int passes) {
+// t_in_smem = false: the T_GLOBAL step kernel, whose logit rows T stay in global memory
+static size_t dit_step_smem(int N, int passes, bool t_in_smem = true) {
   const int d0 = DIT_XC + DIT_EC * N;
-  return (size_t)passes * N * d0 * 4 + (size_t)passes * N * sizeof(NodeStats) + (size_t)N * DIT_EC * 4 + ((N + 15) & ~15) +
-         (size_t)N * N + 16;
+  return (t_in_smem ? (size_t)passes * N * d0 * 4 : 0) + (size_t)passes * N * sizeof(NodeStats) + (size_t)N * DIT_EC * 4 +
+         ((N + 15) & ~15) + (size_t)N * N + 16;
+}
+
+static int smem_per_block_optin() {
+  static int bytes = 0;
+  if (bytes == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&bytes, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (bytes <= 0) bytes = 48 * 1024;
+  }
+  return bytes;
 }
 
 static int dit_carve(llb_dit* h, void* ws, size_t ws_bytes, int B, int Mtok, size_t* need) {
@@ -272,8 +284,8 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
   const bool fused_ln = gemm_ln_supported(H, H) && gemm_ln_supported(H, F) && gemm_ln_enabled() && !latency_regime;
   // LLB_FUSED_LN=0: GEMM + row kernel everywhere; default: both block halves fused on the CTA-pair kernel when H = 1024
   // (other widths have no fused kernel: a full row must fit four pairs' tensor memory).
-  // LLB_ATTN=2: tcgen05 attention (two heads per 128-row tile, P in tensor memory; needs an even head count); default: mma.sync
-  // attention fed by TMA.
+  // LLB_ATTN=2: tcgen05 attention (two heads per 128-row tile, P in tensor memory; needs an even head count and molecules of at
+  // most 64 atoms); default: mma.sync attention fed by TMA, on a 64-row tile unless a molecule of the batch has more atoms.
   static const bool attn_umma_env = getenv("LLB_ATTN") && getenv("LLB_ATTN")[0] == '2';
   const bool attn_umma = attn_umma_env && L.heads % 2 == 0;
   const bool fused_pair = fused_ln;
@@ -300,13 +312,16 @@ static int dit_body(llb_dit* h, cudaStream_t s) {
       const int seqs = (share0 ? 1 : h->passes) * B;
       CUtensorMap tmQKV;
       LLB_TRY(make_tensor_map_2d(&tmQKV, h->qkv, 2, seqs / B * Mtok, 3 * H, 3 * H, DIT_DH, 64, 128));
-      if (attn_umma) {
+      if (attn_umma && h->max_n <= 64) {
         const int units = seqs * (L.heads / 2);
         LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, false, dit_attention_umma4_kernel, dim3(units < num_sms() ? units : num_sms()),
                               dim3(ATT4_THREADS), ATT4_SMEM, s, tmQKV, h->attn, h->mol_off, B, Mtok, H, L.heads, units));
-      } else {
-        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel, dim3((unsigned)(seqs * L.heads)), dim3(128), 0, s, tmQKV,
+      } else if (h->max_n <= 64) {
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel<64>, dim3((unsigned)(seqs * L.heads)), dim3(128), 0, s, tmQKV,
                               h->attn, h->mol_off, B, Mtok, H, L.heads));
+      } else {
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel<128>, dim3((unsigned)(seqs * L.heads)), dim3(256),
+                              ATTT_SMEM128, s, tmQKV, h->attn, h->mol_off, B, Mtok, H, L.heads));
       }
     }
     // x += gate * (LN(linear(.)) (1 + scale) + shift): fused into the GEMM epilogue when a cluster can hold a full row
@@ -457,6 +472,16 @@ static int dit_forward(llb_dit* h, int t, cudaStream_t s) {
 
 static int dit_launch_step(llb_dit* h, DitStepArgs& a, cudaStream_t s) {
   const size_t smem = dit_step_smem(h->L.N, a.passes);
+  if (smem > (size_t)smem_per_block_optin()) {
+    // T does not fit (N > 71 with guidance): its home is the raw output-layer rows, row (p, atom i) = raw row p Mtok + off + i
+    // (raw_ld >= d0).  Nothing reads those rows after the step kernel: the next denoiser pass rewrites them, the logits dump
+    // returns T itself, and the backward recomputes its own copy from the saved residual stream.
+    a.tg = h->raw, a.tg_ld = h->raw_ld;
+    const size_t gsmem = dit_step_smem(h->L.N, a.passes, false);
+    if (h->B <= num_sms())
+      return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<512, true>, dim3(h->B), dim3(512), gsmem, s, a, h->tables);
+    return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<256, true>, dim3(h->B), dim3(256), gsmem, s, a, h->tables);
+  }
   if (h->B <= num_sms())   // fewer molecules than SMs: wider CTAs
     return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<512>, dim3(h->B), dim3(512), smem, s, a, h->tables);
   return launch_kernel(&h->ctr, LLB_PROF_DIT_STEP, false, dit_step_kernel<256>, dim3(h->B), dim3(256), smem, s, a, h->tables);
@@ -483,11 +508,13 @@ static int dit_bind(llb_dit* h, void* workspace, size_t workspace_bytes, int B, 
     off[b + 1] = off[b] + n_nodes_host[b];
   }
   const int Mtok = off[B];
+  int max_n = 0;
+  for (int b = 0; b < B; ++b) max_n = n_nodes_host[b] > max_n ? n_nodes_host[b] : max_n;
   size_t need = 0;
   LLB_TRY(dit_carve(h, workspace, workspace_bytes, B, Mtok, &need));
   if (need > workspace_bytes) return fail(LLB_ERR_WORKSPACE, "dit: workspace needs %zu bytes, got %zu", need, workspace_bytes);
   h->drop_graph();   // the captured launches carry the previous binding's pointers and sizes
-  h->B = B, h->Mtok = Mtok, h->mol_base = mol_index_base;
+  h->B = B, h->Mtok = Mtok, h->mol_base = mol_index_base, h->max_n = max_n;
   std::vector<int32_t> row_mol(Mtok > 0 ? Mtok : 1), row_group(h->passes * Mtok > 0 ? h->passes * Mtok : 1);
   for (int b = 0; b < B; ++b)
     for (int r = off[b]; r < off[b + 1]; ++r) {
@@ -691,6 +718,7 @@ int llb_dit_denoise_c(llb_dit* h, void* workspace, size_t workspace_bytes, int B
   cudaStream_t s = (cudaStream_t)stream;
   const DitLayout& L = h->L;
   const int H = L.H;
+  if (saved) LLB_TRY(dit_grad_check_n(L, "llb_dit_denoise_c with a saved buffer"));
   LLB_TRY(dit_bind(h, workspace, workspace_bytes, B, n_nodes_host, 0, s));
   const int Mtok = h->Mtok;
   DitSaved sv{};

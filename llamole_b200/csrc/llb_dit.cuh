@@ -26,6 +26,8 @@ struct DitLayout {
 };
 
 int make_layout(const llb_dit_config& c, DitLayout& L);
+// The backward of the denoiser (and the saved forward that feeds it) is built for at most DIT_GRAD_MAXN atoms per molecule.
+int dit_grad_check_n(const DitLayout& L, const char* entry);
 
 // What llb_dit_denoise_c keeps for llb_dit_backward_c, carved from the caller's `saved` buffer (dit_saved_carve).  The first
 // group is written by the forward; the rest is scratch of the backward.  The batch bookkeeping is copied too, so that a later
@@ -72,6 +74,7 @@ struct llb_dit {
   llb::LaunchCounter ctr;
   // batch binding
   int B = 0, Mtok = 0, passes = 2;
+  int max_n = 0;                 // atoms of the batch's largest molecule: picks the attention tile
   int64_t mol_base = 0;
   // workspace carve-up
   float* x = nullptr;            // (M,H) residual stream fp32

@@ -68,7 +68,7 @@ __global__ void __launch_bounds__(256) dit_grad_out_tail_kernel(const float* __r
                                                                 const int32_t* __restrict__ mol_off, const float* __restrict__ dX,
                                                                 const float* __restrict__ dE, int N, __nv_bfloat16* __restrict__ draw,
                                                                 int draw_ld, float* __restrict__ dmodout) {
-  __shared__ float s_mean[DIT_MAXN], s_rstd[DIT_MAXN];
+  __shared__ float s_mean[DIT_GRAD_MAXN], s_rstd[DIT_GRAD_MAXN];
   const int b = blockIdx.x;
   const int d0 = DIT_XC + DIT_EC * N;
   const int off = mol_off[b], n = mol_off[b + 1] - off;
@@ -175,7 +175,7 @@ __global__ void dit_grad_sum_slices_kernel(const float* __restrict__ parts, int 
 //   dq^ = dS k^ dh^-1/2,  dk^ = dS^T q^ dh^-1/2,  back through both LayerNorms,
 // and writes dqkv (rows, 3H) bf16 in the [q | k | v] head-major layout of the qkv linear.  fp32 throughout, in shared memory.
 constexpr int AG_LD = DIT_DH + 1;
-constexpr int AG_SMEM = (8 * DIT_MAXN * AG_LD + 4 * DIT_DH + 4 * DIT_MAXN) * 4;
+constexpr int AG_SMEM = (8 * DIT_GRAD_MAXN * AG_LD + 4 * DIT_DH + 4 * DIT_GRAD_MAXN) * 4;
 
 __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __restrict__ qkv_raw, const __nv_bfloat16* __restrict__ v_b,
                                                                  const __nv_bfloat16* __restrict__ dO, const int32_t* __restrict__ mol_off,
@@ -184,14 +184,14 @@ __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __
                                                                  __nv_bfloat16* __restrict__ dqkv) {
   extern __shared__ float ag[];
   float* Qx = ag;                         // normalised q (xh), then dq^
-  float* Kx = Qx + DIT_MAXN * AG_LD;      // normalised k, then dk^
-  float* Qh = Kx + DIT_MAXN * AG_LD;      // q^ = xh w + b
-  float* Kh = Qh + DIT_MAXN * AG_LD;
-  float* V = Kh + DIT_MAXN * AG_LD;
-  float* G = V + DIT_MAXN * AG_LD;        // dO
-  float* P = G + DIT_MAXN * AG_LD;
-  float* dS = P + DIT_MAXN * AG_LD;
-  float* wq = dS + DIT_MAXN * AG_LD;      // qw, qb, kw, kb
+  float* Kx = Qx + DIT_GRAD_MAXN * AG_LD; // normalised k, then dk^
+  float* Qh = Kx + DIT_GRAD_MAXN * AG_LD; // q^ = xh w + b
+  float* Kh = Qh + DIT_GRAD_MAXN * AG_LD;
+  float* V = Kh + DIT_GRAD_MAXN * AG_LD;
+  float* G = V + DIT_GRAD_MAXN * AG_LD;   // dO
+  float* P = G + DIT_GRAD_MAXN * AG_LD;
+  float* dS = P + DIT_GRAD_MAXN * AG_LD;
+  float* wq = dS + DIT_GRAD_MAXN * AG_LD; // qw, qb, kw, kb
   float* st = wq + 4 * DIT_DH;            // q rstd, k rstd, rowsum(P dP), spare
   const int b = blockIdx.x / heads, hd = blockIdx.x % heads;
   const int off = mol_off[b], n = mol_off[b + 1] - off;
@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __
     x[lane] = d0 * rstd, x[lane + 32] = d1 * rstd;
     y[lane] = fmaf(d0 * rstd, w[lane], w[DIT_DH + lane]);
     y[lane + 32] = fmaf(d1 * rstd, w[lane + 32], w[DIT_DH + lane + 32]);
-    if (lane == 0) st[which * DIT_MAXN + i] = rstd;
+    if (lane == 0) st[which * DIT_GRAD_MAXN + i] = rstd;
   }
   __syncthreads();
   // S -> P (row-wise softmax over the n keys), dP = dO V^T
@@ -259,9 +259,9 @@ __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __
     for (int i = 0; i < n; ++i) dv = fmaf(P[i * AG_LD + j], G[i * AG_LD + d], dv);
     dqkv[(size_t)(off + j) * ld3 + 2 * H + c0 + d] = __float2bfloat16(dv);
   }
-  float dq[DIT_MAXN * DIT_DH / 256], dk[DIT_MAXN * DIT_DH / 256];
+  float dq[DIT_GRAD_MAXN * DIT_DH / 256], dk[DIT_GRAD_MAXN * DIT_DH / 256];
 #pragma unroll
-  for (int r = 0; r < DIT_MAXN * DIT_DH / 256; ++r) {
+  for (int r = 0; r < DIT_GRAD_MAXN * DIT_DH / 256; ++r) {
     const int idx = tid + 256 * r;
     const int i = idx / DIT_DH, d = idx % DIT_DH;
     float aq = 0.f, ak = 0.f;
@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __
   __syncthreads();
   // the LayerNorm backward needs the whole row: park dq^ (times gamma) in Qh, dk^ in Kh
 #pragma unroll
-  for (int r = 0; r < DIT_MAXN * DIT_DH / 256; ++r) {
+  for (int r = 0; r < DIT_GRAD_MAXN * DIT_DH / 256; ++r) {
     const int idx = tid + 256 * r;
     const int i = idx / DIT_DH, d = idx % DIT_DH;
     if (i < n) Qh[i * AG_LD + d] = dq[r] * wq[d], Kh[i * AG_LD + d] = dk[r] * wq[2 * DIT_DH + d];
@@ -288,7 +288,7 @@ __global__ void __launch_bounds__(256) dit_grad_attention_kernel(const float* __
     const float* g = (which ? Kh : Qh) + i * AG_LD;
     const float g0 = g[lane], g1 = g[lane + 32], x0 = x[lane], x1 = x[lane + 32];
     const float m1 = warp_sum(g0 + g1) * (1.0f / DIT_DH), m2 = warp_sum(g0 * x0 + g1 * x1) * (1.0f / DIT_DH);
-    const float rstd = st[which * DIT_MAXN + i];
+    const float rstd = st[which * DIT_GRAD_MAXN + i];
     __nv_bfloat16* o = dqkv + (size_t)(off + i) * ld3 + which * H + c0;
     o[lane] = __float2bfloat16(rstd * (g0 - m1 - x0 * m2));
     o[lane + 32] = __float2bfloat16(rstd * (g1 - m1 - x1 * m2));
@@ -335,6 +335,11 @@ void dit_saved_carve(const DitLayout& L, void* saved, int B, int Mtok, DitSaved*
   *bytes = align_up(a.off, 256);
 }
 
+int dit_grad_check_n(const DitLayout& L, const char* entry) {
+  LLB_CHECK_ARG(L.N <= DIT_GRAD_MAXN, "%s: max_nodes=%d must be in [1,%d] (the denoiser's backward)", entry, L.N, DIT_GRAD_MAXN);
+  return LLB_OK;
+}
+
 }  // namespace llb
 
 using namespace llb;
@@ -345,6 +350,7 @@ int llb_dit_grad_packed_bytes(const llb_dit_config* cfg, size_t* bytes) {
   LLB_CHECK_ARG(cfg && bytes, "llb_dit_grad_packed_bytes: null argument");
   DitLayout L;
   LLB_TRY(make_layout(*cfg, L));
+  LLB_TRY(dit_grad_check_n(L, "llb_dit_grad_packed_bytes"));
   DitGradLayout R;
   make_grad_layout(L, R);
   *bytes = R.total;
@@ -355,6 +361,7 @@ int llb_dit_train_saved_bytes(const llb_dit_config* cfg, int B, int num_tokens, 
   LLB_CHECK_ARG(cfg && bytes && B >= 1 && num_tokens >= 0, "llb_dit_train_saved_bytes: bad argument");
   DitLayout L;
   LLB_TRY(make_layout(*cfg, L));
+  LLB_TRY(dit_grad_check_n(L, "llb_dit_train_saved_bytes"));
   LLB_CHECK_ARG(num_tokens <= B * L.N, "llb_dit_train_saved_bytes: %d tokens exceed %d molecules of at most %d atoms", num_tokens, B, L.N);
   dit_saved_carve(L, nullptr, B, num_tokens, nullptr, bytes);
   return LLB_OK;
@@ -363,6 +370,7 @@ int llb_dit_train_saved_bytes(const llb_dit_config* cfg, int B, int num_tokens, 
 int llb_dit_pack_grad_weights(llb_dit* h, void* grad_blob, size_t grad_bytes, llb_stream_t stream) {
   LLB_CHECK_ARG(h && grad_blob, "llb_dit_pack_grad_weights: null argument");
   const DitLayout& L = h->L;
+  LLB_TRY(dit_grad_check_n(L, "llb_dit_pack_grad_weights"));
   DitGradLayout R;
   make_grad_layout(L, R);
   if (grad_bytes < R.total) return fail(LLB_ERR_WORKSPACE, "dit: grad blob needs %zu bytes, got %zu", R.total, grad_bytes);
@@ -394,6 +402,7 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
   LLB_CHECK_ARG(h && saved && grad_blob && dlogits_X && dlogits_E && dc, "llb_dit_backward_c: null argument");
   LLB_CHECK_ARG(B >= 1 && num_tokens >= 0 && num_tokens <= B * h->L.N, "llb_dit_backward_c: bad batch size");
   const DitLayout& L = h->L;
+  LLB_TRY(dit_grad_check_n(L, "llb_dit_backward_c"));
   DitGradLayout R;
   make_grad_layout(L, R);
   if (grad_bytes < R.total) return fail(LLB_ERR_WORKSPACE, "dit: grad blob needs %zu bytes, got %zu", R.total, grad_bytes);
@@ -475,7 +484,7 @@ int llb_dit_backward_c(llb_dit* h, int B, int num_tokens, void* saved, size_t sa
       {
         CUtensorMap tmQKV;
         LLB_TRY(make_tensor_map_2d(&tmQKV, sv.qkv, 2, M, 3 * H, 3 * H, DIT_DH, 64, 128));
-        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel, dim3((unsigned)(B * L.heads)), dim3(128), 0, s, tmQKV, sv.attn,
+        LLB_TRY(launch_kernel(ctr, LLB_PROF_ATTENTION, true, dit_attention_tma_kernel<64>, dim3((unsigned)(B * L.heads)), dim3(128), 0, s, tmQKV, sv.attn,
                               sv.mol_off, B, M, H, L.heads));
       }
       ctr->slot = LLB_PROF_GEMM_PROJ;

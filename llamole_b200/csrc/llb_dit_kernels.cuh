@@ -10,7 +10,8 @@ namespace llb {
 constexpr int DIT_XC = 16;  // atom classes
 constexpr int DIT_EC = 5;   // bond classes
 constexpr int DIT_DH = 64;  // head dim (fixed)
-constexpr int DIT_MAXN = 64;
+constexpr int DIT_MAXN = 128;        // atoms per molecule of the sampler
+constexpr int DIT_GRAD_MAXN = 64;    // atoms per molecule of the denoiser's backward (llb_dit_grad.cu)
 
 // ------------------------------------------------------------------------------------------------
 // QKV GEMM epilogue: per-head affine LayerNorm on q and k (layers.py:49-50,66), softmax scale folded into q.
@@ -93,9 +94,9 @@ static __global__ void dit_cvec_kernel(const float* __restrict__ c1_t, const flo
 }
 
 // ------------------------------------------------------------------------------------------------
-// Attention over one (sequence, head): n <= 64 tokens, dh = 64 (layers.py:68-81; only valid tokens exist
+// Attention over one (sequence, head): n <= ROWS tokens, dh = 64 (layers.py:68-81; only valid tokens exist
 // in the packed layout, which is output-identical to the reference's masking, SURVEY.md section 8a-6).
-// 4 warps, warp w owns query rows [16w, 16w+16).  S = Q K^T and O = P V on mma.sync.m16n8k16 (bf16, fp32 acc).
+// ROWS / 16 warps, warp w owns query rows [16w, 16w+16).  S = Q K^T and O = P V on mma.sync.m16n8k16 (bf16, fp32 acc).
 // q is pre-scaled by dh^-0.5 * log2(e) so the softmax is exp2(s - max).
 // ------------------------------------------------------------------------------------------------
 constexpr int ATT_LD = 72;  // padded smem row (bf16 elements): conflict-free ldmatrix
@@ -119,17 +120,32 @@ __device__ __forceinline__ void mma_bf16_16816(float* c, uint32_t a0, uint32_t a
 // without padding) and the CTA waits on one mbarrier.  Rows past the end of the sequence hold the next sequence's
 // tokens (or zeros past the end of the matrix): keys >= n are masked to -inf exactly as before, so they contribute
 // p = 0 times a finite value; queries >= n are never stored.
+// ROWS = 64 is the kernel of every batch whose molecules have at most 64 atoms.  ROWS = 128 (a batch with a larger molecule):
+// 8 warps, 128 keys, each operand two 64-row boxes stacked in a 16 KB tile (the 128-byte swizzle repeats every 8 rows, so the
+// stacked boxes are one 128-row swizzled tile); the second box is loaded only for a molecule of more than 64 atoms, since rows
+// >= 64 of a smaller one are never read.  Its three tiles exceed the 48 KB of static shared memory: dynamic, ATTT_SMEM128 bytes.
 // ------------------------------------------------------------------------------------------------
-constexpr int ATTT_TILE = 64 * DIT_DH * 2;   // one 64-row operand tile (8 KB)
+constexpr int ATTT_TILE = 64 * DIT_DH * 2;   // one 64-row operand box (8 KB)
+constexpr int ATTT_SMEM128 = 3 * 2 * ATTT_TILE + 1024;   // dynamic shared memory of the 128-row kernel (+ slack to align to 1 KB)
 
 __device__ __forceinline__ uint32_t attt_swz(int row, int chunk) { return (uint32_t)(row * 128 + ((chunk ^ (row & 7)) << 4)); }
 
-static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __grid_constant__ CUtensorMap tmQKV, __nv_bfloat16* __restrict__ out,
-                                                                const int32_t* __restrict__ mol_off, int B, int Mtok, int H, int heads) {
+template <int ROWS>
+static __global__ void __launch_bounds__(2 * ROWS) dit_attention_tma_kernel(const __grid_constant__ CUtensorMap tmQKV, __nv_bfloat16* __restrict__ out,
+                                                                     const int32_t* __restrict__ mol_off, int B, int Mtok, int H, int heads) {
+  static_assert(ROWS == 64 || ROWS == 128, "dit attention: 64- or 128-row tile");
+  constexpr int TILE = ROWS * DIT_DH * 2;   // one operand tile
+  constexpr int KT = ROWS / 8;              // key tiles of 8
   pdl_launch_dependents();
   LLB_STAMP(0x1A, 0, threadIdx.x == 0);
-  __shared__ __align__(1024) uint8_t tiles[3 * ATTT_TILE];
+  // (the 64-row tile is static shared memory, declared ahead of the barrier as it always was)
+  __shared__ __align__(1024) uint8_t tiles64[ROWS == 64 ? 3 * TILE : 1];
   __shared__ __align__(8) uint64_t bar;
+  uint8_t* tiles = tiles64;
+  if constexpr (ROWS == 128) {
+    extern __shared__ uint8_t att_dyn_smem[];
+    tiles = att_dyn_smem + ((1024u - (smem_u32(att_dyn_smem) & 1023u)) & 1023u);
+  }
   const int head = blockIdx.x % heads;
   const int seq = blockIdx.x / heads;  // pass * B + molecule
   const int b = seq % B, pass = seq / B;
@@ -148,25 +164,33 @@ static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __g
   LLB_STAMP(0x2A, 0, threadIdx.x == 0);
   if (n == 0) return;
   if (tid == 0) {
-    mbar_arrive_expect_tx(&bar, 3 * ATTT_TILE);
+    if constexpr (ROWS == 64) {
+      mbar_arrive_expect_tx(&bar, 3 * ATTT_TILE);
 #pragma unroll
-    for (int mat = 0; mat < 3; ++mat) tma_load_2d(tiles + mat * ATTT_TILE, &tmQKV, &bar, mat * H + head * DIT_DH, row0);
+      for (int mat = 0; mat < 3; ++mat) tma_load_2d(tiles + mat * ATTT_TILE, &tmQKV, &bar, mat * H + head * DIT_DH, row0);
+    } else {
+      const int boxes = n > 64 ? 2 : 1;
+      mbar_arrive_expect_tx(&bar, 3 * boxes * ATTT_TILE);
+      for (int mat = 0; mat < 3; ++mat)
+        for (int hb = 0; hb < boxes; ++hb)
+          tma_load_2d(tiles + mat * TILE + hb * ATTT_TILE, &tmQKV, &bar, mat * H + head * DIT_DH, row0 + 64 * hb);
+    }
   }
   if (warp * 16 >= n) return;
-  const uint32_t sQ = smem_u32(tiles), sK = sQ + ATTT_TILE, sV = sK + ATTT_TILE;
+  const uint32_t sQ = smem_u32(tiles), sK = sQ + TILE, sV = sK + TILE;
   const int npad = (n + 15) & ~15;
   const int ntiles = npad >> 3;  // key tiles of 8
   mbar_wait(&bar, 0);
   // ---- S = Q K^T
-  float s[8][4];
+  float s[KT][4];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) s[j][0] = s[j][1] = s[j][2] = s[j][3] = 0.f;
+  for (int j = 0; j < KT; ++j) s[j][0] = s[j][1] = s[j][2] = s[j][3] = 0.f;
 #pragma unroll
   for (int ks = 0; ks < 4; ++ks) {
     uint32_t a0, a1, a2, a3;
     ldsm_x4(sQ + attt_swz(warp * 16 + (lane & 7) + ((lane >> 3) & 1) * 8, ks * 2 + (lane >> 4)), a0, a1, a2, a3);
 #pragma unroll
-    for (int jp = 0; jp < 4; ++jp) {
+    for (int jp = 0; jp < KT / 2; ++jp) {
       if (jp * 2 < ntiles) {
         uint32_t b0, b1, b2, b3;
         ldsm_x4(sK + attt_swz(jp * 16 + (lane & 7) + (lane >> 4) * 8, ks * 2 + ((lane >> 3) & 1)), b0, b1, b2, b3);
@@ -179,7 +203,7 @@ static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __g
   const int t4 = lane & 3;
   float m0 = -INFINITY, m1 = -INFINITY;
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
+  for (int j = 0; j < KT; ++j) {
 #pragma unroll
     for (int e = 0; e < 2; ++e) {
       const int key = j * 8 + t4 * 2 + e;
@@ -193,9 +217,9 @@ static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __g
   m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1));
   m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
   float l0 = 0.f, l1 = 0.f;
-  uint32_t p[8][2];
+  uint32_t p[KT][2];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
+  for (int j = 0; j < KT; ++j) {
     const float e0 = ex2_approx(s[j][0] - m0), e1 = ex2_approx(s[j][1] - m0);   // MUFU.EX2 alone: exp2f adds a range fix-up per call
     const float e2 = ex2_approx(s[j][2] - m1), e3 = ex2_approx(s[j][3] - m1);
     l0 += e0 + e1;
@@ -212,7 +236,7 @@ static __global__ void __launch_bounds__(128) dit_attention_tma_kernel(const __g
 #pragma unroll
   for (int j = 0; j < 8; ++j) o[j][0] = o[j][1] = o[j][2] = o[j][3] = 0.f;
 #pragma unroll
-  for (int ks = 0; ks < 4; ++ks) {
+  for (int ks = 0; ks < KT / 2; ++ks) {
     if (ks * 16 < npad) {
       const uint32_t a0 = p[2 * ks][0], a1 = p[2 * ks][1], a2 = p[2 * ks + 1][0], a3 = p[2 * ks + 1][1];
 #pragma unroll
@@ -492,6 +516,9 @@ struct DitStepArgs {
   float* dumpE;      // optional (B,N,N,5)
   int dump_pass;
   int dump_logits;
+  // T_GLOBAL step kernel only: T's rows in global memory, row (pass p, atom i of molecule b) at (p Mtok + mol_off[b] + i) tg_ld
+  float* tg;
+  int tg_ld;
 };
 
 // Per-node statistics of one pass kept in shared memory.
@@ -524,9 +551,12 @@ __device__ __forceinline__ float post_term(float v, float ux, float p, float pu,
 }
 
 // Dynamic shared memory: T[pass][n][d0] logits rows (fp32), then NodeStats[pass][n], then small arrays.
+// T_GLOBAL (T does not fit a block's shared memory: 2 N d0 4 bytes is 186 KB at N = 64, 701 KB at N = 128): T lives in
+// global memory at a.tg and shared memory starts at NodeStats.  A template parameter rather than a pointer chosen at run time,
+// so that the shared-memory instantiations keep shared-memory (not generic) loads and stores.
 // THREADS = 256 (two CTAs per SM at throughput batch sizes) or 512 (a handful of molecules: one CTA per molecule is all the
 // parallelism there is, so each gets more threads); every loop strides by blockDim.x.
-template <int THREADS>
+template <int THREADS, bool T_GLOBAL = false>
 static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a, const __grid_constant__ DitTablesDev tb) {
   LLB_STAMP(0x1C, 0, threadIdx.x == 0);
   extern __shared__ __align__(16) float sm[];
@@ -539,7 +569,14 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
   int8_t* Eg = a.E + (size_t)b * N * N;
 
   float* T = sm;                                                       // passes * N * d0
-  NodeStats* stats = reinterpret_cast<NodeStats*>(T + (size_t)a.passes * N * d0);   // passes * N
+  const int ld = T_GLOBAL ? a.tg_ld : d0;                              // row stride of T
+  auto tpass = [&](int p) -> float* {                                  // row 0 of pass p
+    return T_GLOBAL ? a.tg + ((size_t)p * a.Mtok + off) * ld : T + (size_t)p * N * d0;
+  };
+  auto trow = [&](int p, int i) -> float* {                            // row i of pass p
+    return T_GLOBAL ? a.tg + ((size_t)p * a.Mtok + off + i) * ld : T + ((size_t)p * N + i) * d0;
+  };
+  NodeStats* stats = reinterpret_cast<NodeStats*>(T_GLOBAL ? sm : T + (size_t)a.passes * N * d0);   // passes * N
   float* cnt = reinterpret_cast<float*>(stats + a.passes * N);         // N * 5
   int8_t* sX = reinterpret_cast<int8_t*>(cnt + N * DIT_EC);            // N
   int8_t* sE = sX + ((N + 15) & ~15);                                  // N * N
@@ -563,11 +600,11 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
       const float* scale = shift + d0;
       for (int i = warp; i < n; i += nthreads / 32) {
         const float* src = a.raw + (size_t)(p * a.Mtok + off + i) * a.raw_ld;
-        float* dst = T + ((size_t)p * N + i) * d0;
+        float* dst = trow(p, i);   // with T_GLOBAL: src itself
         float s = 0.f;
         for (int k = lane; k < d0; k += 32) {
           const float v = src[k];
-          dst[k] = v;
+          if constexpr (!T_GLOBAL) dst[k] = v;
           s += v;
         }
         const float mean = warp_sum(s) / (float)d0;
@@ -583,19 +620,19 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
     __syncthreads();
     // atoms: + one-hot; bonds: symmetrise valid off-diagonal pairs, zero the rest
     for (int p = 0; p < a.passes; ++p) {
-      float* Tp = T + (size_t)p * N * d0;
+      float* Tp = tpass(p);
       for (int idx = tid; idx < n * DIT_XC; idx += nthreads) {
         const int i = idx / DIT_XC, c = idx % DIT_XC;
-        Tp[i * d0 + c] += (sX[i] == c) ? 1.0f : 0.0f;
+        Tp[i * ld + c] += (sX[i] == c) ? 1.0f : 0.0f;
       }
       for (int idx = tid; idx < n * N; idx += nthreads) {
         const int i = idx / N, j = idx % N;
-        float* tij = Tp + i * d0 + DIT_XC + DIT_EC * j;
+        float* tij = Tp + i * ld + DIT_XC + DIT_EC * j;
         if (j >= n || j == i) {
 #pragma unroll
           for (int e = 0; e < DIT_EC; ++e) tij[e] = 0.f;
         } else if (i < j) {
-          float* tji = Tp + j * d0 + DIT_XC + DIT_EC * i;
+          float* tji = Tp + j * ld + DIT_XC + DIT_EC * i;
           const int et = sE[i * N + j];
 #pragma unroll
           for (int e = 0; e < DIT_EC; ++e) {
@@ -611,10 +648,10 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
     for (int p = 0; p < a.passes; ++p) {
       const float* lX = (p == 0 ? a.lcX : a.luX) + (size_t)b * N * DIT_XC;
       const float* lE = (p == 0 ? a.lcE : a.luE) + (size_t)b * N * N * DIT_EC;
-      float* Tp = T + (size_t)p * N * d0;
+      float* Tp = tpass(p);
       for (int idx = tid; idx < n * d0; idx += nthreads) {
         const int i = idx / d0, k = idx % d0;
-        Tp[i * d0 + k] = k < DIT_XC ? lX[i * DIT_XC + k] : lE[(size_t)i * N * DIT_EC + (k - DIT_XC)];
+        Tp[i * ld + k] = k < DIT_XC ? lX[i * DIT_XC + k] : lE[(size_t)i * N * DIT_EC + (k - DIT_XC)];
       }
     }
     __syncthreads();
@@ -622,16 +659,16 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
 
   if (a.dump_logits) {
     // masked logits in the reference's dense layout (zeros outside the valid block)
-    const float* Tp = T + (size_t)a.dump_pass * N * d0;
+    const float* Tp = tpass(a.dump_pass);
     float* oX = a.dumpX + (size_t)b * N * DIT_XC;
     float* oE = a.dumpE + (size_t)b * N * N * DIT_EC;
     for (int idx = tid; idx < N * DIT_XC; idx += nthreads) {
       const int i = idx / DIT_XC;
-      oX[idx] = i < n ? Tp[i * d0 + idx % DIT_XC] : 0.f;
+      oX[idx] = i < n ? Tp[i * ld + idx % DIT_XC] : 0.f;
     }
     for (int idx = tid; idx < N * N * DIT_EC; idx += nthreads) {
       const int i = idx / (N * DIT_EC), k = idx % (N * DIT_EC);
-      oE[idx] = (i < n && k / DIT_EC < n) ? Tp[i * d0 + DIT_XC + k] : 0.f;
+      oE[idx] = (i < n && k / DIT_EC < n) ? Tp[i * ld + DIT_XC + k] : 0.f;
     }
     if (!a.sample) return;
   }
@@ -646,7 +683,7 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
   }
   for (int idx = warp; idx < a.passes * n; idx += nthreads / 32) {
     const int p = idx / n, i = idx % n;
-    const float* ti = T + ((size_t)p * N + i) * d0;
+    const float* ti = trow(p, i);
     NodeStats& st = stats[p * N + i];
     // atom softmax (16 logits: lanes 0..15)
     float l = lane < DIT_XC ? ti[lane] : -INFINITY;
@@ -775,7 +812,7 @@ static __global__ void __launch_bounds__(THREADS) dit_step_kernel(DitStepArgs a,
     for (int p = 0; p < a.passes; ++p) {
       const NodeStats& st = stats[p * N + i];
       float pe[DIT_EC];
-      softmax5(T + ((size_t)p * N + i) * d0 + DIT_XC + DIT_EC * j, pe);
+      softmax5(trow(p, i) + DIT_XC + DIT_EC * j, pe);
       const float Ssum = (st.S[0] + st.S[1]) + (st.S[2] + st.S[3]) + st.S[4];
       float un[DIT_EC], sum = 0.f;
 #pragma unroll

@@ -195,7 +195,8 @@ class GraphDiT(nn.Module):
         return graphdit_loss(self, x, edge_index, edge_attr, graph_batch, properties, text_embedding, no_label_index)
 
     def device_denoiser_ok(self) -> bool:
-        """Whether `forward` runs the denoiser on the sm_100a kernels (see `forward`)."""
+        """Whether `forward` runs the denoiser on the sm_100a kernels (see `forward`).  The sampler takes molecules of up to 128
+        atoms, the device denoiser's backward up to 64: a checkpoint with a larger max_node trains through the eager loss."""
         params = list(self.denoiser.parameters())
         dev = params[0].device
         if dev.type != "cuda" or any(p.requires_grad for p in params):
@@ -206,8 +207,10 @@ class GraphDiT(nn.Module):
             return False
         idx = dev.index if dev.index is not None else torch.cuda.current_device()
         nbytes = C.c_size_t()
+        cfg = _dit_config(self)
         return lib.llb_arch_check(idx) == _cabi.LLB_OK and \
-            lib.llb_dit_packed_bytes(C.byref(_dit_config(self)), C.byref(nbytes)) == _cabi.LLB_OK
+            lib.llb_dit_packed_bytes(C.byref(cfg), C.byref(nbytes)) == _cabi.LLB_OK and \
+            lib.llb_dit_grad_packed_bytes(C.byref(cfg), C.byref(nbytes)) == _cabi.LLB_OK
 
     def denoise_on_device(self, X_t, E_t, node_mask, c):
         """Masked logits (B,N,16), (B,N,N,5) of the one-hot noisy state (X_t, E_t) at condition c (B,H), in the parameters'
