@@ -328,6 +328,47 @@ int llb_gin_predictor_forward_saved(llb_gin* h, const float* c, float* logits, v
 int llb_gin_predictor_backward_c(llb_gin* h, int num_nodes, int num_edges, int num_graphs, const float* c,
                                  const float* dlogits, void* saved, size_t saved_bytes, const void* grad_blob,
                                  size_t grad_bytes, float* dc, llb_stream_t stream);
+/* Backward of GraphCLIP.forward with respect to every parameter of the encoder (GNNEncoder + ProjectionHead).
+ *   llb_gin_encoder_saved_bytes / llb_gin_encoder_forward_saved: llb_gin_encoder_forward (the same kernels: bit-identical
+ *     embeddings, fused layer tail included) that also stores what the backward needs into the caller's `saved` buffer: the
+ *     batch bookkeeping and atom ids, every layer's input and aggregation, the virtual node's pooled rows, the read-out, the head's
+ *     output before the L2 normalisation, and transposed bf16 copies of the weights the backward multiplies by (about 90 MB at
+ *     H = 768, L = 5).  A later llb_gin_bind therefore does not change this forward's gradient.  The buffer also holds the
+ *     backward's scratch: one buffer per forward whose gradient is wanted.
+ *   llb_gin_encoder_backward: d_out (B,H) fp32 = dL/d(embeddings) -> the fp32 gradient of every parameter, written (not
+ *     accumulated) at the parameter's true shape through `grads`, for the forward that filled `saved` (pass that forward's batch
+ *     sizes).  Dropout is not applied (the forward never applies it).  Run-to-run bit-identical.
+ * These entries reject predictor configs; llb_gin_grad_packed_bytes / llb_gin_saved_bytes reject encoder configs. */
+typedef struct {
+  float* atom_emb;                 /* (118,H) */
+  float* vn_emb;                   /* (1,H) */
+  /* per layer arrays [L] */
+  float* const* eps;               /* (1) */
+  float* const* mlp0_w;            /* (4H,H) */
+  float* const* mlp0_b;            /* (4H) */
+  float* const* mlp_ln_w;
+  float* const* mlp_ln_b;          /* (4H) */
+  float* const* mlp4_w;            /* (H,4H) */
+  float* const* mlp4_b;            /* (H) */
+  float* const* bond_emb;          /* (5,H) */
+  float* const* norm_w;
+  float* const* norm_b;            /* (H) */
+  /* virtual-node MLPs, arrays [L-1] */
+  float* const* vn0_w;
+  float* const* vn0_b;
+  float* const* vn_ln_w;
+  float* const* vn_ln_b;
+  float* const* vn4_w;
+  float* const* vn4_b;
+  /* ProjectionHead fc1 / norm1 / fc2 (H,H) */
+  float *head0_w, *head0_b;
+  float *head_ln_w, *head_ln_b;
+  float *head4_w, *head4_b;
+} llb_gin_encoder_grads;
+int llb_gin_encoder_saved_bytes(const llb_gin_config* cfg, int num_nodes, int num_edges, int num_graphs, size_t* bytes);
+int llb_gin_encoder_forward_saved(llb_gin* h, float* out, void* saved, size_t saved_bytes, llb_stream_t stream);
+int llb_gin_encoder_backward(llb_gin* h, int num_nodes, int num_edges, int num_graphs, const float* d_out, void* saved,
+                             size_t saved_bytes, const llb_gin_encoder_grads* grads, llb_stream_t stream);
 /* Kernels this handle has issued since it was created. */
 int64_t llb_gin_launch_count(const llb_gin* h);
 /* Statistics of the last llb_gin_predictor_topk call on this handle: rows that went through the fused head + softmax + top-k

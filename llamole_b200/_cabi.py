@@ -56,6 +56,16 @@ class GinWeights(C.Structure):
     ]
 
 
+class GinEncoderGrads(C.Structure):
+    _fields_ = [
+        ("atom_emb", _F), ("vn_emb", _F),
+        ("eps", _FF), ("mlp0_w", _FF), ("mlp0_b", _FF), ("mlp_ln_w", _FF), ("mlp_ln_b", _FF), ("mlp4_w", _FF),
+        ("mlp4_b", _FF), ("bond_emb", _FF), ("norm_w", _FF), ("norm_b", _FF),
+        ("vn0_w", _FF), ("vn0_b", _FF), ("vn_ln_w", _FF), ("vn_ln_b", _FF), ("vn4_w", _FF), ("vn4_b", _FF),
+        ("head0_w", _F), ("head0_b", _F), ("head_ln_w", _F), ("head_ln_b", _F), ("head4_w", _F), ("head4_b", _F),
+    ]
+
+
 # name -> (restype, argtypes); mirrors include/llamole_b200.h one to one
 _P = C.c_void_p
 _SZ = C.c_size_t
@@ -106,6 +116,9 @@ SIGNATURES = {
     "llb_gin_saved_bytes": (_I, [C.POINTER(GinConfig), _I, _I, _I, C.POINTER(_SZ)]),
     "llb_gin_predictor_forward_saved": (_I, [_P, _P, _P, _P, _SZ, _P]),
     "llb_gin_predictor_backward_c": (_I, [_P, _I, _I, _I, _P, _P, _P, _SZ, _P, _SZ, _P, _P]),
+    "llb_gin_encoder_saved_bytes": (_I, [C.POINTER(GinConfig), _I, _I, _I, C.POINTER(_SZ)]),
+    "llb_gin_encoder_forward_saved": (_I, [_P, _P, _P, _SZ, _P]),
+    "llb_gin_encoder_backward": (_I, [_P, _I, _I, _I, _P, _P, _SZ, C.POINTER(GinEncoderGrads), _P]),
     "llb_gin_launch_count": (C.c_int64, [_P]),
     "llb_gin_stat": (C.c_int64, [_P, _I]),
     "llb_softmax_topk": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P]),
@@ -165,6 +178,16 @@ def params_fingerprint(module) -> tuple:
     """Identity + version of every parameter of `module`: changes when a parameter is replaced, moved, cast or written in
     place (torch bumps `_version` on every in-place write), which is when a packed-weight blob made from it is stale."""
     return tuple((p.data_ptr(), p._version, p.dtype) for p in module.parameters())
+
+
+def arch_ok(device) -> bool:
+    """True when `device` is a CUDA device that passes llb_arch_check (an sm_100 B200)."""
+    import torch
+
+    device = torch.device(device)
+    if device.type != "cuda":
+        return False
+    return lib().llb_arch_check(device.index if device.index is not None else torch.cuda.current_device()) == LLB_OK
 
 
 def require_cuda(t, name: str):

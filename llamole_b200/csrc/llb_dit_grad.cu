@@ -379,7 +379,7 @@ int llb_dit_pack_grad_weights(llb_dit* h, void* grad_blob, size_t grad_bytes, ll
   auto dst = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(base + off); };
   auto tr = [&](size_t src, int rows, int cols, __nv_bfloat16* d, int ld_d) {
     return launch_kernel(&h->ctr, NO_PROF, false, grad_transpose_kernel<__nv_bfloat16>, dim3(ceil_div(cols, 32), ceil_div(rows, 32)), dim3(32, 8), 0, s,
-                         h->w<__nv_bfloat16>(src), cols, rows, cols, d, ld_d);
+                         h->w<__nv_bfloat16>(src), cols, rows, cols, d, ld_d, rows);
   };
   const int H = L.H, F = L.F, D = L.D;
   LLB_CUDA_OK(cudaMemsetAsync(base, 0, R.total, s));   // the K padding of the out-layer and condition operands is zero

@@ -1180,7 +1180,8 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
   }
   for (int l = 0; l < L; ++l) {
     const bool last = (l == L - 1);
-    if (sv && l > 0) LLB_CUDA_OK(cudaMemcpyAsync(sv->hin + (size_t)(l - 1) * n * H, g->h, (size_t)n * H * 4, cudaMemcpyDeviceToDevice, s));
+    if (sv && l >= sv->hin_l0)
+      LLB_CUDA_OK(cudaMemcpyAsync(sv->hin + (size_t)(l - sv->hin_l0) * n * H, g->h, (size_t)n * H * 4, cudaMemcpyDeviceToDevice, s));
     {
       const float* be = g->w<float>(G.bond_emb[l]);
       const float* ep = g->w<float>(G.eps[l]);
@@ -1265,6 +1266,50 @@ static int gin_trunk(llb_gin* g, const float* c, cudaStream_t s, const GinSaved*
                         g->pooled, g->pooled_b));
   if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->pooled_b, g->pooled_b, (size_t)B * H * 2, cudaMemcpyDeviceToDevice, s));
   return LLB_OK;
+}
+
+// GraphCLIP.forward after the bind.  sv != null: also keep what llb_gin_encoder_backward needs (copies of buffers the unchanged
+// kernels write, so the embeddings are the same either way).
+static int gin_encoder_run(llb_gin* g, float* out, float* pooled_or_null, cudaStream_t s, const GinSaved* sv) {
+  const GinLayout& G = g->G;
+  const int B = g->B;
+  LLB_TRY(gin_trunk(g, nullptr, s, sv));
+  // the caller's (B,H) rows come out of the internal (B,Hp) ones
+  if (pooled_or_null)
+    LLB_CUDA_OK(cudaMemcpy2DAsync(pooled_or_null, (size_t)G.H * 4, g->pooled, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
+  LLB_TRY(gin_mlp4(g, g->pooled_b, B, G.head0_w, G.head0_b, G.head_ln_w, G.head_ln_b, G.head4_w, G.head4_b, G.HH, G.HHt, G.HO, g->hz,
+                   g->head_out, G.Hp, s, LLB_PROF_GIN_GEMM_HEAD, LLB_PROF_GIN_GEMM_HEAD));
+  if (sv) LLB_CUDA_OK(cudaMemcpyAsync(sv->y, g->head_out, (size_t)B * G.Hp * 4, cudaMemcpyDeviceToDevice, s));
+  // L2 normalisation (the padded columns are 0 and add nothing): straight into the caller's rows when the row kernel can write
+  // H columns (H % 4 == 0), else in place at the padded width and a strided copy
+  const bool direct = G.H % 4 == 0;
+  RowLnArgs a;
+  a.in = g->head_out, a.in_ld = G.Hp, a.rows = B, a.width = direct ? G.H : G.Hp, a.normalize = false, a.l2_normalize = true;
+  a.out_f32 = direct ? out : g->head_out, a.out_f32_ld = direct ? G.H : G.Hp;
+  a.prof_slot = LLB_PROF_GIN_MISC;
+  LLB_TRY(launch_row_ln(a, s, &g->ctr));
+  if (!direct)
+    LLB_CUDA_OK(cudaMemcpy2DAsync(out, (size_t)G.H * 4, g->head_out, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
+  return LLB_OK;
+}
+
+// The bound batch's bookkeeping into a saved forward's buffer (graph ranges, node -> graph, atom ids, and the source-sorted CSR
+// the transpose of the aggregation walks), so that a later llb_gin_bind cannot change that forward's gradient.
+static int gin_save_batch(llb_gin* g, const GinSaved& sv, cudaStream_t s) {
+  const int n = g->n, B = g->B;
+  LLB_CUDA_OK(cudaMemcpyAsync(sv.graph_ptr, g->graph_ptr, (size_t)(B + 1) * 4, cudaMemcpyDeviceToDevice, s));
+  LLB_CUDA_OK(cudaMemcpyAsync(sv.batch32, g->batch32, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
+  if (sv.x32) LLB_CUDA_OK(cudaMemcpyAsync(sv.x32, g->x32, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
+  // source-sorted CSR (the bound batch's degree scratch is free once llb_gin_bind has built the destination CSR)
+  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
+  const dim3 node_blocks(ceil_div(n, 256));
+  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<0>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, nullptr, g->deg,
+                        nullptr, nullptr, n));
+  LLB_TRY(gin_scan(g, g->deg, sv.srowptr, s));
+  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
+  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<1>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, sv.srowptr,
+                        g->deg, sv.sdst, sv.seid, n));
+  return launch_kernel(&g->ctr, NO_PROF, false, gin_sort_rows_kernel, node_blocks, dim3(256), 0, s, sv.srowptr, sv.sdst, sv.seid, n);
 }
 
 extern "C" {
@@ -1456,26 +1501,7 @@ int llb_gin_input_flags(llb_gin* g, int32_t* flags_host, llb_stream_t stream) {
 
 int llb_gin_encoder_forward(llb_gin* g, float* out, float* pooled_or_null, llb_stream_t stream) {
   LLB_CHECK_ARG(g && out && !g->G.predictor, "llb_gin_encoder_forward: needs an encoder handle and an output buffer");
-  cudaStream_t s = (cudaStream_t)stream;
-  const GinLayout& G = g->G;
-  const int B = g->B;
-  LLB_TRY(gin_trunk(g, nullptr, s));
-  // the caller's (B,H) rows come out of the internal (B,Hp) ones
-  if (pooled_or_null)
-    LLB_CUDA_OK(cudaMemcpy2DAsync(pooled_or_null, (size_t)G.H * 4, g->pooled, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
-  LLB_TRY(gin_mlp4(g, g->pooled_b, B, G.head0_w, G.head0_b, G.head_ln_w, G.head_ln_b, G.head4_w, G.head4_b, G.HH, G.HHt, G.HO, g->hz,
-                   g->head_out, G.Hp, s, LLB_PROF_GIN_GEMM_HEAD, LLB_PROF_GIN_GEMM_HEAD));
-  // L2 normalisation (the padded columns are 0 and add nothing): straight into the caller's rows when the row kernel can write
-  // H columns (H % 4 == 0), else in place at the padded width and a strided copy
-  const bool direct = G.H % 4 == 0;
-  RowLnArgs a;
-  a.in = g->head_out, a.in_ld = G.Hp, a.rows = B, a.width = direct ? G.H : G.Hp, a.normalize = false, a.l2_normalize = true;
-  a.out_f32 = direct ? out : g->head_out, a.out_f32_ld = direct ? G.H : G.Hp;
-  a.prof_slot = LLB_PROF_GIN_MISC;
-  LLB_TRY(launch_row_ln(a, s, &g->ctr));
-  if (!direct)
-    LLB_CUDA_OK(cudaMemcpy2DAsync(out, (size_t)G.H * 4, g->head_out, (size_t)G.Hp * 4, (size_t)G.H * 4, B, cudaMemcpyDeviceToDevice, s));
-  return LLB_OK;
+  return gin_encoder_run(g, out, pooled_or_null, (cudaStream_t)stream, nullptr);
 }
 
 static int gin_head_hidden(llb_gin* g, cudaStream_t s) {
@@ -1521,23 +1547,35 @@ int llb_gin_predictor_forward_saved(llb_gin* g, const float* c, float* logits, v
   size_t need = 0;
   gin_saved_carve(G, saved, n, e, B, &sv, &need);
   if (saved_bytes < need) return fail(LLB_ERR_WORKSPACE, "gin: saved buffer needs %zu bytes, got %zu", need, saved_bytes);
-  LLB_CUDA_OK(cudaMemcpyAsync(sv.graph_ptr, g->graph_ptr, (size_t)(B + 1) * 4, cudaMemcpyDeviceToDevice, s));
-  LLB_CUDA_OK(cudaMemcpyAsync(sv.batch32, g->batch32, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
-  // source-sorted CSR (the bound batch's degree scratch is free once llb_gin_bind has built the destination CSR)
-  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
-  const dim3 node_blocks(ceil_div(n, 256));
-  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<0>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, nullptr, g->deg,
-                        nullptr, nullptr, n));
-  LLB_TRY(gin_scan(g, g->deg, sv.srowptr, s));
-  LLB_CUDA_OK(cudaMemsetAsync(g->deg, 0, (size_t)(n + 1) * 4, s));
-  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_csr_transpose_kernel<1>, node_blocks, dim3(256), 0, s, g->rowptr, g->col, g->eid, sv.srowptr,
-                        g->deg, sv.sdst, sv.seid, n));
-  LLB_TRY(launch_kernel(&g->ctr, NO_PROF, false, gin_sort_rows_kernel, node_blocks, dim3(256), 0, s, sv.srowptr, sv.sdst, sv.seid, n));
+  LLB_TRY(gin_save_batch(g, sv, s));
   // from here on exactly llb_gin_predictor_forward
   LLB_TRY(gin_trunk(g, c, s, &sv));
   LLB_TRY(gin_head_hidden(g, s));
   return gemm_bias_act(g->hz, G.HH, g->w<void>(G.head4_w), G.HH, g->w<float>(G.head4_b), logits, G.out_dim, B, G.out_dim, G.HH,
                        LLB_ACT_NONE, true, s, &g->ctr);
+}
+
+int llb_gin_encoder_saved_bytes(const llb_gin_config* cfg, int num_nodes, int num_edges, int num_graphs, size_t* bytes) {
+  LLB_CHECK_ARG(cfg && bytes && num_nodes >= 1 && num_edges >= 0 && num_graphs >= 1, "llb_gin_encoder_saved_bytes: bad argument");
+  LLB_CHECK_ARG(!cfg->predictor, "llb_gin_encoder_saved_bytes: needs an encoder config");
+  GinLayout G;
+  LLB_TRY(make_layout(*cfg, G));
+  gin_saved_carve(G, nullptr, num_nodes, num_edges, num_graphs, nullptr, bytes);
+  return LLB_OK;
+}
+
+int llb_gin_encoder_forward_saved(llb_gin* g, float* out, void* saved, size_t saved_bytes, llb_stream_t stream) {
+  LLB_CHECK_ARG(g && out && saved && !g->G.predictor, "llb_gin_encoder_forward_saved: needs an encoder handle and output buffers");
+  LLB_CHECK_ARG(g->n > 0 && g->B > 0, "gin: no graph batch bound");
+  cudaStream_t s = (cudaStream_t)stream;
+  GinSaved sv;
+  size_t need = 0;
+  gin_saved_carve(g->G, saved, g->n, g->e, g->B, &sv, &need);
+  if (saved_bytes < need) return fail(LLB_ERR_WORKSPACE, "gin: saved buffer needs %zu bytes, got %zu", need, saved_bytes);
+  LLB_TRY(gin_save_batch(g, sv, s));
+  LLB_TRY(gin_pack_grad_weights(g, sv.wt, s));
+  // from here on exactly llb_gin_encoder_forward
+  return gin_encoder_run(g, out, nullptr, s, &sv);
 }
 
 int llb_gin_predictor_topk(llb_gin* g, const float* c, int k, float* topk_prob, int32_t* topk_idx, llb_stream_t stream) {

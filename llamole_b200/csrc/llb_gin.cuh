@@ -1,5 +1,6 @@
-// State shared by the GIN forward (llb_gin.cu) and the predictor's backward with respect to the text condition
-// (llb_gin_grad.cu): the packed-weight layout, the handle, and the buffers a saved forward leaves for its backward.
+// State shared by the GIN forward (llb_gin.cu) and the backward passes (llb_gin_grad.cu: the predictor's with respect to the
+// text condition, the encoder's with respect to its parameters): the packed-weight layout, the handle, and the buffers a saved
+// forward leaves for its backward.
 #pragma once
 #include <vector>
 
@@ -33,14 +34,16 @@ struct GinLayout {
 
 int make_layout(const llb_gin_config& c, GinLayout& G);
 
-// What llb_gin_predictor_forward_saved keeps for llb_gin_predictor_backward_c, carved from the caller's `saved` buffer.  The
-// first group is written by the forward; the rest is scratch of the backward.  The batch bookkeeping is copied too, so that a
-// later llb_gin_bind on the same handle cannot change the gradient of an earlier forward.
+// What llb_gin_predictor_forward_saved / llb_gin_encoder_forward_saved keep for their backward, carved from the caller's
+// `saved` buffer.  The first group is written by the forward; the rest is scratch of the backward.  The batch bookkeeping is
+// copied too, so that a later llb_gin_bind on the same handle cannot change the gradient of an earlier forward.  Fields that
+// one of the two does not use have size 0.
 struct GinSaved {
   // written by the forward
   int32_t *graph_ptr, *batch32;          // (B+1), (n)
   int32_t *srowptr, *sdst, *seid;        // SOURCE-sorted CSR: out-edges of every node, ordered by edge id (n+1), (e), (e)
-  float* hin;                            // (L-1, n, Hp) fp32: the input h_in_l of layers 1..L-1
+  int hin_l0;                            // first layer whose input is stored: 1 (predictor: layer 0's does not depend on c), 0 (encoder)
+  float* hin;                            // (L-hin_l0, n, Hp) fp32: the input h_in_l of layers hin_l0..L-1
   __nv_bfloat16* agg;                    // (L, n, Hp): the node MLP's input of every layer
   __nv_bfloat16* pool;                   // (L-1, B, Hp): max-pooled rows that feed the virtual-node MLPs
   float* mod;                            // (L, B, 3Hp): [shift | scale | gate] of every layer
@@ -67,6 +70,21 @@ struct GinSaved {
   float* da;                             // (n, Hp)
   __nv_bfloat16* dmod_b;                 // (B, L x 3Hp) all layers' modulation gradients side by side
   float* dctext;                         // (B, text_dim)
+  // encoder only -- written by the forward
+  int32_t* x32;                          // (n) atom ids
+  float* y;                              // (B, Hp) the projection head's output before the L2 normalisation
+  uint8_t* wt;                           // transposed bf16 weights (GinGradLayout), so the gradient belongs to this forward's weights
+  // encoder only -- backward scratch
+  __nv_bfloat16 *hz_post, *vz_post;      // (B, Hp), (B, I) recomputed GELU(LayerNorm) rows (inputs of the head's / vn MLP's fc2)
+  float* dyh;                            // (B, Hp) gradient of the head output
+  __nv_bfloat16* dyh_b;                  // (B, Hp)
+  __nv_bfloat16 *tA, *tW;                // (I, kmax) transposed activations: the operands of the weight-gradient products
+  float* wpart;                          // split-K partial products of a weight gradient
+  float* cpart;                          // partial column sums over row chunks
+  float* apart;                          // (ceil(n / ATOM_CHUNK), 118, Hp) per-chunk atom-embedding sums
+  float* bpart;                          // (ceil(n / GRAD_CHUNK), 6, Hp) per-chunk bond-type (5) and eps (1) sums
+  float* evec;                           // (Hp) eps column sums
+  int kmax;                              // K capacity of tA / tW
 };
 // Carves `saved` (nullptr: sizing only) for a batch of n nodes, e edges, B graphs; *bytes receives the size.
 void gin_saved_carve(const GinLayout& G, void* saved, int n, int e, int B, GinSaved* sv, size_t* bytes);
@@ -74,6 +92,10 @@ void gin_saved_carve(const GinLayout& G, void* saved, int n, int e, int B, GinSa
 // multiples of 64.
 int head_grad_kp(const GinLayout& G);
 int head_grad_split(const GinLayout& G, int B);
+// Bytes of the transposed bf16 weight copies the backward multiplies by, and writes them at `base` (the predictor's grad blob;
+// the encoder's `saved` buffer).
+size_t gin_grad_weights_bytes(const GinLayout& G);
+int gin_pack_grad_weights(llb_gin* g, void* base, cudaStream_t s);
 
 }  // namespace llb
 

@@ -1,4 +1,4 @@
-// Kernels shared by the backward passes with respect to a condition vector (llb_gin_grad.cu, llb_dit_grad.cu).
+// Kernels shared by the backward passes (llb_gin_grad.cu, llb_dit_grad.cu).
 #pragma once
 #include "llb_common.cuh"
 
@@ -7,11 +7,13 @@ namespace {
 
 __device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(float v) { return v; }
 
-// dst (cols, rows) bf16 with row stride ld_d  <-  src (rows, cols) with row stride ld_s; 32 x 32 tiles through shared memory
+// dst (cols, rows_out) bf16 with row stride ld_d  <-  src (rows, cols) with row stride ld_s, zero in dst columns [rows, rows_out)
+// (the K padding of a split-K product); 32 x 32 tiles through shared memory, grid (ceil(cols/32), ceil(rows_out/32))
 template <class T>
 __global__ void __launch_bounds__(256) grad_transpose_kernel(const T* __restrict__ src, int ld_s, int rows, int cols,
-                                                             __nv_bfloat16* __restrict__ dst, int ld_d) {
+                                                             __nv_bfloat16* __restrict__ dst, int ld_d, int rows_out) {
   __shared__ float tile[32][33];
   const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32, tx = threadIdx.x, ty = threadIdx.y;
   for (int k = ty; k < 32; k += 8) {
@@ -21,7 +23,7 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const T* __restrict
   __syncthreads();
   for (int k = ty; k < 32; k += 8) {
     const int c = c0 + k, r = r0 + tx;
-    if (c < cols && r < rows) dst[(size_t)c * ld_d + r] = __float2bfloat16(tile[tx][k]);
+    if (c < cols && r < rows_out) dst[(size_t)c * ld_d + r] = __float2bfloat16(tile[tx][k]);
   }
 }
 

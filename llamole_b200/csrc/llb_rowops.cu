@@ -166,9 +166,11 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(RowLnBwdArgs a) {
       p0 = dt, p1 = dt * xh, p2 = dyv * (a.gelu ? gelu_erf(t) : t);
     }
     if (a.out_bf16) a.out_bf16[(size_t)row * a.out_ld + c] = __float2bfloat16(dx);
+    if (a.out_f32) a.out_f32[(size_t)row * a.out_ld + c] = dx;   // after the last read of dy[c] by this lane
     if (a.prod) {
       float* pr = a.prod + (size_t)row * a.prod_ld + c;
-      pr[0] = p0, pr[W] = p1, pr[2 * W] = p2;
+      pr[0] = p0, pr[W] = p1;
+      if (a.prod_sets > 2) pr[2 * W] = p2;
     }
   }
 }

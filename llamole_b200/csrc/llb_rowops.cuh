@@ -42,8 +42,9 @@ int launch_row_ln(const RowLnArgs& a, cudaStream_t stream, LaunchCounter* ctr);
 
 // Backward of the row LayerNorm above without residual / addvec (they pass the gradient through unchanged): with
 //   xh = LN(x) over the first `valid` columns,  t = xh * gamma + beta  or  xh * (1 + scale[g]) + shift[g],  out = gate[g] * act(t),
-// and dy = dL/d(out), writes dx = dL/dx (bf16, 0 in the padded columns) and, when `prod` is set, the per-row products whose
-// per-group sums are the gradients of [shift | scale | gate]: [dt | dt * xh | dy * act(t)] at columns 0, width, 2 width.
+// and dy = dL/d(out), writes dx = dL/dx (bf16 and/or fp32, 0 in the padded columns; the fp32 copy may overwrite dy in place)
+// and, when `prod` is set, the per-row products whose per-group sums are the gradients of [shift | scale | gate] (or, summed
+// over all rows, of [beta | gamma]): [dt | dt * xh | dy * act(t)] at columns 0, width, 2 width (the first prod_sets of them).
 // act is GELU (exact derivative of the erf form) or none.  One warp per row, sums in a fixed order: run-to-run deterministic.
 struct RowLnBwdArgs {
   const void* x = nullptr;   // the forward's LayerNorm input
@@ -64,8 +65,10 @@ struct RowLnBwdArgs {
   bool gelu = false;
   float* prod = nullptr;
   int prod_ld = 0;
+  int prod_sets = 3;
   __nv_bfloat16* out_bf16 = nullptr;
   int out_ld = 0;
+  float* out_f32 = nullptr;   // row stride out_ld as well
   int prof_slot = LLB_PROF_GIN_ROWLN;
 };
 int launch_row_ln_bwd(const RowLnBwdArgs& a, cudaStream_t stream, LaunchCounter* ctr);

@@ -148,6 +148,63 @@ class GinEngine:
                         "llb_gin_encoder_forward")
         return (out, pooled) if want_pooled else out
 
+    def encoder_forward_saved(self):
+        """encoder_forward (bit-identical embeddings) that also returns what encoder_backward needs: the `saved` buffer and the
+        batch sizes it was filled for.  The buffer belongs to this call, so several forwards can be back-propagated in any order."""
+        out = torch.empty((self.B, self.H), dtype=torch.float32, device=self.device)
+        dims = (self.n, self.e, self.B)
+        with torch.cuda.device(self.device):
+            need = C.c_size_t()
+            _cabi.check(self.lib.llb_gin_encoder_saved_bytes(C.byref(self.cfg), *dims, C.byref(need)), "llb_gin_encoder_saved_bytes")
+            saved = torch.empty(need.value, dtype=torch.uint8, device=self.device)
+            _cabi.check(self.lib.llb_gin_encoder_forward_saved(self.handle, _cabi.ptr(out), _cabi.ptr(saved), need.value, _cabi.stream_ptr()),
+                        "llb_gin_encoder_forward_saved")
+        return out, saved, dims
+
+    def encoder_backward(self, d_out: torch.Tensor, saved: torch.Tensor, dims):
+        """fp32 gradients of every encoder parameter from dL/d(embeddings) (B,H) of the forward that filled `saved`:
+        ({trunk state-dict key: grad}, {ProjectionHead state-dict key: grad})."""
+        n, e, B = dims
+        H, L, dev = self.H, self.L, self.device
+        d_out = d_out.to(dev, torch.float32).contiguous()
+        assert d_out.shape == (B, H), (d_out.shape, B, H)
+        new = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)  # noqa: E731
+        trunk = {"atom_encoder.weight": new(118, H), "virtualnode_embedding.weight": new(1, H)}
+        for l in range(L):
+            p = f"convs.{l}."
+            trunk.update({p + "eps": new(1), p + "mlp.0.weight": new(4 * H, H), p + "mlp.0.bias": new(4 * H),
+                          p + "mlp.1.weight": new(4 * H), p + "mlp.1.bias": new(4 * H), p + "mlp.4.weight": new(H, 4 * H),
+                          p + "mlp.4.bias": new(H), p + "bond_encoder.weight": new(5, H),
+                          f"norms.{l}.weight": new(H), f"norms.{l}.bias": new(H)})
+        for l in range(L - 1):
+            p = f"mlp_virtualnode_list.{l}."
+            trunk.update({p + "0.weight": new(4 * H, H), p + "0.bias": new(4 * H), p + "1.weight": new(4 * H), p + "1.bias": new(4 * H),
+                          p + "4.weight": new(H, 4 * H), p + "4.bias": new(H)})
+        head = {k: new(H, H) if k.endswith("weight") and k.startswith("fc") else new(H)
+                for k in ("fc1.weight", "fc1.bias", "norm1.weight", "norm1.bias", "fc2.weight", "fc2.bias")}
+        keep = []
+
+        def arr(fmt, count):
+            a = _cabi.ptr_array([trunk[fmt.format(i)] for i in range(count)])
+            keep.append(a)
+            return C.cast(a, C.POINTER(C.c_void_p))
+
+        p = lambda t: _cabi.ptr(t)  # noqa: E731
+        gr = _cabi.GinEncoderGrads(
+            p(trunk["atom_encoder.weight"]), p(trunk["virtualnode_embedding.weight"]),
+            arr("convs.{}.eps", L), arr("convs.{}.mlp.0.weight", L), arr("convs.{}.mlp.0.bias", L), arr("convs.{}.mlp.1.weight", L),
+            arr("convs.{}.mlp.1.bias", L), arr("convs.{}.mlp.4.weight", L), arr("convs.{}.mlp.4.bias", L),
+            arr("convs.{}.bond_encoder.weight", L), arr("norms.{}.weight", L), arr("norms.{}.bias", L),
+            arr("mlp_virtualnode_list.{}.0.weight", L - 1), arr("mlp_virtualnode_list.{}.0.bias", L - 1),
+            arr("mlp_virtualnode_list.{}.1.weight", L - 1), arr("mlp_virtualnode_list.{}.1.bias", L - 1),
+            arr("mlp_virtualnode_list.{}.4.weight", L - 1), arr("mlp_virtualnode_list.{}.4.bias", L - 1),
+            p(head["fc1.weight"]), p(head["fc1.bias"]), p(head["norm1.weight"]), p(head["norm1.bias"]), p(head["fc2.weight"]),
+            p(head["fc2.bias"]))
+        with torch.cuda.device(dev):
+            _cabi.check(self.lib.llb_gin_encoder_backward(self.handle, n, e, B, _cabi.ptr(d_out), _cabi.ptr(saved), saved.numel(),
+                                                          C.byref(gr), _cabi.stream_ptr()), "llb_gin_encoder_backward")
+        return trunk, head
+
     def predictor_forward(self, c: Optional[torch.Tensor]):
         logits = torch.empty((self.B, self.out_dim), dtype=torch.float32, device=self.device)
         if c is not None:
